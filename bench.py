@@ -19,6 +19,9 @@ of it is reported under `configs`).  One fused polyphase-FIR stage on the FP64 t
              (kind "port": the reference is Julia and cannot run here)
 
 `--impl reference` times that CPU restatement alone on the same config.
+`--dump-outputs DIR` writes a fixed sample of the outputs of the last timed step of cfg3 and of each sub-config
+(dump_sample); inputs are seeded, so two builds run with the same arguments can be compared output for output.
+Normpower sums x² with atomics, so outputs downstream of it (cfg4) may differ in the last bits from run to run.
 Multi-GPU: one rank per GPU under torchrun, instances sharded, no data-path collective
 (weak scaling: 1024 signals per GPU).  `--single-process` instead drives all N GPUs from ONE
 process through `sigops_ctx_create(devices, N)` (the drop-in's own sharding).
@@ -181,6 +184,31 @@ class ClockSampler:
     def stop(self):
         self._stop.set()
         self.t.join(timeout=2)
+
+
+DUMP_BYTES = {"cfg3": 32 << 20, "cfg2": 8 << 20, "cfg4": 8 << 20, "cfg5": 8 << 20}   # 56 MiB in all
+
+
+def dump_sample(out_dir, name, y):
+    """Writes a fixed, seeded sample of one batch output y (ninst, nchannels, nframes), on the device or the
+    host, as out_dir/<name>.npy in y's own dtype: up to 8 instances (the first and the last among them) x every
+    channel x the first and last frames and a seeded draw of the frames in between, DUMP_BYTES[name] at most.
+    The same shape of y always gives the same sample, so two builds can be compared value for value."""
+    import torch
+    ninst, nch, nframes = y.shape
+    rng = np.random.default_rng(1983)
+    inst = np.unique(np.concatenate([[0, ninst - 1], rng.permutation(np.arange(1, ninst - 1))[:6]]))
+    nf = max(1, DUMP_BYTES[name] // (len(inst) * nch * y.element_size()))
+    if nf >= nframes:
+        frames = np.arange(nframes)
+    else:
+        edge = min(1024, nf // 4)
+        middle = edge + rng.choice(nframes - 2 * edge, nf - 2 * edge, replace=False)
+        frames = np.sort(np.concatenate([np.arange(edge), middle, np.arange(nframes - edge, nframes)]))
+    frames = torch.from_numpy(frames).to(y.device)
+    s = torch.stack([y[int(i)].index_select(1, frames) for i in inst])
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, name + ".npy"), s.cpu().numpy())
 
 
 def bind_to_gpu_numa_node(gpu_index):
@@ -388,7 +416,7 @@ def parity_sub(name, batch):
     return worst
 
 
-def run_subconfig(name, ctx, dev, stream, barrier, rank, steps, min_seconds=0.5):
+def run_subconfig(name, ctx, dev, stream, barrier, rank, steps, min_seconds=0.5, dump_dir=None):
     import torch
     cfg = SUBCONFIGS[name]
     batch = DeviceBatch(ctx, cfg["graph"](), cfg["ninst"], dev, 1983 + 17 * rank)
@@ -401,6 +429,8 @@ def run_subconfig(name, ctx, dev, stream, barrier, rank, steps, min_seconds=0.5)
     ms1, _, _ = time_steps(batch, stream, 1, barrier, ctx)
     k = max(steps, int(math.ceil(min_seconds * 1e3 / max(ms1, 1e-3))))
     ms, prof, _ = time_steps(batch, stream, k, barrier, ctx)
+    if dump_dir:
+        dump_sample(dump_dir, name, batch.ys[0])
     peak, _ = measured_peaks()
     kind = cfg["kernel"]
     kms, kn = prof.get(kind, (0.0, 0))
@@ -483,6 +513,8 @@ def run_gpu(args, rank, world, local_rank):
 
     # ---- timed region: exactly K steps, device resident
     ms, prof, clocks = time_steps(batch, stream, args.steps, barrier, ctx, sampler)
+    if args.dump_outputs and rank == 0:
+        dump_sample(args.dump_outputs, "cfg3", batch.ys[0])
     # ---- the same loop for >= 2 s (power / thermal behaviour; reported beside the K-step number)
     k_sus = max(args.steps, int(math.ceil(2000.0 / max(ms / args.steps, 1e-3))))
     ms_sus, _, clocks_sus = time_steps(batch, stream, k_sus, barrier, ctx, sampler)
@@ -556,7 +588,8 @@ def run_gpu(args, rank, world, local_rank):
     if rank == 0 and args.configs:
         for name in args.configs.split(","):
             if name in SUBCONFIGS:
-                subs[name] = run_subconfig(name, ctx, dev, stream, lambda: torch.cuda.synchronize(), rank, 5)
+                subs[name] = run_subconfig(name, ctx, dev, stream, lambda: torch.cuda.synchronize(), rank, args.steps,
+                                           dump_dir=args.dump_outputs)
     if sampler:
         sampler.stop()
 
@@ -649,6 +682,8 @@ def run_single_process(args):
     for _ in range(args.steps):
         step()
     sec = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_sample(args.dump_outputs, "cfg3", yh)
     which = sorted({0, ninst - 1})
     want = cpu_resample_batch(np.stack([xh[i].numpy() for i in which]), len(which))
     err = max(float(np.max(np.abs(yh[i].numpy() - want[k])) / np.sqrt(np.mean(want[k] ** 2))) for k, i in enumerate(which))
@@ -669,7 +704,12 @@ def main():
     ap.add_argument("--e2e-ninst", type=int, default=0, help="signals per end-to-end step (0 = sized from host memory)")
     ap.add_argument("--configs", default="cfg2,cfg4,cfg5", help="sub-records to add (comma separated; '' = none)")
     ap.add_argument("--single-process", action="store_true", help="drive all --gpus devices from one process/context")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write a fixed sample of what the last step computed as DIR/<config>.npy "
+                         "(rank 0's cfg3 and each sub-config; 56 MiB at most)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU arm's results; --impl reference has none")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
