@@ -4,6 +4,7 @@
 // sharding over devices (no collectives: instances are independent, SURVEY.md
 // §8e) and the host<->device pipeline of `sigops_plan_run`.
 #include <algorithm>
+#include <array>
 #include <atomic>
 #include <chrono>
 #include <cmath>
@@ -482,19 +483,21 @@ void derive_iir(sigops_plan& p, StageRT& s, int idx) {
 constexpr size_t kFirSmemLimit = 200 * 1024;
 constexpr size_t kFirMmaSmemLimit = 220 * 1024;
 constexpr size_t kFirTmSmemLimit = 232448 - 512;   // 227 KB per block minus the kernel's static barriers
-constexpr int kFirT = 64;     // table padding granularity (largest tile)
+constexpr int kFirT = 64;     // k_fir's tile (outputs), the table padding granularity (largest tile)
 
-// k_fir<G> geometry: merged-tap rows, window pitch and dynamic shared memory
+// k_fir<G, 8> geometry: merged-tap rows, window pitch and dynamic shared memory.  Eight warps make a 64-output
+// tile (measured on B200, config 3: 3.8 ms against 4.7 ms with four warps and 32-output tiles — the smaller tile's
+// extra halo and per-tile set-up cost more than overlapping two blocks per SM buys)
 struct FirGeom {
     int hbase, tpad, xpitch;
     size_t smem;
 };
-FirGeom fir_geometry(const FirDerived& f, int tapsper, int G, int max_stack, int W = 8) {
+FirGeom fir_geometry(const FirDerived& f, int tapsper, int G, int max_stack) {
     FirGeom g;
-    const int T = 8 * W, ypitch = T + 2, pmax = W == 8 ? f.pmax : f.pmax32;
+    constexpr int W = 8, T = 8 * W, ypitch = T + 2;
     g.hbase = (f.dpad + 2) & ~1;                                   // even, >= dmax + 1
     g.tpad = (g.hbase + tapsper + f.dpad + 5 + 8) & ~1;            // + 8: slack read by the 4-pair unrolled tail
-    const int need = pmax + 4 + 8;                               // positions of a tile (+ even start, pair tail rounded to a pair, unroll slack)
+    const int need = f.pmax + 4 + 8;                             // positions of a tile (+ even start, pair tail rounded to a pair, unroll slack)
     g.xpitch = need + ((2 - need % 4) + 4) % 4;                    // = 2 mod 4: lane=row 128-bit reads conflict free
     const size_t xrows = (size_t)std::max(g.xpitch, ypitch);
     g.smem = ((size_t)T * g.tpad + (size_t)32 * G * xrows + (size_t)max_stack * 2 * W * 32) * sizeof(double);
@@ -796,7 +799,7 @@ struct IirLaunch {
     int blocks_per_row;
     int64_t L, Wc, nchunks;
     bool need_matrix;
-    double cost = 0.0;       // the flat chooser's estimate, in lane-frames
+    double cost = 0.0;       // the flat and tensor-map choosers' estimate, in lane-frames
 };
 
 // Chunking for k_iir_tma: chunks are numbered over all rows jointly, so L can be chosen
@@ -827,7 +830,6 @@ IirLaunch choose_iir_chunking_flat(const StageRT& s, int64_t rows, int sm_count,
         if (N % L) cost *= 1.02;                                     // ragged last chunk takes the scalar path
         if (cost < best) { best = cost; bestL = L; }
     }
-    if (const char* e = getenv("SIGOPS_IIR_L")) bestL = std::max<int64_t>(kStageCols, round_up(atoll(e), kStageCols));
     IirLaunch r;
     r.blocks_per_row = 0;
     r.L = bestL;
@@ -838,6 +840,24 @@ IirLaunch choose_iir_chunking_flat(const StageRT& s, int64_t rows, int sm_count,
     return r;
 }
 
+// Chunking for k_iir_tmap: lanes = rows, one group of 32 rows per warp, blocks of `nw` warps in whole waves of one
+// block per SM; a lane walks L + Wc frames with Wc = Wst (the kernel only runs WARM, so L > Wst).  With fused
+// row-invariant programs the warps of a block share a chunk (see k_iir_tmap).
+IirLaunch choose_tmap_chunking(int64_t N, int64_t rows, int64_t stage_cols, int64_t Wst, int nw, bool rowinv, int sm_count) {
+    const int64_t groups = (rows + 31) / 32;
+    const int64_t jmax = std::max<int64_t>(1, (N + stage_cols - 1) / stage_cols);
+    double best = 1e300;
+    int64_t bestL = 0;
+    for (int64_t j = Wst / stage_cols + 1; j <= jmax; j += std::max<int64_t>(1, jmax / 4096)) {
+        const int64_t L = j * stage_cols, cpr = (N + L - 1) / L;
+        const int64_t blocks = rowinv ? cpr * ((groups + nw - 1) / nw) : (groups * cpr + nw - 1) / nw;
+        const int64_t waves = (blocks + sm_count - 1) / sm_count;
+        const double cost = (double)waves * ((double)L + (cpr > 1 ? (double)Wst : 0.0) + 600.0);
+        if (cost < best) { best = cost; bestL = L; }
+    }
+    return IirLaunch{0, bestL, Wst, bestL ? (N + bestL - 1) / bestL : 0, false, best};
+}
+
 IirLaunch choose_iir_chunking(const StageRT& s, int64_t rows, int sm_count) {
     const int64_t N = s.st.n_out;
     const int64_t W32 = round_up(std::max<int64_t>(s.iir.W, 1), 32);
@@ -846,7 +866,6 @@ IirLaunch choose_iir_chunking(const StageRT& s, int64_t rows, int sm_count) {
     auto Lof = [&](int b) { return std::max<int64_t>(32, round_up((N + (int64_t)b * kIirThreads - 1) / ((int64_t)b * kIirThreads), 32)); };
     const int64_t Lmin = std::max<int64_t>(256, std::min<int64_t>(4 * W32, 8192));
     while (rows * bpr < target_blocks && Lof(bpr * 2) >= Lmin && bpr < 4096) bpr *= 2;
-    if (const char* e = getenv("SIGOPS_IIR_BPR")) bpr = std::max(1, atoi(e));   // tuning knob
     IirLaunch r;
     r.blocks_per_row = bpr;
     r.L = Lof(bpr);
@@ -894,6 +913,486 @@ size_t wave_workspace_bytes(const sigops_plan& p, int64_t ninst, int sm_count) {
     return temp_bytes_per_instance(p) * ninst + iir_state_bytes(p, ninst, sm_count) +
            (size_t)ninst * p.nbuf() * sizeof(BufRef) + (size_t)ninst * std::max<uint32_t>(p.h.n_scalars, 1) * sizeof(double) +
            (1 << 16);
+}
+
+// ---- stage launch planning ------------------------------------------------------
+// One planner per stage kind turns a stage of the wave into prepared launches.  Every choice depends on the plan,
+// the wave's BufRef table, the device and the SIGOPS_NO_* switches (read per wave) alone.
+
+struct Wave {                 // what the wave knows when its stages are planned
+    sigops_plan& p;
+    PlanDev& pd;
+    int sm_count;
+    const BufRef* refs;       // host copy of the wave's BufRef table, [ninst][nbuf]
+    BufRef* d_refs;           // its device copy
+    double* scalars;          // [ninst][nscal], zeroed at the start of the wave
+    int nbuf, nscal;
+    int64_t ninst, inst0;
+    size_t si;                // stage being planned
+    Arena& arena;             // IIR state
+    cudaStream_t stream;      // (the synchronous SIGOPS_FIR_DBG launches)
+    std::vector<Slot::Prepared>& launches;
+    void add(int kind, std::function<void(cudaStream_t)> fn) const { launches.push_back({kind, std::move(fn)}); }
+};
+
+// Every instance's rows of buffer `buf` start on a 16-byte boundary (several channels: an even number of
+// elements apart), and with `f64` hold Float64: what the bulk copies of the TMA and tensor-core kernels need.
+bool rows_aligned(const BufRef* refs, int64_t ninst, int nbuf, int buf, bool f64) {
+    for (int64_t i = 0; i < ninst; ++i) {
+        const BufRef& r = refs[i * nbuf + buf];
+        if (((uintptr_t)r.ptr & 15) || (r.nch > 1 && (r.ld & 1)) || (f64 && r.dtype != SIGOPS_F64)) return false;
+    }
+    return true;
+}
+
+// Every row of buffer `buf` in the wave at base + row*stride with 16-byte aligned base and stride, all of type
+// `dtype` (one batch tensor, or the library's own staging): one 2-D tensor map covers the buffer of the whole wave.
+bool strided_matrix(const BufRef* refs, int64_t ninst, int nbuf, int buf, int elem_bytes, int dtype, char** base, int64_t* stride) {
+    const BufRef& r0 = refs[buf];
+    *base = (char*)r0.ptr;
+    *stride = r0.ld * elem_bytes;
+    if ((*stride & 15) || ((uintptr_t)*base & 15) || r0.dtype != dtype) return false;
+    for (int64_t i = 0; i < ninst; ++i) {
+        const BufRef& rb = refs[i * nbuf + buf];
+        if (rb.ld != r0.ld || rb.nch != r0.nch || rb.dtype != dtype || (char*)rb.ptr != *base + (int64_t)i * r0.nch * *stride)
+            return false;
+    }
+    return true;
+}
+
+// Segments along the time axis of the tensor-core FIR kernels (grid = segments x row groups): whole waves of one
+// block per SM; a segment pays about three tiles of start-up (first window, pipeline fill).
+int64_t choose_tiles_per_segment(int64_t ntiles, int64_t groups, int sm_count) {
+    int64_t best_tps = ntiles;
+    double best_cost = 1e300;
+    for (int w = 1; w <= 8; ++w) {
+        int64_t nseg = std::max<int64_t>(1, std::min<int64_t>(ntiles, ((int64_t)w * sm_count + groups - 1) / groups));
+        const int64_t tps = (ntiles + nseg - 1) / nseg;
+        nseg = (ntiles + tps - 1) / tps;
+        const int64_t waves = (groups * nseg + sm_count - 1) / sm_count;
+        const double cost = (double)waves * (double)(tps + 3);
+        if (cost < best_cost) { best_cost = cost; best_tps = tps; }
+    }
+    return best_tps;
+}
+
+// Merged tap bands of one period of a periodic resampler for k_fir_tmap, one table per epoch ([tile][4 groups][ks][8],
+// columns XOR-swizzled like the helper warps write them, the constant-gain epilogue folded in): built and uploaded
+// once per plan, stage, band height and device.
+const double* period_bands(const Wave& w, int ks) {
+    const uint64_t key = ((uint64_t)w.si << 16) | (uint64_t)ks;
+    auto it = w.pd.bands.find(key);
+    if (it != w.pd.bands.end()) return it->second;
+    const sigops_plan& p = w.p;
+    const StageRT& s = p.stages[w.si];
+    const sigops_stage& g = s.st;
+    const int64_t Pp = s.fir.period;
+    const double* hp = p.blob.data() + p.tables[g.pfb_table].offset;
+    const double* hd = g.dpfb_table >= 0 ? p.blob.data() + p.tables[g.dpfb_table].offset : nullptr;
+    const size_t per_epoch = (size_t)(Pp / 8) * ks * 8;
+    std::vector<double> tab(per_epoch * (size_t)s.fir.n_epochs, 0.0);
+    for (int64_t e = 0; e < s.fir.n_epochs; ++e) {
+        const int64_t start = e * s.fir.epoch_tiles * kFmT;          // the epoch's own first period
+        for (int64_t q = 0; q < Pp; ++q) {
+            const int64_t m = start + q, m0 = m & ~int64_t(7);
+            const int n = (int)(m - m0), stn = (int)(s.fir.xi0[m] - s.fir.xi0[m0]);
+            double* band = tab.data() + per_epoch * (size_t)e + (size_t)((q & ~int64_t(7)) / 8) * ks * 8;
+            for (int t = 0; t < g.taps_per_phase && stn + t < ks; ++t) {
+                const double pf = hp[s.fir.poff[m] + t] * s.fir.epi_scale;
+                const double h = hd ? std::fma(hd[s.fir.poff[m] + t] * s.fir.epi_scale, s.fir.alpha[m], pf) : pf;
+                const int k = stn + t;
+                band[k * 8 + (n ^ (((k >> 1) & 1) << 2))] = h;
+            }
+        }
+    }
+    double* dptr = nullptr;
+    CUDA_OK(cudaMalloc(&dptr, tab.size() * sizeof(double)));
+    CUDA_OK(cudaMemcpy(dptr, tab.data(), tab.size() * sizeof(double), cudaMemcpyHostToDevice));
+    w.pd.bands.emplace(key, dptr);
+    return dptr;
+}
+
+// Tuning aid (SIGOPS_FIR_DBG=1): `launch` runs a FIR kernel once with per-block cycle counters ([nblocks][8]); the
+// counters summed over the blocks, per tile.
+std::array<double, 8> fir_cycles_per_tile(cudaStream_t stream, size_t nblocks, int64_t tiles_per_seg,
+                                          const std::function<void(long long*)>& launch) {
+    long long* dbg = nullptr;
+    CUDA_OK(cudaMalloc(&dbg, nblocks * 8 * sizeof(long long)));
+    CUDA_OK(cudaMemset(dbg, 0, nblocks * 8 * sizeof(long long)));
+    launch(dbg);
+    CUDA_OK(cudaStreamSynchronize(stream));
+    std::vector<long long> h(nblocks * 8);
+    CUDA_OK(cudaMemcpy(h.data(), dbg, h.size() * sizeof(long long), cudaMemcpyDeviceToHost));
+    cudaFree(dbg);
+    std::array<double, 8> sum{};
+    for (size_t b = 0; b < nblocks; ++b)
+        for (int k = 0; k < 8; ++k) sum[k] += (double)h[b * 8 + k];
+    const double per = 1.0 / ((double)nblocks * (double)tiles_per_seg);
+    for (double& v : sum) v *= per;
+    return sum;
+}
+
+// One launch with `smem` bytes of dynamic shared memory (opted in once per kernel, size and device).
+template <class... P, class... A>
+void launch_dyn_smem(void (*kernel)(P...), dim3 grid, int threads, size_t smem, cudaStream_t st, const A&... args) {
+    ensure_dyn_smem(kernel, smem);
+    kernel<<<grid, threads, smem, st>>>(args...);
+}
+
+void plan_map_stage(const Wave& w) {
+    const sigops_plan& p = w.p;
+    const sigops_stage& g = p.stages[w.si].st;
+    MapParams P{};
+    P.instrs = w.pd.instrs; P.bufrefs = w.d_refs; P.scalars = w.scalars; P.inst0 = w.inst0;
+    P.nbuf = w.nbuf; P.nscalars = w.nscal;
+    P.out_buf = g.out_buf; P.sumsq_slot = g.sumsq_slot; P.out_nch = p.bufs[g.out_buf].nchannels;
+    P.n_pieces = g.n_pieces;
+    // frames per block: four 2048-frame passes amortise the per-block set-up, unless that would
+    // leave the GPU with fewer than a few blocks per SM
+    int64_t subs = 0;
+    for (int k = 0; k < g.n_pieces; ++k)
+        subs += (p.pieces[g.piece_start + k].out_len + kMapSub - 1) / kMapSub * p.pieces[g.piece_start + k].ch_count;
+    P.passes = subs * w.ninst >= (int64_t)kMapPasses * w.sm_count * 8 ? kMapPasses : 1;
+    const int64_t per_block = (int64_t)kMapSub * P.passes;
+    int tiles = 0;
+    for (int k = 0; k < g.n_pieces; ++k) {
+        P.pieces[k] = p.pieces[g.piece_start + k];
+        P.tile_prefix[k] = tiles;
+        tiles += (int)((P.pieces[k].out_len + per_block - 1) / per_block);
+    }
+    P.tile_prefix[g.n_pieces] = tiles;
+    if (tiles == 0) return;
+    const size_t stack_map = p.max_stack ? (size_t)p.max_stack * kMapV * kMapThreads * sizeof(double) : 0;
+    if (stack_map > 16 * 1024) ensure_dyn_smem(k_map, stack_map);
+    for (int64_t i0 = 0; i0 < w.ninst; i0 += 65535) {
+        const int64_t ni = std::min<int64_t>(65535, w.ninst - i0);
+        MapParams Q = P;
+        Q.bufrefs = w.d_refs + i0 * w.nbuf;
+        Q.scalars = w.scalars + i0 * w.nscal;
+        dim3 grid(tiles, P.out_nch, (unsigned)ni);
+        w.add(KIND_MAP, [=](cudaStream_t st) { k_map<<<grid, kMapThreads, stack_map, st>>>(Q); });
+    }
+}
+
+// Tensor-map IIR kernel (k_iir_tmap.cuh; SIGOPS_NO_TMAP=1 switches it off): lanes = rows.  Needs every row of the
+// wave at base + row*stride for both buffers, enough rows to fill warps, and a filter that decays within a chunk
+// (WARM).  `tma`: the stage could take the per-lane TMA kernel.  Returns whether this one applies.
+bool plan_iir_tmap(const Wave& w, bool tma) {
+    const StageRT& s = w.p.stages[w.si];
+    const sigops_stage& g = s.st;
+    const int64_t rows = w.ninst * g.nchannels;
+    const bool f32 = s.iir.fast32;
+    const bool rowinv = tma && s.iir.tma_prog && s.iir.rowinv && !getenv("SIGOPS_NO_TMAP_LEAVES");
+    const int esz = f32 ? 4 : 8;
+    const int stage_cols = f32 ? 32 * kTmSubsPerStageF32 : (rowinv ? kTmSub * kTmSubsPerStageLv : kTmStageCols);
+    if (!((tma && s.iir.fast) || f32 || rowinv) || getenv("SIGOPS_NO_TMAP") || !iir_tmap_available() ||
+        !(rows % 32 == 0 || rows >= 256) || rows * 32 >= (int64_t(1) << 31) || g.n_out >= (int64_t(1) << 30))
+        return false;
+    char *bin = nullptr, *bout = nullptr;
+    int64_t sin_ = 0, sout = 0;
+    const int dtype = f32 ? SIGOPS_F32 : SIGOPS_F64;
+    const int64_t Wst = round_up(std::max<int64_t>(s.iir.W, 1), stage_cols);
+    if (!strided_matrix(w.refs, w.ninst, w.nbuf, s.iir.plain_buf, esz, dtype, &bin, &sin_) ||
+        !strided_matrix(w.refs, w.ninst, w.nbuf, g.out_buf, esz, dtype, &bout, &sout) || 2 * Wst > g.n_out)
+        return false;
+    const int64_t N = g.n_out, groups = (rows + 31) / 32;
+    const int nw = f32 ? kTmWarpsF32 : (rowinv ? kTmWarpsLv : kTmWarps);
+    const IirLaunch c = choose_tmap_chunking(N, rows, stage_cols, Wst, nw, rowinv, w.sm_count);
+    // A slowly decaying filter is better served by k_iir_tma's short chunks and carry pass.
+    // Both estimates are in lane-frames; a lane-frame takes about max(100, 0.82 * lanes per SM)
+    // cycles (measured: 210 with 256 lanes, 102 with 128), which makes them comparable.
+    auto frame_cycles = [](int lanes) { return std::max(100.0, 0.82 * lanes); };
+    const bool tmap_wins = c.cost * frame_cycles(32 * nw) <=
+                           choose_iir_chunking_flat(s, rows, w.sm_count).cost * frame_cycles(32 * kTmaWarps);
+    TensorMapBlob mi, mo;
+    // (a Float32 stage has no other fast kernel to fall back on: take this one whenever it applies)
+    if (!(c.L > Wst && (tmap_wins || f32 || rowinv) &&
+          iir_tmap_encode(&mi, bin, std::min<int64_t>(s.iir.plain_len, N), rows, sin_, esz, rowinv ? kTmSubsPerStageLv : 0) &&
+          iir_tmap_encode(&mo, bout, N, rows, sout, esz, rowinv ? kTmSubsPerStageLv : 0)))
+        return false;
+    IirTmapParams T{};
+    T.bufrefs = w.d_refs; T.scalars = w.scalars; T.nbuf = w.nbuf; T.nscalars = w.nscal;
+    T.out_buf = g.out_buf; T.sumsq_slot = g.sumsq_slot; T.nch = g.nchannels; T.nrows = rows;
+    T.N = N; T.L = c.L; T.Wc = Wst;
+    T.cpr = c.nchunks;
+    T.nunits = groups * T.cpr;
+    T.gain = g.gain;
+    T.scale = s.iir.scale[0];          // (applied one after the other, like the reference's nested maps)
+    T.scale2 = s.iir.scale[1];
+    if (rowinv) {
+        T.scale = T.scale2 = 1.0;
+        T.n_in_ops = (int)s.iir.rv_in.size();
+        T.n_ep_ops = (int)s.iir.rv_ep.size();
+        for (int j = 0; j < T.n_in_ops; ++j) T.ops[j] = s.iir.rv_in[j];
+        for (int j = 0; j < T.n_ep_ops; ++j) T.ops[kTmMaxLeafOps + j] = s.iir.rv_ep[j];
+    }
+    const double* tc = w.p.blob.data() + w.p.tables[g.coef_table].offset;
+    for (int j = 0; j < s.iir.M; ++j)
+        for (int k = 0; k < 5; ++k) T.coef[j][k] = tc[j * 5 + k];
+    const int M_ = s.iir.M;
+    const bool unitb = s.iir.unitb;
+    dim3 tgrid((unsigned)(rowinv ? T.cpr * ((groups + nw - 1) / nw) : (T.nunits + nw - 1) / nw));
+    if (getenv("SIGOPS_DEBUG"))
+        fprintf(stderr, "[sigops] IIR stage %zu: tensor-map%s rows=%lld N=%lld M=%d W=%lld L=%lld chunks/row=%lld blocks=%u\n", w.si,
+                f32 ? " (Float32)" : (rowinv ? " (fused row-invariant programs)" : ""),
+                (long long)rows, (long long)N, M_, (long long)s.iir.W, (long long)T.L, (long long)T.cpr, tgrid.x);
+    w.add(KIND_IIR_MAIN, [=](cudaStream_t st) { launch_iir_tmap(f32, M_, unitb, tgrid, st, T, &mi, &mo); });
+    return true;
+}
+
+// IIR: the tensor-map kernel, else per-lane TMA (with fused programs or plain; WARM or MAIN + CARRY + FIX), else
+// cp.async (Float64 rows that are not 16-byte aligned), else the generic program-carrying kernel.
+void plan_iir_stage(const Wave& w) {
+    const sigops_plan& p = w.p;
+    const StageRT& s = p.stages[w.si];
+    const sigops_stage& g = s.st;
+    if (g.n_out == 0) return;
+    const int64_t rows = w.ninst * g.nchannels;
+    // TMA path: fast-path stage whose every channel starts on a 16-byte boundary
+    bool tma = (s.iir.fast || s.iir.tma_prog) && rows_aligned(w.refs, w.ninst, w.nbuf, s.iir.plain_buf, false) &&
+               rows_aligned(w.refs, w.ninst, w.nbuf, g.out_buf, false);
+    if (plan_iir_tmap(w, tma)) return;
+    // (the program-carrying TMA kernel has no MAIN/FIX form: keep it to chunkings it can run)
+    IirLaunch c = tma ? choose_iir_chunking_flat(s, rows, w.sm_count, !s.iir.tma_prog) : choose_iir_chunking(s, rows, w.sm_count);
+    // the program-carrying TMA kernel only exists in the single-launch WARM form
+    bool tprog = tma && s.iir.tma_prog;
+    if (tprog && c.need_matrix) {
+        tma = tprog = false;
+        c = choose_iir_chunking(s, rows, w.sm_count);
+    }
+    IirParams P{};
+    P.instrs = w.pd.instrs; P.bufrefs = w.d_refs; P.scalars = w.scalars; P.inst0 = w.inst0;
+    P.nbuf = w.nbuf; P.nscalars = w.nscal;
+    P.out_buf = g.out_buf; P.sumsq_slot = g.sumsq_slot;
+    P.in_prog_start = g.in_prog_start; P.in_prog_len = g.in_prog_len;
+    P.epi_prog_start = g.epi_prog_start; P.epi_prog_len = g.epi_prog_len;
+    P.plain_in_buf = (s.iir.plain_in || tprog) ? s.iir.plain_buf : -1;
+    P.plain_in_len = s.iir.plain_len;
+    P.nch = g.nchannels; P.blocks_per_row = c.blocks_per_row;
+    P.N = g.n_out; P.L = c.L; P.Wc = c.Wc;
+    P.slots_per_row = tma ? c.nchunks : (int64_t)c.blocks_per_row * kIirThreads;
+    P.M = s.iir.M; P.gain = g.gain;
+    const double* t = p.blob.data() + p.tables[g.coef_table].offset;
+    for (int j = 0; j < s.iir.M; ++j)
+        for (int k = 0; k < 5; ++k) P.coef[j][k] = t[j * 5 + k];
+    const size_t nslots = (size_t)rows * P.slots_per_row;
+    const int S = 2 * s.iir.M;
+    P.state_zs = (double*)w.arena.take(nslots * S * sizeof(double));
+    P.state_in = (double*)w.arena.take(nslots * S * sizeof(double));
+    P.n_epi_scale = s.iir.n_scale;
+    P.epi_scale[0] = s.iir.scale[0]; P.epi_scale[1] = s.iir.scale[1];
+    P.carry_is_shift = c.need_matrix ? 0 : 1;
+    IirTmaParams Q{};
+    Q.base = P; Q.cpr = c.nchunks; Q.total_chunks = rows * c.nchunks;
+    if (tprog) {
+        Q.base.in_prog_start = s.iir.prog_in_start; Q.base.in_prog_len = s.iir.prog_in_len;
+        Q.base.n_epi_scale = 0; Q.base.epi_scale[0] = Q.base.epi_scale[1] = 1.0;
+    }
+    if (getenv("SIGOPS_DEBUG"))
+        fprintf(stderr, "[sigops] IIR stage %zu: %s rows=%lld N=%lld M=%d W=%lld L=%lld chunks/row=%lld Wc=%lld matrix=%d\n", w.si,
+                tma ? "tma" : (s.iir.fast ? "cp.async" : "generic"), (long long)rows, (long long)g.n_out, s.iir.M,
+                (long long)s.iir.W, (long long)c.L, (long long)c.nchunks, (long long)c.Wc, (int)c.need_matrix);
+    const int64_t tma_blocks = ((Q.total_chunks + 31) / 32 + kTmaWarps - 1) / kTmaWarps;
+    dim3 grid((unsigned)(tma ? tma_blocks : rows * c.blocks_per_row));
+    const bool warm = tma && !c.need_matrix;     // single self-contained launch
+    const size_t stack_iir = p.max_stack ? (size_t)p.max_stack * kIirV * kIirThreads * sizeof(double) : 0;
+    const int M_ = s.iir.M;
+    const bool unitb = s.iir.unitb, fast = s.iir.fast;
+    w.add(KIND_IIR_MAIN, [=](cudaStream_t st) {
+        if (warm) launch_iir_tma_any(LAUNCH_WARM, tprog, M_, unitb, grid, st, Q);
+        else if (tma) launch_iir_tma_any(LAUNCH_MAIN, false, M_, unitb, grid, st, Q);
+        else if (fast) launch_iir_cpasync(LAUNCH_MAIN, M_, unitb, grid, st, P);
+        else launch_iir_generic(LAUNCH_MAIN, M_, grid, stack_iir, st, P);
+    });
+    if (c.nchunks <= 1 || warm) return;
+    if (c.need_matrix) {
+        CarryParams C{};
+        C.state_zs = P.state_zs; C.state_in = P.state_in;
+        C.nrows = rows; C.slots_per_row = P.slots_per_row; C.nchunks = c.nchunks; C.M2 = S;
+        // L-step transition matrix: computed and uploaded once per (stage, chunk length) and device
+        const uint64_t akey = ((uint64_t)w.si << 40) ^ (uint64_t)c.L;
+        double*& dAL = w.pd.carry[akey];
+        if (!dAL) {
+            std::vector<double> AL = transition_matrix(P.coef, s.iir.M, c.L);
+            CUDA_OK(cudaMalloc(&dAL, AL.size() * sizeof(double)));
+            CUDA_OK(cudaMemcpy(dAL, AL.data(), AL.size() * sizeof(double), cudaMemcpyHostToDevice));
+        }
+        C.AL = dAL;
+        const unsigned cblocks = (unsigned)((rows + 3) / 4);        // one warp per row
+        w.add(KIND_IIR_CARRY, [=](cudaStream_t st) { k_iir_carry<<<cblocks, 128, 0, st>>>(C); });
+    }
+    w.add(KIND_IIR_FIX, [=](cudaStream_t st) {
+        if (tma) launch_iir_tma_any(LAUNCH_FIX, false, M_, unitb, grid, st, Q);
+        else if (fast) launch_iir_cpasync(LAUNCH_FIX, M_, unitb, grid, st, P);
+        else launch_iir_generic(LAUNCH_FIX, M_, grid, stack_iir, st, P);
+    });
+}
+
+// Tensor-map FIR kernel (k_fir_tmap.cuh; SIGOPS_NO_FIR_TMAP=1 switches it off): every row of the wave at base +
+// row*stride, more than 64 rows, band <= 64 positions, a tile's window inside the ring.  Returns whether it applies.
+bool plan_fir_tmap(const Wave& w, const FirParams& P) {
+    const StageRT& s = w.p.stages[w.si];
+    const sigops_stage& g = s.st;
+    const int64_t rows = P.nrows;
+    if (rows <= 64 || getenv("SIGOPS_NO_FIR_TMAP") || !iir_tmap_available() || rows >= (int64_t(1) << 31) ||
+        g.n_out >= (int64_t(1) << 31) || s.fir.in_len >= (int64_t(1) << 31))
+        return false;
+    // a group's band starts at its first window position; the helpers build it in blocks of 8 rows
+    const int ks = (int)round_up(s.fir.dpad + g.taps_per_phase, 8);
+    const int win_slots = (s.fir.pmax32 + 3 + 14) / 16 + 1;      // worst alignment of a tile's window (+ 3 positions read past it)
+    const bool has_d = P.dpfb != nullptr;
+    // periodic resamplers read the merged tap bands of a tile from the period tables: no banks in shared
+    // memory then, which buys one more ring slot
+    const double* bands_g = nullptr;
+    int period_tiles = 0;
+    if (s.fir.period > 0 && g.sumsq_slot < 0 && !getenv("SIGOPS_NO_FIR_BANDS") &&
+        (size_t)(s.fir.period / 8) * ks * 64 * (size_t)s.fir.n_epochs <= (size_t(96) << 20)) {
+        bands_g = period_bands(w, ks);
+        period_tiles = (int)(s.fir.period / kFmT);
+    }
+    const int64_t tabd = bands_g ? 0 : (int64_t)g.n_phases * g.taps_per_phase;
+    int nslot = kFtMaxSlots;
+    while (nslot > win_slots + 1 && fir_tm_smem_bytes(nslot, ks, (int)tabd, has_d) > kFirTmSmemLimit) --nslot;
+    char *bin = nullptr, *bout = nullptr;
+    int64_t sin_ = 0, sout = 0;
+    TensorMapBlob mi, mo;
+    if (!(ks <= kFtMaxKs && nslot >= win_slots + 1 && fir_tm_smem_bytes(nslot, ks, (int)tabd, has_d) <= kFirTmSmemLimit &&
+          strided_matrix(w.refs, w.ninst, w.nbuf, s.fir.in_buf, 8, SIGOPS_F64, &bin, &sin_) &&
+          strided_matrix(w.refs, w.ninst, w.nbuf, g.out_buf, 8, SIGOPS_F64, &bout, &sout) && s.fir.in_len >= 1 &&
+          tmap_encode_2d_f64(&mi, bin, s.fir.in_len, rows, sin_, kFtSlotPos, kFtRows) &&
+          tmap_encode_2d_f64(&mo, bout, g.n_out, rows, sout, 16, kFtRows / 2)))
+        return false;
+    FirTmParams T{};
+    T.scalars = w.scalars; T.nscalars = w.nscal; T.sumsq_slot = g.sumsq_slot; T.nch = g.nchannels;
+    T.nrows = rows; T.n_out = g.n_out; T.tapsper = g.taps_per_phase; T.ks = ks; T.nslot = nslot;
+    T.ntiles = (g.n_out + kFmT - 1) / kFmT;
+    T.pfb = P.pfb; T.dpfb = P.dpfb; T.xi0 = P.xi0; T.poff = w.pd.poff[w.si]; T.alpha = w.pd.alpha[w.si];
+    T.tab_doubles = (int)tabd;
+    T.bands_g = bands_g; T.period_tiles = period_tiles;
+    T.epoch_tiles = s.fir.epoch_tiles; T.n_epochs = (int)s.fir.n_epochs;
+    T.gain = s.fir.epi_scale;
+    if (const char* e = getenv("SIGOPS_FIR_EXP")) T.exp = atoi(e);
+    const int64_t groups = (rows + kFtRows - 1) / kFtRows;
+    if (groups > 65535) return false;
+    T.tiles_per_seg = choose_tiles_per_segment(T.ntiles, groups, w.sm_count);
+    const int64_t nseg = (T.ntiles + T.tiles_per_seg - 1) / T.tiles_per_seg;
+    const size_t smem = fir_tm_smem_bytes(nslot, ks, (int)tabd, has_d);
+    dim3 tgrid((unsigned)nseg, (unsigned)groups);
+    if (getenv("SIGOPS_DEBUG")) {
+        fprintf(stderr, "[sigops] FIR stage %zu: tensor-map rows=%lld n_out=%lld taps=%d ks=%d slots=%d (window %d) grid=%lldx%lld tiles/seg=%lld smem=%zu gain=%g period=%lld outputs%s\n",
+                w.si, (long long)rows, (long long)g.n_out, T.tapsper, ks, nslot, win_slots, (long long)nseg, (long long)groups,
+                (long long)T.tiles_per_seg, smem, T.gain, (long long)s.fir.period, bands_g ? " (tap bands from the period tables)" : "");
+        if (bands_g) fprintf(stderr, "[sigops]   %lld epochs of %lld tiles\n", (long long)s.fir.n_epochs, (long long)s.fir.epoch_tiles);
+    }
+    if (getenv("SIGOPS_FIR_DBG")) {
+        const auto c = fir_cycles_per_tile(w.stream, (size_t)nseg * groups, T.tiles_per_seg, [&](long long* dbg) {
+            FirTmParams D = T;
+            D.dbg = dbg;
+            launch_dyn_smem(k_fir_tmap<false, true>, tgrid, kFtThreads, smem, w.stream, D, *(const CUtensorMap*)&mi,
+                            *(const CUtensorMap*)&mo);
+        });
+        fprintf(stderr, "[sigops] FIR tmap cycles/tile  compute: set-up %.0f (of it wait_taps %.0f) staging %.0f (of it wait_stg %.0f) total %.0f | helper: wait_done %.0f build %.0f\n",
+                c[1], c[0], c[6], c[2], c[3], c[4], c[5]);
+    }
+    const auto kernel = g.sumsq_slot >= 0 ? k_fir_tmap<true> : k_fir_tmap<false>;
+    w.add(KIND_FIR, [=](cudaStream_t st) {
+        launch_dyn_smem(kernel, tgrid, kFtThreads, smem, st, T, *(const CUtensorMap*)&mi, *(const CUtensorMap*)&mo);
+    });
+    return true;
+}
+
+// Per-row tensor-core FIR kernel (k_fir_mma.cuh: 8 compute warps, RB/16 row fragments each).  Returns whether it applies.
+bool plan_fir_mma(const Wave& w, const FirParams& P) {
+    const StageRT& s = w.p.stages[w.si];
+    const sigops_stage& g = s.st;
+    const int64_t rows = P.nrows;
+    FirMmaParams Q{};
+    Q.bufrefs = w.d_refs; Q.scalars = w.scalars; Q.nbuf = w.nbuf; Q.nscalars = w.nscal;
+    Q.in_buf = s.fir.in_buf; Q.out_buf = g.out_buf; Q.sumsq_slot = g.sumsq_slot;
+    Q.in_len = s.fir.in_len; Q.nch = g.nchannels; Q.nrows = rows; Q.n_out = g.n_out;
+    Q.tapsper = g.taps_per_phase;
+    Q.ks = (int)round_up(s.fir.dpad + g.taps_per_phase, 4);
+    Q.ring = s.fir.ring32;
+    Q.pitch = Q.ring + ((4 - Q.ring % 16) + 16) % 16;
+    Q.pfb = P.pfb; Q.dpfb = P.dpfb; Q.xi0 = P.xi0; Q.poff = w.pd.poff[w.si]; Q.alpha = w.pd.alpha[w.si];
+    Q.ntiles = (g.n_out + kFmT - 1) / kFmT;
+    Q.gain = s.fir.epi_scale;
+    // both polyphase banks ride along in shared memory when that leaves the ring its room
+    const int64_t tabd = (int64_t)g.n_phases * g.taps_per_phase;
+    const size_t tab_bytes = (size_t)tabd * 8 * (P.dpfb ? 2 : 1);
+    Q.tab_doubles = (int)tabd;
+    if (tab_bytes > 48 * 1024) return false;      // banks too large to ride along in shared memory
+    auto smem_for = [&](int RBx) {
+        return (size_t)RBx * Q.pitch * 8 + (size_t)2 * 4 * Q.ks * kFmHbPitch * 8 + tab_bytes;
+    };
+    // rows per block RB: as many as the batch fills and shared memory holds
+    int RB = rows > 64 ? 128 : (rows > 32 ? 64 : 32);
+    while (RB > 32 && smem_for(RB) > kFirMmaSmemLimit) RB >>= 1;
+    const int64_t groups = (rows + RB - 1) / RB;
+    if (smem_for(RB) > kFirMmaSmemLimit || groups > 65535) return false;
+    Q.tiles_per_seg = choose_tiles_per_segment(Q.ntiles, groups, w.sm_count);
+    const int64_t nseg = (Q.ntiles + Q.tiles_per_seg - 1) / Q.tiles_per_seg;
+    const size_t smem = smem_for(RB);
+    dim3 grid((unsigned)nseg, (unsigned)groups);
+    if (getenv("SIGOPS_DEBUG"))
+        fprintf(stderr, "[sigops] FIR stage %zu: mma rows=%lld n_out=%lld taps=%d ks=%d ring=%d pitch=%d rows/block=%d grid=%lldx%lld tiles/seg=%lld smem=%zu\n",
+                w.si, (long long)rows, (long long)g.n_out, Q.tapsper, Q.ks, Q.ring, Q.pitch, RB, (long long)nseg,
+                (long long)groups, (long long)Q.tiles_per_seg, smem);
+    if (getenv("SIGOPS_FIR_DBG")) {
+        const auto c = fir_cycles_per_tile(w.stream, (size_t)nseg * groups, Q.tiles_per_seg, [&](long long* dbg) {
+            FirMmaParams D = Q;
+            D.dbg = dbg;
+            if (RB == 128) launch_dyn_smem(k_fir_mma<8, 2, false>, grid, 16 * 32, smem, w.stream, D);
+        });
+        fprintf(stderr, "[sigops] FIR cycles/tile  aux: wait_done %.0f extend %.0f taps %.0f | compute: wait_taps %.0f wait_data %.0f dmma %.0f store %.0f\n",
+                c[0], c[1], c[2], c[3], c[4], c[5], c[6]);
+    }
+    const bool ssq = Q.sumsq_slot >= 0;
+    const auto kernel = RB == 128 ? (ssq ? k_fir_mma<8, 2, true> : k_fir_mma<8, 2, false>)
+                      : RB == 64  ? (ssq ? k_fir_mma<4, 2, true> : k_fir_mma<4, 2, false>)
+                                  : (ssq ? k_fir_mma<2, 2, true> : k_fir_mma<2, 2, false>);
+    w.add(KIND_FIR, [=](cudaStream_t st) { launch_dyn_smem(kernel, grid, 16 * 32, smem, st, Q); });
+    return true;
+}
+
+// FIR: the tensor-core kernels for plain Float64 rows on 16-byte boundaries with no epilogue or a constant gain
+// (k_fir_tmap, else k_fir_mma), else the scalar-FMA kernel k_fir.
+void plan_fir_stage(const Wave& w) {
+    const sigops_plan& p = w.p;
+    const StageRT& s = p.stages[w.si];
+    const sigops_stage& g = s.st;
+    if (g.n_out == 0) return;
+    const int64_t rows = w.ninst * g.nchannels;
+    FirParams P{};
+    P.instrs = w.pd.instrs; P.bufrefs = w.d_refs; P.scalars = w.scalars; P.inst0 = w.inst0;
+    P.nbuf = w.nbuf; P.nscalars = w.nscal;
+    P.out_buf = g.out_buf; P.sumsq_slot = g.sumsq_slot;
+    P.in_buf = s.fir.in_buf; P.in_len = s.fir.in_len;
+    P.epi_prog_start = g.epi_prog_start; P.epi_prog_len = g.epi_prog_len;
+    P.nch = g.nchannels; P.nrows = rows; P.n_out = g.n_out;
+    P.tapsper = g.taps_per_phase;
+    P.pfb = w.pd.blob + p.tables[g.pfb_table].offset;
+    P.dpfb = g.dpfb_table >= 0 ? w.pd.blob + p.tables[g.dpfb_table].offset : nullptr;
+    P.xi0 = w.pd.xi0[w.si]; P.phi = w.pd.phi[w.si];
+    const bool mma = s.fir.epi_const && !getenv("SIGOPS_NO_FIR_MMA") &&
+                     p.bufs[s.fir.in_buf].dtype == SIGOPS_F64 && p.bufs[g.out_buf].dtype == SIGOPS_F64 &&
+                     rows_aligned(w.refs, w.ninst, w.nbuf, s.fir.in_buf, true) && rows_aligned(w.refs, w.ninst, w.nbuf, g.out_buf, true);
+    if (mma && (plan_fir_tmap(w, P) || plan_fir_mma(w, P))) return;
+    // rows per thread: as many as fit in shared memory, but no more than the batch can fill
+    int G = 4;
+    while (G > 1 && (fir_smem_bytes(s.fir, g.taps_per_phase, G, p.max_stack) > kFirSmemLimit || rows <= 16 * G)) G >>= 1;
+    const FirGeom geo = fir_geometry(s.fir, g.taps_per_phase, G, p.max_stack);
+    P.hbase = geo.hbase; P.tpad = geo.tpad; P.xpitch = geo.xpitch;
+    const size_t smem = geo.smem;
+    const int64_t tiles = (g.n_out + kFirT - 1) / kFirT;
+    const int64_t groups = (rows + 32 * G - 1) / (32 * G);
+    if (groups > 65535) fail(SIGOPS_ERR_UNSUPPORTED, "FIR stage over more than %d rows per wave", 65535 * 32 * G);
+    dim3 grid((unsigned)tiles, (unsigned)groups);
+    if (getenv("SIGOPS_DEBUG"))
+        fprintf(stderr, "[sigops] FIR stage %zu: scalar rows=%lld n_out=%lld taps=%d G=%d tiles=%lld smem=%zu\n", w.si,
+                (long long)rows, (long long)g.n_out, g.taps_per_phase, G, (long long)tiles, smem);
+    const auto kernel = G == 4 ? k_fir<4, 8> : (G == 2 ? k_fir<2, 8> : k_fir<1, 8>);
+    w.add(KIND_FIR, [=](cudaStream_t st) { launch_dyn_smem(kernel, grid, 256, smem, st, P); });
 }
 
 // Enqueue every stage of the plan for one wave. Returns kernels launched.
@@ -1002,519 +1501,14 @@ int64_t enqueue_wave(sigops_plan& p, int di, Slot& slot, cudaStream_t stream, co
     drop_graph();
     slot.cache_launches.clear();
     slot.cache_plan = 0;
-    auto add = [&](int kind, std::function<void(cudaStream_t)> fn) { slot.cache_launches.push_back({kind, std::move(fn)}); };
-
-    const size_t stack_map = p.max_stack ? (size_t)p.max_stack * kMapV * kMapThreads * sizeof(double) : 0;
-    const size_t stack_iir = p.max_stack ? (size_t)p.max_stack * kIirV * kIirThreads * sizeof(double) : 0;
-
-    for (size_t si = 0; si < p.stages.size(); ++si) {
-        const StageRT& s = p.stages[si];
-        const sigops_stage& g = s.st;
-        if (g.kind == SIGOPS_STAGE_MAP) {
-            MapParams P{};
-            P.instrs = pd.instrs; P.bufrefs = d_refs; P.scalars = scalars; P.inst0 = io.inst0;
-            P.nbuf = nbuf; P.nscalars = nscal;
-            P.out_buf = g.out_buf; P.sumsq_slot = g.sumsq_slot; P.out_nch = p.bufs[g.out_buf].nchannels;
-            P.n_pieces = g.n_pieces;
-            // frames per block: four 2048-frame passes amortise the per-block set-up, unless that would
-            // leave the GPU with fewer than a few blocks per SM
-            int64_t subs = 0;
-            for (int k = 0; k < g.n_pieces; ++k)
-                subs += (p.pieces[g.piece_start + k].out_len + kMapSub - 1) / kMapSub * p.pieces[g.piece_start + k].ch_count;
-            P.passes = subs * ninst >= (int64_t)kMapPasses * dev.sm_count * 8 ? kMapPasses : 1;
-            const int64_t per_block = (int64_t)kMapSub * P.passes;
-            int tiles = 0;
-            for (int k = 0; k < g.n_pieces; ++k) {
-                P.pieces[k] = p.pieces[g.piece_start + k];
-                P.tile_prefix[k] = tiles;
-                tiles += (int)((P.pieces[k].out_len + per_block - 1) / per_block);
-            }
-            P.tile_prefix[g.n_pieces] = tiles;
-            if (tiles == 0) continue;
-            if (stack_map > 16 * 1024) ensure_dyn_smem(k_map, stack_map);
-            for (int64_t i0 = 0; i0 < ninst; i0 += 65535) {
-                const int64_t ni = std::min<int64_t>(65535, ninst - i0);
-                MapParams Q = P;
-                Q.bufrefs = d_refs + i0 * nbuf;
-                Q.scalars = scalars + i0 * nscal;
-                dim3 grid(tiles, P.out_nch, (unsigned)ni);
-                add(KIND_MAP, [=](cudaStream_t st) { k_map<<<grid, kMapThreads, stack_map, st>>>(Q); });
-            }
-        } else if (g.kind == SIGOPS_STAGE_IIR) {
-            if (g.n_out == 0) continue;
-            const int64_t rows = ninst * g.nchannels;
-            // TMA path: fast-path stage whose every channel starts on a 16-byte boundary
-            bool tma = (s.iir.fast || s.iir.tma_prog) && !getenv("SIGOPS_NO_TMA");
-            if (tma) {
-                for (int64_t i = 0; i < ninst && tma; ++i)
-                    for (int b : {s.iir.plain_buf, g.out_buf}) {
-                        const BufRef& rb = ((const BufRef*)slot.last_table.data())[i * nbuf + b];
-                        if (((uintptr_t)rb.ptr & 15) || (rb.nch > 1 && (rb.ld & 1))) tma = false;
-                    }
-            }
-            // Tensor-map path (k_iir_tmap.cuh; SIGOPS_NO_TMAP=1 switches it off):
-            // lanes = rows.  Needs every row of the wave at base + row*stride for both buffers (one batch
-            // tensor, or the library's own staging), enough rows to fill warps, and a filter that decays
-            // within a chunk (WARM).
-            const bool f32 = s.iir.fast32;
-            const bool rowinv_pre = tma && s.iir.tma_prog && s.iir.rowinv && !getenv("SIGOPS_NO_TMAP_LEAVES");
-            const int esz = f32 ? 4 : 8;
-            const int stage_cols = f32 ? 32 * kTmSubsPerStageF32 : (rowinv_pre ? kTmSub * kTmSubsPerStageLv : kTmStageCols);
-            const bool rowinv = rowinv_pre;
-            if (((tma && s.iir.fast && !s.iir.tma_prog) || f32 || rowinv) && !getenv("SIGOPS_NO_TMAP") && iir_tmap_available() &&
-                (rows % 32 == 0 || rows >= 256) && rows * 32 < (int64_t(1) << 31) && g.n_out < (int64_t(1) << 30)) {
-                const BufRef* refs = (const BufRef*)slot.last_table.data();
-                auto uniform = [&](int b, char*& base, int64_t& stride) {
-                    const BufRef& r0 = refs[b];
-                    base = (char*)r0.ptr;
-                    stride = r0.ld * esz;
-                    const int want = f32 ? SIGOPS_F32 : SIGOPS_F64;
-                    if ((stride & 15) || ((uintptr_t)base & 15) || r0.dtype != want) return false;
-                    for (int64_t i = 0; i < ninst; ++i) {
-                        const BufRef& rb = refs[i * nbuf + b];
-                        if (rb.ld != r0.ld || rb.nch != r0.nch || rb.dtype != want ||
-                            (char*)rb.ptr != base + (int64_t)i * r0.nch * stride)
-                            return false;
-                    }
-                    return true;
-                };
-                char *bin = nullptr, *bout = nullptr;
-                int64_t sin_ = 0, sout = 0;
-                const int64_t Wst = round_up(std::max<int64_t>(s.iir.W, 1), stage_cols);
-                if (uniform(s.iir.plain_buf, bin, sin_) && uniform(g.out_buf, bout, sout) && 2 * Wst <= g.n_out) {
-                    // chunk length: whole waves of one block (8 warps = 8 units) per SM; a unit walks L + Wc frames
-                    const int64_t N = g.n_out, groups = (rows + 31) / 32;
-                    const int nw = f32 ? kTmWarpsF32 : (rowinv ? kTmWarpsLv : kTmWarps);
-                    const int64_t jmax = std::max<int64_t>(1, (N + stage_cols - 1) / stage_cols);
-                    double best = 1e300;
-                    int64_t bestL = 0;
-                    for (int64_t j = Wst / stage_cols + 1; j <= jmax; j += std::max<int64_t>(1, jmax / 4096)) {
-                        const int64_t L = j * stage_cols, cpr = (N + L - 1) / L;
-                        // (fused programs: the warps of a block share a chunk, see k_iir_tmap)
-                        const int64_t blocks = rowinv ? cpr * ((groups + nw - 1) / nw) : (groups * cpr + nw - 1) / nw;
-                        const int64_t waves = (blocks + dev.sm_count - 1) / dev.sm_count;
-                        const double cost = (double)waves * ((double)L + (cpr > 1 ? (double)Wst : 0.0) + 600.0);
-                        if (cost < best) { best = cost; bestL = L; }
-                    }
-                    if (const char* e = getenv("SIGOPS_IIR_L")) bestL = std::max<int64_t>(Wst + stage_cols, round_up(atoll(e), stage_cols));
-                    // A slowly decaying filter is better served by k_iir_tma's short chunks and carry pass.
-                    // Both estimates are in lane-frames; a lane-frame takes about max(100, 0.82 * lanes per SM)
-                    // cycles (measured: 210 with 256 lanes, 102 with 128), which makes them comparable.
-                    auto frame_cycles = [](int lanes) { return std::max(100.0, 0.82 * lanes); };
-                    const bool tmap_wins = best * frame_cycles(32 * nw) <=
-                                           choose_iir_chunking_flat(s, rows, dev.sm_count).cost * frame_cycles(32 * kTmaWarps);
-                    TensorMapBlob mi, mo;
-                    // (a Float32 stage has no other fast kernel to fall back on: take this one whenever it applies)
-                    if (bestL > Wst && (tmap_wins || f32 || rowinv) &&
-                        iir_tmap_encode(&mi, bin, std::min<int64_t>(s.iir.plain_len, N), rows, sin_, esz, rowinv ? kTmSubsPerStageLv : 0) &&
-                        iir_tmap_encode(&mo, bout, N, rows, sout, esz, rowinv ? kTmSubsPerStageLv : 0)) {
-                        IirTmapParams T{};
-                        T.bufrefs = d_refs; T.scalars = scalars; T.nbuf = nbuf; T.nscalars = nscal;
-                        T.out_buf = g.out_buf; T.sumsq_slot = g.sumsq_slot; T.nch = g.nchannels; T.nrows = rows;
-                        T.N = N; T.L = bestL; T.Wc = Wst;
-                        T.cpr = (N + bestL - 1) / bestL;
-                        T.nunits = groups * T.cpr;
-                        T.gain = g.gain;
-                        T.scale = s.iir.scale[0];          // (applied one after the other, like the reference's nested maps)
-                        T.scale2 = s.iir.scale[1];
-                        if (rowinv) {
-                            T.scale = T.scale2 = 1.0;
-                            T.n_in_ops = (int)s.iir.rv_in.size();
-                            T.n_ep_ops = (int)s.iir.rv_ep.size();
-                            for (int j = 0; j < T.n_in_ops; ++j) T.ops[j] = s.iir.rv_in[j];
-                            for (int j = 0; j < T.n_ep_ops; ++j) T.ops[kTmMaxLeafOps + j] = s.iir.rv_ep[j];
-                        }
-                        const double* tc = p.blob.data() + p.tables[g.coef_table].offset;
-                        for (int j = 0; j < s.iir.M; ++j)
-                            for (int k = 0; k < 5; ++k) T.coef[j][k] = tc[j * 5 + k];
-                        const int M_ = s.iir.M;
-                        const bool unitb = s.iir.unitb;
-                        dim3 tgrid((unsigned)(rowinv ? T.cpr * ((groups + nw - 1) / nw) : (T.nunits + nw - 1) / nw));
-                        if (getenv("SIGOPS_DEBUG"))
-                            fprintf(stderr, "[sigops] IIR stage %zu: tensor-map%s rows=%lld N=%lld M=%d W=%lld L=%lld chunks/row=%lld blocks=%u\n", si,
-                                    f32 ? " (Float32)" : (rowinv ? " (fused row-invariant programs)" : ""),
-                                    (long long)rows, (long long)N, M_, (long long)s.iir.W, (long long)T.L, (long long)T.cpr, tgrid.x);
-                        add(KIND_IIR_MAIN, [=](cudaStream_t st) { launch_iir_tmap(f32, M_, unitb, tgrid, st, T, &mi, &mo); });
-                        continue;
-                    }
-                }
-            }
-            // (the program-carrying TMA kernel has no MAIN/FIX form: keep it to chunkings it can run)
-            IirLaunch c = tma ? choose_iir_chunking_flat(s, rows, dev.sm_count, !s.iir.tma_prog) : choose_iir_chunking(s, rows, dev.sm_count);
-            // the program-carrying TMA kernel only exists in the single-launch WARM form
-            const bool tprog = tma && s.iir.tma_prog;
-            if (tprog && c.need_matrix) {
-                tma = false;
-                c = choose_iir_chunking(s, rows, dev.sm_count);
-            }
-            IirParams P{};
-            P.instrs = pd.instrs; P.bufrefs = d_refs; P.scalars = scalars; P.inst0 = io.inst0;
-            P.nbuf = nbuf; P.nscalars = nscal;
-            P.out_buf = g.out_buf; P.sumsq_slot = g.sumsq_slot;
-            P.in_prog_start = g.in_prog_start; P.in_prog_len = g.in_prog_len;
-            P.epi_prog_start = g.epi_prog_start; P.epi_prog_len = g.epi_prog_len;
-            P.plain_in_buf = (s.iir.plain_in || (tma && s.iir.tma_prog)) ? s.iir.plain_buf : -1;
-            P.plain_in_len = s.iir.plain_len;
-            P.nch = g.nchannels; P.blocks_per_row = c.blocks_per_row;
-            P.N = g.n_out; P.L = c.L; P.Wc = c.Wc;
-            P.slots_per_row = tma ? c.nchunks : (int64_t)c.blocks_per_row * kIirThreads;
-            P.M = s.iir.M; P.gain = g.gain;
-            const double* t = p.blob.data() + p.tables[g.coef_table].offset;
-            for (int j = 0; j < s.iir.M; ++j)
-                for (int k = 0; k < 5; ++k) P.coef[j][k] = t[j * 5 + k];
-            const size_t nslots = (size_t)rows * P.slots_per_row;
-            const int S = 2 * s.iir.M;
-            P.state_zs = (double*)slot.arena.take(nslots * S * sizeof(double));
-            P.state_in = (double*)slot.arena.take(nslots * S * sizeof(double));
-            P.n_epi_scale = s.iir.n_scale;
-            P.epi_scale[0] = s.iir.scale[0]; P.epi_scale[1] = s.iir.scale[1];
-            P.carry_is_shift = c.need_matrix ? 0 : 1;
-            IirTmaParams Q{};
-            Q.base = P; Q.cpr = c.nchunks; Q.total_chunks = rows * c.nchunks;
-            if (tma && s.iir.tma_prog) {
-                Q.base.in_prog_start = s.iir.prog_in_start; Q.base.in_prog_len = s.iir.prog_in_len;
-                Q.base.n_epi_scale = 0; Q.base.epi_scale[0] = Q.base.epi_scale[1] = 1.0;
-            }
-            if (getenv("SIGOPS_DEBUG"))
-                fprintf(stderr, "[sigops] IIR stage %zu: %s rows=%lld N=%lld M=%d W=%lld L=%lld chunks/row=%lld Wc=%lld matrix=%d\n", si,
-                        tma ? "tma" : (s.iir.fast ? "cp.async" : "generic"), (long long)rows, (long long)g.n_out, s.iir.M,
-                        (long long)s.iir.W, (long long)c.L, (long long)c.nchunks, (long long)c.Wc, (int)c.need_matrix);
-            const int64_t tma_blocks = ((Q.total_chunks + 31) / 32 + kTmaWarps - 1) / kTmaWarps;
-            dim3 grid((unsigned)(tma ? tma_blocks : rows * c.blocks_per_row));
-            const bool warm = tma && !c.need_matrix;     // single self-contained launch
-            {
-                const int M_ = s.iir.M;
-                const bool unitb = s.iir.unitb, fast = s.iir.fast;
-                add(KIND_IIR_MAIN, [=](cudaStream_t st) {
-                    if (warm) launch_iir_tma_any(LAUNCH_WARM, tprog, M_, unitb, grid, st, Q);
-                    else if (tma) launch_iir_tma_any(LAUNCH_MAIN, false, M_, unitb, grid, st, Q);
-                    else if (fast) launch_iir_cpasync(LAUNCH_MAIN, M_, unitb, grid, st, P);
-                    else launch_iir_generic(LAUNCH_MAIN, M_, grid, stack_iir, st, P);
-                });
-            }
-            if (c.nchunks > 1 && !warm) {
-                if (c.need_matrix) {
-                    CarryParams C{};
-                    C.state_zs = P.state_zs; C.state_in = P.state_in;
-                    C.nrows = rows; C.slots_per_row = P.slots_per_row; C.nchunks = c.nchunks; C.M2 = S;
-                    double cc[kIirMaxSections][5];
-                    for (int j = 0; j < s.iir.M; ++j)
-                        for (int k = 0; k < 5; ++k) cc[j][k] = P.coef[j][k];
-                    // L-step transition matrix: computed and uploaded once per (stage, chunk length) and device
-                    const uint64_t akey = ((uint64_t)si << 40) ^ (uint64_t)c.L;
-                    double*& dAL = pd.carry[akey];
-                    if (!dAL) {
-                        std::vector<double> AL = transition_matrix(cc, s.iir.M, c.L);
-                        CUDA_OK(cudaMalloc(&dAL, AL.size() * sizeof(double)));
-                        CUDA_OK(cudaMemcpy(dAL, AL.data(), AL.size() * sizeof(double), cudaMemcpyHostToDevice));
-                    }
-                    C.AL = dAL;
-                    const unsigned cblocks = (unsigned)((rows + 3) / 4);        // one warp per row
-                    add(KIND_IIR_CARRY, [=](cudaStream_t st) { k_iir_carry<<<cblocks, 128, 0, st>>>(C); });
-                }
-                {
-                    const int M_ = s.iir.M;
-                    const bool unitb = s.iir.unitb, fast = s.iir.fast;
-                    add(KIND_IIR_FIX, [=](cudaStream_t st) {
-                        if (tma) launch_iir_tma_any(LAUNCH_FIX, false, M_, unitb, grid, st, Q);
-                        else if (fast) launch_iir_cpasync(LAUNCH_FIX, M_, unitb, grid, st, P);
-                        else launch_iir_generic(LAUNCH_FIX, M_, grid, stack_iir, st, P);
-                    });
-                }
-            }
-        } else {
-            if (g.n_out == 0) continue;
-            const int64_t rows = ninst * g.nchannels;
-            FirParams P{};
-            P.instrs = pd.instrs; P.bufrefs = d_refs; P.scalars = scalars; P.inst0 = io.inst0;
-            P.nbuf = nbuf; P.nscalars = nscal;
-            P.out_buf = g.out_buf; P.sumsq_slot = g.sumsq_slot;
-            P.in_buf = s.fir.in_buf; P.in_len = s.fir.in_len;
-            P.epi_prog_start = g.epi_prog_start; P.epi_prog_len = g.epi_prog_len;
-            P.nch = g.nchannels; P.nrows = rows; P.n_out = g.n_out;
-            P.tapsper = g.taps_per_phase;
-            P.pfb = pd.blob + p.tables[g.pfb_table].offset;
-            P.dpfb = g.dpfb_table >= 0 ? pd.blob + p.tables[g.dpfb_table].offset : nullptr;
-            P.xi0 = pd.xi0[si]; P.phi = pd.phi[si];
-            // Tensor-core paths: plain Float64 rows on 16-byte boundaries, epilogue = none or a constant gain
-            bool mma = s.fir.epi_const && !getenv("SIGOPS_NO_FIR_MMA") &&
-                       p.bufs[s.fir.in_buf].dtype == SIGOPS_F64 && p.bufs[g.out_buf].dtype == SIGOPS_F64;
-            for (int64_t i = 0; i < ninst && mma; ++i)
-                for (int b : {s.fir.in_buf, (int)g.out_buf}) {
-                    const BufRef& rb = ((const BufRef*)slot.last_table.data())[i * nbuf + b];
-                    if (((uintptr_t)rb.ptr & 15) || (rb.nch > 1 && (rb.ld & 1)) || rb.dtype != SIGOPS_F64) mma = false;
-                }
-            const int64_t tabd_ = (int64_t)g.n_phases * g.taps_per_phase;
-            // Tensor-map kernel (k_fir_tmap.cuh): every row of the wave at base + row*stride, more than 64 rows,
-            // band <= 64 positions, a tile's window inside the ring
-            if (mma && rows > 64 && !getenv("SIGOPS_NO_FIR_TMAP") && iir_tmap_available() && rows < (int64_t(1) << 31) &&
-                g.n_out < (int64_t(1) << 31) && s.fir.in_len < (int64_t(1) << 31)) {
-                const BufRef* refs = (const BufRef*)slot.last_table.data();
-                auto uniform = [&](int b, char*& base, int64_t& stride) {
-                    const BufRef& r0 = refs[b];
-                    base = (char*)r0.ptr;
-                    stride = r0.ld * 8;
-                    if ((stride & 15) || ((uintptr_t)base & 15)) return false;
-                    for (int64_t i = 0; i < ninst; ++i) {
-                        const BufRef& rb = refs[i * nbuf + b];
-                        if (rb.ld != r0.ld || rb.nch != r0.nch || (char*)rb.ptr != base + (int64_t)i * r0.nch * stride) return false;
-                    }
-                    return true;
-                };
-                char *bin = nullptr, *bout = nullptr;
-                int64_t sin_ = 0, sout = 0;
-                // a group's band starts at its first window position; the helpers build it in blocks of 8 rows
-                const int ks = (int)round_up(s.fir.dpad + g.taps_per_phase, 8);
-                const int win_slots = (s.fir.pmax32 + 3 + 14) / 16 + 1;      // worst alignment of a tile's window (+ 3 positions read past it)
-                int nslot = kFtMaxSlots;
-                const bool has_d = P.dpfb != nullptr;
-                while (nslot > win_slots + 1 && fir_tm_smem_bytes(nslot, ks, (int)tabd_, has_d) > kFirTmSmemLimit) --nslot;
-                if (const char* e = getenv("SIGOPS_FIR_NSLOT")) nslot = std::max(win_slots + 1, std::min(kFtMaxSlots, atoi(e)));
-                // periodic resamplers: merged tap bands of one period, built once per plan and device ([tile][4 groups][ks][8],
-                // columns XOR-swizzled like the helpers write them, the constant-gain epilogue folded in); no banks in shared
-                // memory then, which buys one more ring slot
-                const double* bands_g = nullptr;
-                int period_tiles = 0;
-                if (s.fir.period > 0 && g.sumsq_slot < 0 && !getenv("SIGOPS_NO_FIR_BANDS") &&
-                    (size_t)(s.fir.period / 8) * ks * 64 * (size_t)s.fir.n_epochs <= (size_t(96) << 20)) {
-                    const uint64_t key = ((uint64_t)si << 16) | (uint64_t)ks;
-                    auto it = pd.bands.find(key);
-                    if (it == pd.bands.end()) {
-                        const int64_t Pp = s.fir.period;
-                        const double* hp = p.blob.data() + p.tables[g.pfb_table].offset;
-                        const double* hd = g.dpfb_table >= 0 ? p.blob.data() + p.tables[g.dpfb_table].offset : nullptr;
-                        const size_t per_epoch = (size_t)(Pp / 8) * ks * 8;
-                        std::vector<double> tab(per_epoch * (size_t)s.fir.n_epochs, 0.0);
-                        for (int64_t e = 0; e < s.fir.n_epochs; ++e) {
-                            const int64_t start = e * s.fir.epoch_tiles * kFmT;          // the epoch's own first period
-                            for (int64_t q = 0; q < Pp; ++q) {
-                                const int64_t m = start + q, m0 = m & ~int64_t(7);
-                                const int n = (int)(m - m0), stn = (int)(s.fir.xi0[m] - s.fir.xi0[m0]);
-                                double* band = tab.data() + per_epoch * (size_t)e + (size_t)((q & ~int64_t(7)) / 8) * ks * 8;
-                                for (int t = 0; t < g.taps_per_phase && stn + t < ks; ++t) {
-                                    const double pf = hp[s.fir.poff[m] + t] * s.fir.epi_scale;
-                                    const double h = hd ? std::fma(hd[s.fir.poff[m] + t] * s.fir.epi_scale, s.fir.alpha[m], pf) : pf;
-                                    const int k = stn + t;
-                                    band[k * 8 + (n ^ (((k >> 1) & 1) << 2))] = h;
-                                }
-                            }
-                        }
-                        double* dptr = nullptr;
-                        CUDA_OK(cudaMalloc(&dptr, tab.size() * sizeof(double)));
-                        CUDA_OK(cudaMemcpy(dptr, tab.data(), tab.size() * sizeof(double), cudaMemcpyHostToDevice));
-                        it = pd.bands.emplace(key, dptr).first;
-                    }
-                    bands_g = it->second;
-                    period_tiles = (int)(s.fir.period / kFmT);
-                }
-                const int64_t tabd_eff = bands_g ? 0 : tabd_;
-                if (bands_g) {
-                    nslot = kFtMaxSlots;
-                    while (nslot > win_slots + 1 && fir_tm_smem_bytes(nslot, ks, 0, has_d) > kFirTmSmemLimit) --nslot;
-                    if (const char* e = getenv("SIGOPS_FIR_NSLOT")) nslot = std::max(win_slots + 1, std::min(kFtMaxSlots, atoi(e)));
-                }
-                TensorMapBlob mi, mo;
-                if (ks <= kFtMaxKs && nslot >= win_slots + 1 && fir_tm_smem_bytes(nslot, ks, (int)tabd_eff, has_d) <= kFirTmSmemLimit &&
-                    uniform(s.fir.in_buf, bin, sin_) && uniform(g.out_buf, bout, sout) && s.fir.in_len >= 1 &&
-                    tmap_encode_2d_f64(&mi, bin, s.fir.in_len, rows, sin_, kFtSlotPos, kFtRows) &&
-                    tmap_encode_2d_f64(&mo, bout, g.n_out, rows, sout, 16, kFtRows / 2)) {
-                    FirTmParams T{};
-                    T.scalars = scalars; T.nscalars = nscal; T.sumsq_slot = g.sumsq_slot; T.nch = g.nchannels;
-                    T.nrows = rows; T.n_out = g.n_out; T.tapsper = g.taps_per_phase; T.ks = ks; T.nslot = nslot;
-                    T.ntiles = (g.n_out + kFmT - 1) / kFmT;
-                    T.pfb = P.pfb; T.dpfb = P.dpfb; T.xi0 = P.xi0; T.poff = pd.poff[si]; T.alpha = pd.alpha[si];
-                    T.tab_doubles = (int)tabd_eff;
-                    T.bands_g = bands_g; T.period_tiles = period_tiles;
-                    T.epoch_tiles = s.fir.epoch_tiles; T.n_epochs = (int)s.fir.n_epochs;
-                    T.gain = s.fir.epi_scale;
-                    if (const char* e = getenv("SIGOPS_FIR_EXP")) T.exp = atoi(e);
-                    const int64_t groups = (rows + kFtRows - 1) / kFtRows;
-                    // segments along the time axis: whole waves of one block per SM; a segment pays about
-                    // three tiles of start-up (first window, pipeline fill)
-                    int64_t best_tps = T.ntiles;
-                    double best_cost = 1e300;
-                    for (int w = 1; w <= 8; ++w) {
-                        int64_t nseg = std::max<int64_t>(1, std::min<int64_t>(T.ntiles, ((int64_t)w * dev.sm_count + groups - 1) / groups));
-                        const int64_t tps = (T.ntiles + nseg - 1) / nseg;
-                        nseg = (T.ntiles + tps - 1) / tps;
-                        const int64_t waves = (groups * nseg + dev.sm_count - 1) / dev.sm_count;
-                        const double cost = (double)waves * (double)(tps + 3);
-                        if (cost < best_cost) { best_cost = cost; best_tps = tps; }
-                    }
-                    if (const char* e = getenv("SIGOPS_FIR_TPS")) best_tps = std::max<int64_t>(1, atoll(e));
-                    T.tiles_per_seg = best_tps;
-                    const int64_t nseg = (T.ntiles + best_tps - 1) / best_tps;
-                    const size_t smem = fir_tm_smem_bytes(nslot, ks, (int)tabd_eff, has_d);
-                    dim3 tgrid((unsigned)nseg, (unsigned)groups);
-                    if (groups <= 65535) {
-                        if (getenv("SIGOPS_DEBUG"))
-                            fprintf(stderr, "[sigops] FIR stage %zu: tensor-map rows=%lld n_out=%lld taps=%d ks=%d slots=%d (window %d) grid=%lldx%lld tiles/seg=%lld smem=%zu gain=%g period=%lld outputs%s\n",
-                                    si, (long long)rows, (long long)g.n_out, T.tapsper, ks, nslot, win_slots, (long long)nseg, (long long)groups,
-                                    (long long)best_tps, smem, T.gain, (long long)s.fir.period, bands_g ? " (tap bands from the period tables)" : "");
-                            if (getenv("SIGOPS_DEBUG") && bands_g) fprintf(stderr, "[sigops]   %lld epochs of %lld tiles\n", (long long)s.fir.n_epochs, (long long)s.fir.epoch_tiles);
-                        const bool ssq = g.sumsq_slot >= 0;
-                        if (getenv("SIGOPS_FIR_DBG")) {
-                            // tuning aid: one synchronous launch with cycle counters, printed per role
-                            const size_t nb = (size_t)nseg * groups;
-                            long long* dbg = nullptr;
-                            CUDA_OK(cudaMalloc(&dbg, nb * 8 * sizeof(long long)));
-                            CUDA_OK(cudaMemset(dbg, 0, nb * 8 * sizeof(long long)));
-                            FirTmParams D = T;
-                            D.dbg = dbg;
-                            ensure_dyn_smem(k_fir_tmap<false, true>, smem);
-                            k_fir_tmap<false, true><<<tgrid, kFtThreads, smem, stream>>>(D, *(const CUtensorMap*)&mi, *(const CUtensorMap*)&mo);
-                            CUDA_OK(cudaStreamSynchronize(stream));
-                            std::vector<long long> h(nb * 8);
-                            CUDA_OK(cudaMemcpy(h.data(), dbg, h.size() * sizeof(long long), cudaMemcpyDeviceToHost));
-                            cudaFree(dbg);
-                            double sum[8] = {0};
-                            for (size_t b = 0; b < nb; ++b)
-                                for (int k = 0; k < 8; ++k) sum[k] += (double)h[b * 8 + k];
-                            const double per = 1.0 / ((double)nb * (double)best_tps);
-                            fprintf(stderr, "[sigops] FIR tmap cycles/tile  compute: set-up %.0f (of it wait_taps %.0f) staging %.0f (of it wait_stg %.0f) total %.0f | helper: wait_done %.0f build %.0f\n",
-                                    sum[1] * per, sum[0] * per, sum[6] * per, sum[2] * per, sum[3] * per, sum[4] * per, sum[5] * per);
-                        }
-                        add(KIND_FIR, [=](cudaStream_t st) {
-                            const CUtensorMap& a = *(const CUtensorMap*)&mi;
-                            const CUtensorMap& b = *(const CUtensorMap*)&mo;
-#define SIGOPS_FIR_TM_CASE(SSQ_)                                        \
-    {                                                                    \
-        ensure_dyn_smem(k_fir_tmap<SSQ_>, smem);                         \
-        k_fir_tmap<SSQ_><<<tgrid, kFtThreads, smem, st>>>(T, a, b);      \
-    }
-                            if (ssq) SIGOPS_FIR_TM_CASE(true)
-                            else SIGOPS_FIR_TM_CASE(false)
-#undef SIGOPS_FIR_TM_CASE
-                        });
-                        continue;
-                    }
-                }
-            }
-            if (mma) {
-                FirMmaParams Q{};
-                Q.bufrefs = d_refs; Q.scalars = scalars; Q.nbuf = nbuf; Q.nscalars = nscal;
-                Q.in_buf = s.fir.in_buf; Q.out_buf = g.out_buf; Q.sumsq_slot = g.sumsq_slot;
-                Q.in_len = s.fir.in_len; Q.nch = g.nchannels; Q.nrows = rows; Q.n_out = g.n_out;
-                Q.tapsper = g.taps_per_phase;
-                Q.ks = (int)round_up(s.fir.dpad + g.taps_per_phase, 4);
-                Q.ring = s.fir.ring32;
-                Q.pitch = Q.ring + ((4 - Q.ring % 16) + 16) % 16;
-                Q.pfb = P.pfb; Q.dpfb = P.dpfb; Q.xi0 = P.xi0; Q.poff = pd.poff[si]; Q.alpha = pd.alpha[si];
-                Q.ntiles = (g.n_out + kFmT - 1) / kFmT;
-                Q.gain = s.fir.epi_scale;
-                // both polyphase banks ride along in shared memory when that leaves the ring its room
-                const int64_t tabd = (int64_t)g.n_phases * g.taps_per_phase;
-                const size_t tab_bytes = (size_t)tabd * 8 * (P.dpfb ? 2 : 1);
-                Q.tab_doubles = (int)tabd;
-                if (tab_bytes > 48 * 1024) mma = false;      // banks too large to ride along in shared memory
-                auto smem_for = [&](int RBx) {
-                    return (size_t)RBx * Q.pitch * 8 + (size_t)2 * 4 * Q.ks * kFmHbPitch * 8 + tab_bytes;
-                };
-                // rows per block RB: as many as the batch fills and shared memory holds
-                int RB = rows > 64 ? 128 : (rows > 32 ? 64 : 32);
-                if (const char* e = getenv("SIGOPS_FIR_RB")) RB = atoi(e) >= 128 ? 128 : (atoi(e) >= 64 ? 64 : 32);
-                while (RB > 32 && smem_for(RB) > kFirMmaSmemLimit) RB >>= 1;
-                const int RH = getenv("SIGOPS_FIR_RH") ? std::max(1, std::min(2, atoi(getenv("SIGOPS_FIR_RH")))) : 2;
-                const int MF = RB;      // (kept for the debug line)
-                const int64_t groups = (rows + RB - 1) / RB;
-                if (mma && smem_for(RB) <= kFirMmaSmemLimit && groups <= 65535) {
-                    // segments along the time axis: whole waves of one block per SM; a segment pays
-                    // about three tiles of start-up (first window, pipeline fill)
-                    int64_t best_tps = Q.ntiles;
-                    double best_cost = 1e300;
-                    for (int w = 1; w <= 8; ++w) {
-                        int64_t nseg = std::max<int64_t>(1, std::min<int64_t>(Q.ntiles, ((int64_t)w * dev.sm_count + groups - 1) / groups));
-                        const int64_t tps = (Q.ntiles + nseg - 1) / nseg;
-                        nseg = (Q.ntiles + tps - 1) / tps;
-                        const int64_t waves = (groups * nseg + dev.sm_count - 1) / dev.sm_count;
-                        const double cost = (double)waves * (double)(tps + 3);
-                        if (cost < best_cost) { best_cost = cost; best_tps = tps; }
-                    }
-                    if (const char* e = getenv("SIGOPS_FIR_TPS")) best_tps = std::max<int64_t>(1, atoll(e));
-                    Q.tiles_per_seg = best_tps;
-                    const int64_t nseg = (Q.ntiles + best_tps - 1) / best_tps;
-                    const size_t smem = smem_for(RB);
-                    dim3 grid((unsigned)nseg, (unsigned)groups);
-                    if (getenv("SIGOPS_DEBUG"))
-                        fprintf(stderr, "[sigops] FIR stage %zu: mma rows=%lld n_out=%lld taps=%d ks=%d ring=%d pitch=%d rows/block=%d grid=%lldx%lld tiles/seg=%lld smem=%zu\n",
-                                si, (long long)rows, (long long)g.n_out, Q.tapsper, Q.ks, Q.ring, Q.pitch, MF, (long long)nseg,
-                                (long long)groups, (long long)best_tps, smem);
-                    if (getenv("SIGOPS_FIR_DBG")) {
-                        // tuning aid: one synchronous launch with cycle counters, printed per role
-                        const size_t nb = (size_t)nseg * groups;
-                        long long* dbg = nullptr;
-                        CUDA_OK(cudaMalloc(&dbg, nb * 8 * sizeof(long long)));
-                        CUDA_OK(cudaMemset(dbg, 0, nb * 8 * sizeof(long long)));
-                        FirMmaParams D = Q;
-                        D.dbg = dbg;
-                        if (RB == 128 && RH == 2) {
-                            ensure_dyn_smem(k_fir_mma<8, 2, false>, smem);
-                            k_fir_mma<8, 2, false><<<grid, 16 * 32, smem, stream>>>(D);
-                        } else if (RB == 128) {
-                            ensure_dyn_smem(k_fir_mma<16, 1, false>, smem);
-                            k_fir_mma<16, 1, false><<<grid, 8 * 32, smem, stream>>>(D);
-                        }
-                        CUDA_OK(cudaStreamSynchronize(stream));
-                        std::vector<long long> h(nb * 8);
-                        CUDA_OK(cudaMemcpy(h.data(), dbg, h.size() * sizeof(long long), cudaMemcpyDeviceToHost));
-                        cudaFree(dbg);
-                        double sum[8] = {0};
-                        for (size_t b = 0; b < nb; ++b)
-                            for (int k = 0; k < 8; ++k) sum[k] += (double)h[b * 8 + k];
-                        const double per = 1.0 / ((double)nb * (double)best_tps);
-                        fprintf(stderr, "[sigops] FIR cycles/tile  aux: wait_done %.0f extend %.0f taps %.0f | compute: wait_taps %.0f wait_data %.0f dmma %.0f store %.0f\n",
-                                sum[0] * per, sum[1] * per, sum[2] * per, sum[3] * per, sum[4] * per, sum[5] * per, sum[6] * per);
-                    }
-                    add(KIND_FIR, [=](cudaStream_t st) {
-#define SIGOPS_FIR_MMA_CASE(rb, rh)                                                          \
-    if (RB == rb && RH == rh) {                                                              \
-        if (Q.sumsq_slot >= 0) {                                                             \
-            ensure_dyn_smem(k_fir_mma<rb / (8 * rh), rh, true>, smem);                       \
-            k_fir_mma<rb / (8 * rh), rh, true><<<grid, 8 * rh * 32, smem, st>>>(Q);         \
-        } else {                                                                             \
-            ensure_dyn_smem(k_fir_mma<rb / (8 * rh), rh, false>, smem);                      \
-            k_fir_mma<rb / (8 * rh), rh, false><<<grid, 8 * rh * 32, smem, st>>>(Q);        \
-        }                                                                                    \
-    }
-                        SIGOPS_FIR_MMA_CASE(128, 1) SIGOPS_FIR_MMA_CASE(64, 1) SIGOPS_FIR_MMA_CASE(32, 1)
-                        SIGOPS_FIR_MMA_CASE(128, 2) SIGOPS_FIR_MMA_CASE(64, 2) SIGOPS_FIR_MMA_CASE(32, 2)
-#undef SIGOPS_FIR_MMA_CASE
-                    });
-                    continue;
-                }
-            }
-            // rows per thread: as many as fit in shared memory, but no more than the batch can fill
-            int G = 4;
-            if (const char* e = getenv("SIGOPS_FIR_G")) G = std::max(1, std::min(4, atoi(e)));
-            while (G > 1 && (fir_smem_bytes(s.fir, g.taps_per_phase, G, p.max_stack) > kFirSmemLimit || rows <= 16 * G)) G >>= 1;
-            // 32-output tiles when two such blocks fit on an SM (copies of one overlap FMAs of the other)
-            // (measured on B200, config 3: 64-output tiles 3.8 ms vs 32-output tiles 4.7 ms — the smaller
-            //  tile's extra halo and per-tile set-up cost more than the overlap buys; kept as a knob)
-            int W = 8;
-            if (const char* e = getenv("SIGOPS_FIR_W")) W = atoi(e) == 4 && G == 4 ? 4 : 8;
-            const FirGeom geo = fir_geometry(s.fir, g.taps_per_phase, G, p.max_stack, W);
-            P.hbase = geo.hbase; P.tpad = geo.tpad; P.xpitch = geo.xpitch;
-            const size_t smem = geo.smem;
-            const int T = 8 * W;
-            const int64_t tiles = (g.n_out + T - 1) / T;
-            const int64_t groups = (rows + 32 * G - 1) / (32 * G);
-            if (groups > 65535) fail(SIGOPS_ERR_UNSUPPORTED, "FIR stage over more than %d rows per wave", 65535 * 32 * G);
-            dim3 grid((unsigned)tiles, (unsigned)groups);
-            add(KIND_FIR, [=](cudaStream_t st) {
-                if (G == 4 && W == 4) {
-                    ensure_dyn_smem(k_fir<4, 4>, smem);
-                    k_fir<4, 4><<<grid, 128, smem, st>>>(P);
-                } else if (G == 4) {
-                    ensure_dyn_smem(k_fir<4, 8>, smem);
-                    k_fir<4, 8><<<grid, 256, smem, st>>>(P);
-                } else if (G == 2) {
-                    ensure_dyn_smem(k_fir<2, 8>, smem);
-                    k_fir<2, 8><<<grid, 256, smem, st>>>(P);
-                } else {
-                    ensure_dyn_smem(k_fir<1, 8>, smem);
-                    k_fir<1, 8><<<grid, 256, smem, st>>>(P);
-                }
-            });
+    // (slot.last_table now holds this wave's table)
+    Wave w{p, pd, dev.sm_count, (const BufRef*)slot.last_table.data(), d_refs, scalars, nbuf, nscal, ninst, io.inst0, 0,
+           slot.arena, stream, slot.cache_launches};
+    for (w.si = 0; w.si < p.stages.size(); ++w.si) {
+        switch (p.stages[w.si].st.kind) {
+            case SIGOPS_STAGE_MAP: plan_map_stage(w); break;
+            case SIGOPS_STAGE_IIR: plan_iir_stage(w); break;
+            default: plan_fir_stage(w);
         }
     }
     slot.cache_plan = p.uid;
