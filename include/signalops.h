@@ -178,12 +178,18 @@ typedef struct sigops_tabledesc {
  *   PUSH             save acc on a small stack (depth <= SIGOPS_MAX_STACK)
  *   POPADD/...       acc = popped (op) acc
  *   NEG, CAST_F32    unary on acc
+ *   FN1              acc = f(acc)          f = SIGOPS_EFN_* in `fn`, no leaf; d0, d1 = constant
+ *                                          parameters (CLAMP: lo, hi)
+ *   FN2              acc = g(acc, leaf)    g in `fn`: the leaf must not read `fn` itself, so only
+ *                                          CONST, BUF, CHANSUM, RMS, STAGE and RANDN leaves
+ *   POPFN2           acc = g(popped, acc)  (generator and ramp operands: PUSH ... POPFN2)
  * Julia's left-to-right `((a+b)+c)` order is kept by construction
  * (src/mapsignal.jl:249-255). */
 enum {
     SIGOPS_OP_LOAD = 1, SIGOPS_OP_ADD, SIGOPS_OP_SUB, SIGOPS_OP_MUL, SIGOPS_OP_DIV,
     SIGOPS_OP_PUSH, SIGOPS_OP_POPADD, SIGOPS_OP_POPSUB, SIGOPS_OP_POPMUL, SIGOPS_OP_POPDIV,
-    SIGOPS_OP_NEG, SIGOPS_OP_CAST_F32, SIGOPS_OP_CAST_I64
+    SIGOPS_OP_NEG, SIGOPS_OP_CAST_F32, SIGOPS_OP_CAST_I64,
+    SIGOPS_OP_FN1, SIGOPS_OP_FN2, SIGOPS_OP_POPFN2
 };
 #define SIGOPS_MAX_STACK 4
 #define SIGOPS_MAX_PROG 48
@@ -220,6 +226,30 @@ enum {
     SIGOPS_FN_IDENTITY,    /* x                                                            */
     SIGOPS_FN_SINRAMP      /* sinpi(0.5x)             (src/ramps.jl:4)                     */
 };
+
+/* elementwise functions of OperateOn closures (`fn` of FN1 / FN2 / POPFN2), Julia's Base semantics on
+ * Float64 (src/mapsignal.jl:131-145 calls the closure per sample).  Where Julia throws a DomainError
+ * (sqrt(-1.0), log(-1.0), a non-integer power of a negative number) the device returns NaN.
+ * Exact: ABS .. CLAMP and MIN .. MOD.  Within a few ulp of Julia's libm: EXP .. CBRT, POW, HYPOT. */
+enum {
+    /* unary (FN1) */
+    SIGOPS_EFN_ABS = 1, SIGOPS_EFN_SIGN, SIGOPS_EFN_FLOOR, SIGOPS_EFN_CEIL, SIGOPS_EFN_TRUNC,
+    SIGOPS_EFN_ROUND,      /* ties to even (Julia `round`, numpy `rint`)                  */
+    SIGOPS_EFN_SQRT,       /* correctly rounded                                           */
+    SIGOPS_EFN_CLAMP,      /* clamp(x, d0, d1): x > d1 ? d1 : x < d0 ? d0 : x (NaN stays) */
+    SIGOPS_EFN_EXP, SIGOPS_EFN_EXP2, SIGOPS_EFN_EXPM1, SIGOPS_EFN_LOG, SIGOPS_EFN_LOG2, SIGOPS_EFN_LOG10,
+    SIGOPS_EFN_LOG1P, SIGOPS_EFN_SIN, SIGOPS_EFN_COS, SIGOPS_EFN_TAN, SIGOPS_EFN_TANH, SIGOPS_EFN_SINH,
+    SIGOPS_EFN_COSH, SIGOPS_EFN_ATAN, SIGOPS_EFN_CBRT,
+    /* binary (FN2, POPFN2): g(a, b) */
+    SIGOPS_EFN_MIN = 32,   /* Julia `min`: NaN propagates, -0.0 < 0.0 (not fmin)          */
+    SIGOPS_EFN_MAX,        /* Julia `max`, likewise                                       */
+    SIGOPS_EFN_COPYSIGN,
+    SIGOPS_EFN_REM,        /* fmod                                                        */
+    SIGOPS_EFN_MOD,        /* Julia `mod`: rem, + b when the signs differ, 0 takes b's sign */
+    SIGOPS_EFN_POW, SIGOPS_EFN_HYPOT
+};
+#define SIGOPS_EFN_UNARY_LAST SIGOPS_EFN_CBRT
+#define SIGOPS_EFN_BINARY_LAST SIGOPS_EFN_HYPOT
 
 typedef struct sigops_instr {
     uint8_t op, leaf, fn, flags;

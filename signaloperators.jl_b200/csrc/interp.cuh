@@ -233,6 +233,72 @@ __device__ __forceinline__ double binop(int op, double a, double b) {
     }
 }
 
+// ---- OperateOn closure functions (SIGOPS_EFN_*), Julia's Base semantics on Float64 ----
+// Julia `min` / `max` (base/math.jl): a NaN operand wins, and -0.0 orders below 0.0.  CUDA's fmin/fmax drop NaNs.
+__device__ __forceinline__ double jl_min(double a, double b) {
+    if (a != a || b != b) return a + b;
+    return a == b ? (signbit(a) ? a : b) : (a < b ? a : b);
+}
+__device__ __forceinline__ double jl_max(double a, double b) {
+    if (a != a || b != b) return a + b;
+    return a == b ? (signbit(a) ? b : a) : (a > b ? a : b);
+}
+
+// Every function but the four efn_vec keeps in line, out of line for the reason leaf_value_slow is: inlined at
+// every V-wide call site libm bodies took the fused IIR kernels from 7k to 54k SASS instructions (DESIGN §3 K1),
+// and even the one-instruction roundings nearly double the fused kernels' code when each gets a V-wide case.
+static __device__ __noinline__ double efn_slow(int fn, double a, double b) {
+    switch (fn) {
+        case SIGOPS_EFN_SIGN: return (a > 0.0) ? 1.0 : ((a < 0.0) ? -1.0 : a);       // keeps +-0 and NaN
+        case SIGOPS_EFN_FLOOR: return floor(a);
+        case SIGOPS_EFN_CEIL: return ceil(a);
+        case SIGOPS_EFN_TRUNC: return trunc(a);
+        case SIGOPS_EFN_ROUND: return rint(a);
+        case SIGOPS_EFN_COPYSIGN: return copysign(a, b);
+        case SIGOPS_EFN_SQRT: return sqrt(a);
+        case SIGOPS_EFN_EXP: return exp(a);
+        case SIGOPS_EFN_EXP2: return exp2(a);
+        case SIGOPS_EFN_EXPM1: return expm1(a);
+        case SIGOPS_EFN_LOG: return log(a);
+        case SIGOPS_EFN_LOG2: return log2(a);
+        case SIGOPS_EFN_LOG10: return log10(a);
+        case SIGOPS_EFN_LOG1P: return log1p(a);
+        case SIGOPS_EFN_SIN: return sin(a);
+        case SIGOPS_EFN_COS: return cos(a);
+        case SIGOPS_EFN_TAN: return tan(a);
+        case SIGOPS_EFN_TANH: return tanh(a);
+        case SIGOPS_EFN_SINH: return sinh(a);
+        case SIGOPS_EFN_COSH: return cosh(a);
+        case SIGOPS_EFN_ATAN: return atan(a);
+        case SIGOPS_EFN_CBRT: return cbrt(a);
+        case SIGOPS_EFN_REM: return fmod(a, b);
+        case SIGOPS_EFN_MOD: {
+            const double r = fmod(a, b);
+            if (r == 0.0) return copysign(r, b);
+            return ((r > 0.0) != (b > 0.0)) ? r + b : r;
+        }
+        case SIGOPS_EFN_POW: return pow(a, b);
+        case SIGOPS_EFN_HYPOT: return hypot(a, b);
+    }
+    return __longlong_as_double(0x7ff8000000000000LL);
+}
+
+// a[j] = f(a[j]) (FN1: b(j), c = the instruction's d0, d1) or g(a[j], b(j)) (FN2, POPFN2) for V values; the function
+// is decoded once.  abs, clamp, min and max (envelopes, clipping, rectifiers) run in line, everything else is one
+// efn_slow call per value.
+template <int V, class B>
+__device__ __forceinline__ void efn_vec(int fn, double* a, B b, double c) {
+#define SIGOPS_EFN_LOOP(expr) _Pragma("unroll") for (int j = 0; j < V; ++j) { const double x = a[j]; a[j] = (expr); } break
+    switch (fn) {
+        case SIGOPS_EFN_ABS: SIGOPS_EFN_LOOP(fabs(x));
+        case SIGOPS_EFN_CLAMP: SIGOPS_EFN_LOOP(x > c ? c : (x < b(j) ? b(j) : x));
+        case SIGOPS_EFN_MIN: SIGOPS_EFN_LOOP(jl_min(x, b(j)));
+        case SIGOPS_EFN_MAX: SIGOPS_EFN_LOOP(jl_max(x, b(j)));
+        default: SIGOPS_EFN_LOOP(efn_slow(fn, x, b(j)));
+    }
+#undef SIGOPS_EFN_LOOP
+}
+
 // V frames of a buffer leaf, `nstride` apart.  The common case (Float64, every frame
 // inside the valid range) is V plain loads off one base pointer; everything else falls
 // back to the per-frame path (pads, other sample types).
@@ -263,7 +329,9 @@ __device__ __forceinline__ void buf_values(const sigops_instr& I, const sigops_i
 // [depth][V] with stride `sstride` doubles between consecutive slots (so neighbouring
 // threads interleave and stay bank-conflict free).  Each instruction is decoded once
 // (copied to registers) and its leaf is evaluated for all V frames by a vector routine.
-template <int V>
+// FN: the program may hold closure functions (FN1 / FN2 / POPFN2).  The hot kernels have a variant without them, chosen
+// by the host from the plan, so that programs without functions keep their registers and spill-free code.
+template <int V, bool FN = true>
 __device__ __forceinline__ void eval_program(const sigops_instr* sprog, const double* leafconst,
                                              const double2* leafrot, int len, const Env& env,
                                              int64_t n0, int64_t nstride, int c, const double* stageval,
@@ -274,7 +342,7 @@ __device__ __forceinline__ void eval_program(const sigops_instr* sprog, const do
     for (int pc = 0; pc < len; ++pc) {
         const sigops_instr I = sprog[pc];
         const int op = I.op;
-        if (op <= SIGOPS_OP_DIV) {
+        if (op <= SIGOPS_OP_DIV || (FN && op == SIGOPS_OP_FN2)) {
             double v[V];
             switch (I.leaf) {
                 case SIGOPS_LEAF_CONST:
@@ -348,6 +416,9 @@ __device__ __forceinline__ void eval_program(const sigops_instr* sprog, const do
 #pragma unroll
                     for (int j = 0; j < V; ++j) acc[j] *= v[j];
                     break;
+                case SIGOPS_OP_FN2:
+                    if constexpr (FN) efn_vec<V>(I.fn, acc, [&](int j) { return v[j]; }, 0.0);
+                    break;
                 default:
 #pragma unroll
                     for (int j = 0; j < V; ++j) acc[j] /= v[j];
@@ -369,6 +440,16 @@ __device__ __forceinline__ void eval_program(const sigops_instr* sprog, const do
         } else if (op == SIGOPS_OP_CAST_I64) {
 #pragma unroll
             for (int j = 0; j < V; ++j) acc[j] = (double)(long long)acc[j];
+        } else if (FN && op == SIGOPS_OP_FN1) {
+            efn_vec<V>(I.fn, acc, [&](int) { return I.d0; }, I.d1);
+        } else if (FN && op == SIGOPS_OP_POPFN2) {
+            --sp;
+            double l[V];
+#pragma unroll
+            for (int j = 0; j < V; ++j) l[j] = stack[(sp * V + j) * sstride];
+            efn_vec<V>(I.fn, l, [&](int j) { return acc[j]; }, 0.0);
+#pragma unroll
+            for (int j = 0; j < V; ++j) acc[j] = l[j];
         }
     }
 }

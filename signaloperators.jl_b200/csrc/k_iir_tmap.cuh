@@ -72,7 +72,9 @@ struct IirTmapParams {
     double coef[kIirMaxSections][5];
     // Fused elementwise programs whose leaves do not depend on the row (constants, generators, ramps — e.g.
     // BASELINE config 5: x * (0.5 sin + 0.5) before the cascade, y * ramp_on * ramp_off + tone after it):
-    // ops[0 .. n_in_ops) combine the loaded sample with their leaf, ops[4 .. 4 + n_ep_ops) the filter output.
+    // ops[0 .. n_in_ops) combine the loaded sample with their leaf, ops[4 .. 4 + n_ep_ops) the filter output.  A
+    // closure function f(x) (FN1) or g(x, constant) (FN2) takes an op slot and no leaf vector (e.g. abs before an
+    // envelope follower's lowpass, tanh after a filter).
     int n_in_ops, n_ep_ops;
     sigops_instr ops[2 * kTmMaxLeafOps];
 };
@@ -96,8 +98,14 @@ __device__ __forceinline__ void tmap_store_3d(const CUtensorMap* tm, int c0, int
 // reference's DF2T filter state, and results are rounded on store.
 // Returns sum(out^2) over the first `nvalid` outputs as stored.
 // acc[k] = acc[k] (op) v[k] for 16 frames, the operator decoded once (v: warp-uniform values in shared memory)
-__device__ __forceinline__ void apply_leaf16(int op, double* acc, const double* v) {
-    switch (op) {
+// (FN1 / FN2 with a constant: acc[k] = f(acc[k]) or g(acc[k], d0), no leaf vector)
+template <bool FN>
+__device__ __forceinline__ void apply_leaf16(const sigops_instr& I, double* acc, const double* v) {
+    if (FN && (I.op == SIGOPS_OP_FN1 || I.op == SIGOPS_OP_FN2)) {
+        efn_vec<16>(I.fn, acc, [&](int) { return I.d0; }, I.d1);
+        return;
+    }
+    switch (I.op) {
         case SIGOPS_OP_ADD:
 #pragma unroll
             for (int k = 0; k < 16; ++k) acc[k] = acc[k] + v[k];
@@ -117,7 +125,8 @@ __device__ __forceinline__ void apply_leaf16(int op, double* acc, const double* 
     }
 }
 
-template <int M, bool UNITB, class T, bool LV = false>
+// LV: 0 none, 1 row-invariant leaf operations, 2 the same with closure functions among them
+template <int M, bool UNITB, class T, int LV = 0>
 __device__ __forceinline__ double cascade16_swz(Cascade<M>& f, unsigned char* row, int key, int blk, double gain, double sc, double sc2,
                                                 int nvalid, bool want_ss, const IirTmapParams* P = nullptr, const double* lv = nullptr,
                                                 int lvpitch = 0, unsigned skip = 0u) {
@@ -139,7 +148,7 @@ __device__ __forceinline__ double cascade16_swz(Cascade<M>& f, unsigned char* ro
     //  outside its short region — which is the identity, bit for bit)
     if (LV) {
         for (int j = 0; j < P->n_in_ops; ++j)
-            if (!((skip >> j) & 1u)) apply_leaf16(P->ops[j].op, xr, lv + j * lvpitch);
+            if (!((skip >> j) & 1u)) apply_leaf16<LV == 2>(P->ops[j], xr, lv + j * lvpitch);
     }
     double pipe[M], out[16];
 #pragma unroll
@@ -166,7 +175,7 @@ __device__ __forceinline__ double cascade16_swz(Cascade<M>& f, unsigned char* ro
     if (LV) {
         for (int j = 0; j < P->n_ep_ops; ++j)
             if (!((skip >> (kTmMaxLeafOps + j)) & 1u))
-                apply_leaf16(P->ops[kTmMaxLeafOps + j].op, out, lv + (kTmMaxLeafOps + j) * lvpitch);
+                apply_leaf16<LV == 2>(P->ops[kTmMaxLeafOps + j], out, lv + (kTmMaxLeafOps + j) * lvpitch);
     }
     if (sizeof(T) == 8) {
 #pragma unroll
@@ -195,7 +204,7 @@ __device__ __forceinline__ double rowinv_leaf(const sigops_instr* I, int64_t n) 
     return I->leaf == SIGOPS_LEAF_CONST ? I->d0 : leaf_value_slow(I, nullptr, n, 0);
 }
 
-template <int M, bool UNITB, int NW, int NS, int SUBS, class T, bool LV = false>
+template <int M, bool UNITB, int NW, int NS, int SUBS, class T, int LV = 0>
 __global__ void __launch_bounds__(NW * 32, 1)
 k_iir_tmap(const __grid_constant__ IirTmapParams P, const __grid_constant__ CUtensorMap tm_in,
            const __grid_constant__ CUtensorMap tm_out) {
@@ -306,7 +315,7 @@ k_iir_tmap(const __grid_constant__ IirTmapParams P, const __grid_constant__ CUte
             for (int v = threadIdx.x; v < nops * SC; v += NW * 32) {
                 const int jj = v / SC, fr = v - jj * SC;
                 const int j = jj < P.n_in_ops ? jj : kTmMaxLeafOps + jj - P.n_in_ops;
-                if ((skip >> j) & 1u) continue;
+                if (((skip >> j) & 1u) || (LV == 2 && P.ops[j].op >= SIGOPS_OP_FN1)) continue;   // (functions: no vector)
                 lvw[j * SC + fr] = ((ones >> j) & 1u) ? 1.0 : rowinv_leaf(&P.ops[j], n0 + fr);
             }
             __syncthreads();

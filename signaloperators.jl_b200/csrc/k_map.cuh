@@ -39,6 +39,7 @@ struct MapParams {
     int tile_prefix[kMaxPieces + 1];
 };
 
+template <bool FN>      // the plan holds closure functions (eval_program)
 __global__ void __launch_bounds__(kMapThreads, 4)
 k_map(const __grid_constant__ MapParams P) {
     __shared__ sigops_instr sprog[SIGOPS_MAX_PROG];
@@ -73,7 +74,7 @@ k_map(const __grid_constant__ MapParams P) {
         const int64_t n0 = pc.out_start + (tile * P.passes + pass) * (int64_t)kMapSub + threadIdx.x;
         if (n0 - threadIdx.x >= nend) break;
         double acc[kMapV];
-        eval_program<kMapV>(sprog, leafconst, leafrot, pc.prog_len, env, n0, kMapThreads, c, nullptr, acc,
+        eval_program<kMapV, FN>(sprog, leafconst, leafrot, pc.prog_len, env, n0, kMapThreads, c, nullptr, acc,
                             stack + threadIdx.x, kMapThreads);
         if (ob.dtype == SIGOPS_F64) {
             double* op = reinterpret_cast<double*>(ob.ptr) + (int64_t)c * ob.ld + n0;

@@ -22,9 +22,9 @@ EncodeTiledFn encode_fn() {
     return fn;
 }
 
-template <int M, int NW, int NS, int SUBS, class T, bool LV>
+template <int M, int NW, int NS, int SUBS, class T, int LV>
 void launch_cfg(bool unitb, dim3 grid, cudaStream_t st, const IirTmapParams& P, const CUtensorMap& a, const CUtensorMap& b) {
-    constexpr size_t smem = tm_smem_bytes(NW, NS, SUBS, LV, 128 / (int)sizeof(T));
+    constexpr size_t smem = tm_smem_bytes(NW, NS, SUBS, LV != 0, 128 / (int)sizeof(T));
     if (unitb) {
         ensure_dyn_smem(k_iir_tmap<M, true, NW, NS, SUBS, T, LV>, smem);
         k_iir_tmap<M, true, NW, NS, SUBS, T, LV><<<grid, NW * 32, smem, st>>>(P, a, b);
@@ -37,9 +37,12 @@ void launch_cfg(bool unitb, dim3 grid, cudaStream_t st, const IirTmapParams& P, 
 template <int M>
 void launch_m(bool f32, bool unitb, dim3 grid, cudaStream_t st, const IirTmapParams& P, const CUtensorMap& a, const CUtensorMap& b) {
     const bool lv = P.n_in_ops + P.n_ep_ops > 0;
-    if (f32) launch_cfg<M, kTmWarpsF32, kTmStages, kTmSubsPerStageF32, float, false>(unitb, grid, st, P, a, b);
-    else if (lv) launch_cfg<M, kTmWarpsLv, kTmStages, kTmSubsPerStageLv, double, true>(unitb, grid, st, P, a, b);
-    else launch_cfg<M, kTmWarps, kTmStages, kTmSubsPerStage, double, false>(unitb, grid, st, P, a, b);
+    bool fn = false;                   // a closure function among the fused operations: the variant that applies them
+    for (int j = 0; j < 2 * kTmMaxLeafOps; ++j) fn = fn || P.ops[j].op == SIGOPS_OP_FN1 || P.ops[j].op == SIGOPS_OP_FN2;
+    if (f32) launch_cfg<M, kTmWarpsF32, kTmStages, kTmSubsPerStageF32, float, 0>(unitb, grid, st, P, a, b);
+    else if (lv && fn) launch_cfg<M, kTmWarpsLv, kTmStages, kTmSubsPerStageLv, double, 2>(unitb, grid, st, P, a, b);
+    else if (lv) launch_cfg<M, kTmWarpsLv, kTmStages, kTmSubsPerStageLv, double, 1>(unitb, grid, st, P, a, b);
+    else launch_cfg<M, kTmWarps, kTmStages, kTmSubsPerStage, double, 0>(unitb, grid, st, P, a, b);
 }
 
 }  // namespace

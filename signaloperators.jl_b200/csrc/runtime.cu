@@ -255,12 +255,16 @@ struct sigops_plan {
     int nbuf() const { return (int)bufs.size(); }
     int max_stack = 0;
     bool has_randn = false;        // some program draws device noise (LEAF_RANDN): launches depend on the wave's first instance index
+    bool has_fn = false;           // some program applies closure functions (FN1 / FN2 / POPFN2): k_map's variant with them
     uint64_t uid = 0;
 };
 
 namespace {
 
 // ---- plan validation ----------------------------------------------------------
+
+// LOAD, ADD .. DIV and FN2 evaluate a leaf
+bool op_has_leaf(int op) { return (op >= SIGOPS_OP_LOAD && op <= SIGOPS_OP_DIV) || op == SIGOPS_OP_FN2; }
 
 int program_stack_depth(const sigops_plan& p, int start, int len, bool allow_stage, const char* what) {
     if (len < 0 || start < 0 || (size_t)start + len > p.instrs.size())
@@ -270,9 +274,16 @@ int program_stack_depth(const sigops_plan& p, int start, int len, bool allow_sta
     int sp = 0, maxsp = 0;
     for (int i = 0; i < len; ++i) {
         const sigops_instr& I = p.instrs[start + i];
-        if (I.op < SIGOPS_OP_LOAD || I.op > SIGOPS_OP_CAST_I64) fail(SIGOPS_ERR_INVALID, "%s: bad opcode %d", what, I.op);
+        if (I.op < SIGOPS_OP_LOAD || I.op > SIGOPS_OP_POPFN2) fail(SIGOPS_ERR_INVALID, "%s: bad opcode %d", what, I.op);
         if (i == 0 && I.op != SIGOPS_OP_LOAD) fail(SIGOPS_ERR_INVALID, "%s: program must start with LOAD", what);
-        if (I.op <= SIGOPS_OP_DIV) {
+        if (I.op == SIGOPS_OP_FN1 && (I.fn < SIGOPS_EFN_ABS || I.fn > SIGOPS_EFN_UNARY_LAST))
+            fail(SIGOPS_ERR_UNSUPPORTED, "%s: unary function %d", what, I.fn);
+        if ((I.op == SIGOPS_OP_FN2 || I.op == SIGOPS_OP_POPFN2) && (I.fn < SIGOPS_EFN_MIN || I.fn > SIGOPS_EFN_BINARY_LAST))
+            fail(SIGOPS_ERR_UNSUPPORTED, "%s: binary function %d", what, I.fn);
+        // FN2 keeps its function in `fn`, so its leaf must be one that does not read `fn` (generators and ramps do)
+        if (I.op == SIGOPS_OP_FN2 && (I.leaf == SIGOPS_LEAF_GEN || I.leaf == SIGOPS_LEAF_RAMP_ON || I.leaf == SIGOPS_LEAF_RAMP_OFF))
+            fail(SIGOPS_ERR_INVALID, "%s: FN2 on a generator or ramp leaf (use PUSH ... POPFN2)", what);
+        if (op_has_leaf(I.op)) {
             switch (I.leaf) {
                 case SIGOPS_LEAF_CONST: break;
                 case SIGOPS_LEAF_BUF:
@@ -305,7 +316,7 @@ int program_stack_depth(const sigops_plan& p, int start, int len, bool allow_sta
         } else if (I.op == SIGOPS_OP_PUSH) {
             if (++sp > SIGOPS_MAX_STACK) fail(SIGOPS_ERR_UNSUPPORTED, "%s: expression nests deeper than SIGOPS_MAX_STACK", what);
             maxsp = std::max(maxsp, sp);
-        } else if (I.op <= SIGOPS_OP_POPDIV) {
+        } else if (I.op <= SIGOPS_OP_POPDIV || I.op == SIGOPS_OP_POPFN2) {
             if (--sp < 0) fail(SIGOPS_ERR_INVALID, "%s: POP on empty stack", what);
         }
     }
@@ -432,7 +443,7 @@ void derive_iir(sigops_plan& p, StageRT& s, int idx) {
         auto scan = [&](int start, int len, bool is_input) {
             for (int i = 0; i < len; ++i) {
                 const sigops_instr& I = p.instrs[start + i];
-                if (I.op > SIGOPS_OP_DIV) { if (I.op == SIGOPS_OP_PUSH) ok = false; continue; }   // no stack in this path
+                if (!op_has_leaf(I.op)) { if (I.op == SIGOPS_OP_PUSH) ok = false; continue; }   // no stack in this path
                 if (I.leaf == SIGOPS_LEAF_RMS || I.leaf == SIGOPS_LEAF_CHANSUM || I.leaf == SIGOPS_LEAF_RANDN) ok = false;
                 if (I.leaf == SIGOPS_LEAF_BUF) {
                     if (!is_input) { ok = false; continue; }
@@ -459,10 +470,15 @@ void derive_iir(sigops_plan& p, StageRT& s, int idx) {
             }
             if (s.iir.prog_in_len == 1) s.iir.prog_in_len = 0;      // bare load: nothing to evaluate
             // Row-invariant form: `LOAD buffer, (op leaf)*` before and `LOAD stage, (op leaf)*` after the cascade,
-            // every leaf a constant, generator or ramp (the same value for all rows at a frame)
+            // every leaf a constant, generator or ramp (the same value for all rows at a frame); closure functions
+            // f(acc) and g(acc, constant) take an operation slot and no leaf vector
             auto rowinv_ops = [&](int start, int len, std::vector<sigops_instr>& ops) {
                 for (int i = 1; i < len; ++i) {
                     const sigops_instr& I = p.instrs[start + i];
+                    if (I.op == SIGOPS_OP_FN1 || (I.op == SIGOPS_OP_FN2 && I.leaf == SIGOPS_LEAF_CONST)) {
+                        ops.push_back(I);
+                        continue;
+                    }
                     if (I.op < SIGOPS_OP_ADD || I.op > SIGOPS_OP_DIV) return false;
                     if (I.leaf != SIGOPS_LEAF_CONST && I.leaf != SIGOPS_LEAF_GEN && I.leaf != SIGOPS_LEAF_RAMP_ON &&
                         I.leaf != SIGOPS_LEAF_RAMP_OFF)
@@ -737,8 +753,10 @@ void parse_plan(sigops_plan& p, const void* bytes, size_t nbytes) {
         } else
             fail(SIGOPS_ERR_INVALID, "%s: unknown kind %d", what, g.kind);
     }
-    for (const sigops_instr& I : p.instrs)
-        if (I.op >= SIGOPS_OP_LOAD && I.op <= SIGOPS_OP_DIV && I.leaf == SIGOPS_LEAF_RANDN) p.has_randn = true;
+    for (const sigops_instr& I : p.instrs) {
+        if (op_has_leaf(I.op) && I.leaf == SIGOPS_LEAF_RANDN) p.has_randn = true;
+        if (I.op >= SIGOPS_OP_FN1) p.has_fn = true;
+    }
 }
 
 // ---- device-side plan constants -------------------------------------------------
@@ -1063,14 +1081,18 @@ void plan_map_stage(const Wave& w) {
     P.tile_prefix[g.n_pieces] = tiles;
     if (tiles == 0) return;
     const size_t stack_map = p.max_stack ? (size_t)p.max_stack * kMapV * kMapThreads * sizeof(double) : 0;
-    if (stack_map > 16 * 1024) ensure_dyn_smem(k_map, stack_map);
+    const bool fn = p.has_fn;
+    if (stack_map > 16 * 1024) ensure_dyn_smem(fn ? k_map<true> : k_map<false>, stack_map);
     for (int64_t i0 = 0; i0 < w.ninst; i0 += 65535) {
         const int64_t ni = std::min<int64_t>(65535, w.ninst - i0);
         MapParams Q = P;
         Q.bufrefs = w.d_refs + i0 * w.nbuf;
         Q.scalars = w.scalars + i0 * w.nscal;
         dim3 grid(tiles, P.out_nch, (unsigned)ni);
-        w.add(KIND_MAP, [=](cudaStream_t st) { k_map<<<grid, kMapThreads, stack_map, st>>>(Q); });
+        w.add(KIND_MAP, [=](cudaStream_t st) {
+            if (fn) k_map<true><<<grid, kMapThreads, stack_map, st>>>(Q);
+            else k_map<false><<<grid, kMapThreads, stack_map, st>>>(Q);
+        });
     }
 }
 
@@ -2144,7 +2166,7 @@ int sigops_plan_algorithmic_bytes(sigops_plan* plan, int64_t* bytes) {
             int64_t b = 0;
             for (int i = 0; i < len; ++i) {
                 const sigops_instr& I = plan->instrs[start + i];
-                if (I.op > SIGOPS_OP_DIV) continue;
+                if (!op_has_leaf(I.op)) continue;
                 if (I.leaf == SIGOPS_LEAF_BUF) b += frames * nch * (int64_t)elem_size(plan->bufs[I.buf].dtype);
                 if (I.leaf == SIGOPS_LEAF_CHANSUM) b += frames * I.i2 * (int64_t)elem_size(plan->bufs[I.buf].dtype);
             }

@@ -24,6 +24,7 @@ import numpy as np
 from . import dspjl, graph as G
 from .functors import functor_code
 from .philox import PhiloxRNG
+from .trace import TraceError, trace
 from .wav import WavSignal
 
 # ---- constants mirrored from include/signalops.h -------------------------------
@@ -31,11 +32,19 @@ F32, F64, I64 = 1, 2, 3
 OP_LOAD, OP_ADD, OP_SUB, OP_MUL, OP_DIV = 1, 2, 3, 4, 5
 OP_PUSH, OP_POPADD, OP_POPSUB, OP_POPMUL, OP_POPDIV = 6, 7, 8, 9, 10
 OP_NEG, OP_CAST_F32, OP_CAST_I64 = 11, 12, 13
+OP_FN1, OP_FN2, OP_POPFN2 = 14, 15, 16
 LEAF_NONE, LEAF_CONST, LEAF_BUF, LEAF_CHANSUM, LEAF_GEN = 0, 1, 2, 3, 4
 LEAF_RAMP_ON, LEAF_RAMP_OFF, LEAF_RMS, LEAF_STAGE, LEAF_RANDN = 5, 6, 7, 8, 9
 PAD_CONST, PAD_CYCLE, PAD_MIRROR, PAD_LAST = 0, 1, 2, 3
 FLAG_HAS_OMEGA = 1
 FN_SIN, FN_COS, FN_SAW, FN_AFFINE_SIN, FN_AFFINE_COS, FN_IDENTITY, FN_SINRAMP = 1, 2, 3, 4, 5, 6, 7
+# closure functions (SIGOPS_EFN_*): unary codes for FN1, binary codes (from 32) for FN2 / POPFN2
+EFN = {"abs": 1, "sign": 2, "floor": 3, "ceil": 4, "trunc": 5, "round": 6, "sqrt": 7, "clamp": 8, "exp": 9, "exp2": 10,
+       "expm1": 11, "log": 12, "log2": 13, "log10": 14, "log1p": 15, "sin": 16, "cos": 17, "tan": 18, "tanh": 19,
+       "sinh": 20, "cosh": 21, "atan": 22, "cbrt": 23,
+       "min": 32, "max": 33, "copysign": 34, "rem": 35, "mod": 36, "pow": 37, "hypot": 38}
+# leaves FN2 may take: the ones that do not read `fn` (generators and ramps keep their function there)
+FN2_LEAVES = (LEAF_CONST, LEAF_BUF, LEAF_CHANSUM, LEAF_RMS, LEAF_STAGE, LEAF_RANDN)
 STAGE_MAP, STAGE_IIR, STAGE_FIR = 1, 2, 3
 FIR_ARBITRARY, FIR_RATIONAL, FIR_DECIMATOR = 1, 2, 3
 MAX_STACK, MAX_PROG, MAX_PIECES, MAX_BUFS, MAX_SECTIONS = 4, 48, 64, 32, 8
@@ -216,9 +225,75 @@ def _stack_depth(prog):
         if I.op == OP_PUSH:
             sp += 1
             mx = max(mx, sp)
-        elif OP_POPADD <= I.op <= OP_POPDIV:
+        elif OP_POPADD <= I.op <= OP_POPDIV or I.op == OP_POPFN2:
             sp -= 1
     return mx
+
+
+class _TooLong(Exception):
+    pass
+
+
+def _traced_program(node, argprog, f32):
+    """Accumulator program computing the traced expression `node` (host/trace.py) from the programs of its
+    arguments.  IEEE results are kept: operands are never reassociated, only the exact swap of `+ * min max`
+    operands is used, and `c - v` becomes `-v + c` (the definition of subtraction).  A Float32 map rounds after
+    every operation, as the reference's Float32 arithmetic does.  Shared subexpressions are evaluated again."""
+    rnd = [Instr(op=OP_CAST_F32)] if f32 else []
+
+    def const(v):
+        return float(np.float32(v)) if f32 else float(v)     # numpy: a Python float meets Float32 samples as Float32
+
+    def leaf(p, ok=None):
+        return _isleaf(p) and (ok is None or p[0].leaf in ok)
+
+    def emit(nd):
+        out = _emit(nd)
+        if len(out) > MAX_PROG:
+            raise _TooLong
+        return out
+
+    def _emit(nd):
+        k = nd.kind
+        if k == "arg":
+            return list(argprog[nd.key])
+        if k == "const":
+            return [Instr(OP_LOAD, LEAF_CONST, d0=const(nd.value))]
+        if k == "neg":
+            return emit(nd.args[0]) + [Instr(op=OP_NEG)]
+        if k == "clamp":
+            lo, hi = nd.value
+            return emit(nd.args[0]) + [Instr(op=OP_FN1, fn=EFN[k], d0=const(lo), d1=const(hi))] + rnd
+        if len(nd.args) == 1:
+            return emit(nd.args[0]) + [Instr(op=OP_FN1, fn=EFN[k])] + rnd
+        pa, pb = emit(nd.args[0]), emit(nd.args[1])
+        if k in ("+", "*", "min", "max") and leaf(pa, (LEAF_CONST,)) and not leaf(pb, (LEAF_CONST,)):
+            pa, pb = pb, pa            # the sample first (`max(0, v)` as `max(v, 0)`): the fused filter forms want it so
+        if k in _ARITH_OPS:
+            direct, popop = _ARITH_OPS[k]
+            if leaf(pb):
+                return pa + [replace(pb[0], op=direct)] + rnd
+            if leaf(pa) and k in "+*":
+                return pb + [replace(pa[0], op=direct)] + rnd
+            if leaf(pa) and k == "-":
+                return pb + [Instr(op=OP_NEG), replace(pa[0], op=OP_ADD)] + rnd
+            return pa + [Instr(op=OP_PUSH)] + pb + [Instr(op=popop)] + rnd
+        code = EFN[k]
+        if leaf(pb, FN2_LEAVES):
+            return pa + [replace(pb[0], op=OP_FN2, fn=code)] + rnd
+        if leaf(pa, FN2_LEAVES) and k in ("min", "max"):
+            return pb + [replace(pa[0], op=OP_FN2, fn=code)] + rnd
+        return pa + [Instr(op=OP_PUSH)] + pb + [Instr(op=OP_POPFN2, fn=code)] + rnd
+
+    return emit(node)
+
+
+def _node_args(node, out):
+    if node.kind == "arg":
+        out.add(node.key)
+    for a in node.args:
+        _node_args(a, out)
+    return out
 
 
 def _intersect(a: Piece, b: Piece):
@@ -681,8 +756,7 @@ class Lowerer:
                 ps = self.lower(kids[0], shift, lo, hi, cm, co, clo, chi)
                 return [Piece(p.lo, p.hi, p.clo, p.chi, p.prog + [Instr(op=OP_NEG)]) for p in ps]
             if x.op not in _ARITH_OPS:
-                raise LoweringError(f"OperateOn({getattr(fn, '__name__', fn)!r}, ...) is not in the "
-                                    "enumerated operator set of the GPU sink")
+                return self._lower_traced(x, shift, lo, hi, cm, co, clo, chi)
             acc = self.lower(kids[0], shift, lo, hi, cm, co, clo, chi)
             if len(kids) == 1 and x.op == "-":
                 return [Piece(p.lo, p.hi, p.clo, p.chi, p.prog + [Instr(op=OP_NEG)]) for p in acc]
@@ -749,8 +823,76 @@ class Lowerer:
                 src = c * cm + co if cm else co
                 out += self.lower(kids[0], shift, lo, hi, 0, C - 1 - src, c, c + 1)
             return out
-        raise LoweringError("whole-frame OperateOn functions other than ToChannels/AddChannel/"
-                            "SelectChannel/reverse are not lowered to the GPU sink")
+        return self._lower_traced(x, shift, lo, hi, cm, co, clo, chi)
+
+    def _lower_traced(self, x, shift, lo, hi, cm, co, clo, chi):
+        """OperateOn with any other function: trace it (host/trace.py) and compile the expression.  By channel, one
+        expression serves every channel; a whole-frame closure (bychannel=false) gives one expression per output
+        channel, which becomes one piece per channel like `reverse`."""
+        kids = x.padded_signals
+        name = getattr(x.fn, "__name__", repr(x.fn))
+        try:
+            if x.bychannel:
+                roots = trace(x.fn, len(kids))
+            else:
+                roots = trace(x.fn, len(kids), [k.nchannels for k in kids])
+        except TraceError as e:
+            raise LoweringError(f"OperateOn({name}) cannot be compiled for the GPU sink: {e}") from None
+        T = np.dtype(x.sampletype)
+        f32 = T == np.float32
+        tail = [Instr(op=OP_CAST_I64)] if T.kind in "iub" else []
+        # (consumer channels, node channel map, expression) of each group of output channels
+        if x.bychannel:
+            groups = [(clo, chi, cm, co, roots)]
+        else:
+            groups = [(c, c + 1, 0, c * cm + co if cm else co, roots[c * cm + co if cm else co]) for c in range(clo, chi)]
+
+        def arg_pieces(key, a, b, gcm, gco, materialise):
+            k, ch = (key, None) if x.bychannel else key
+            kcm, kco = (gcm, gco) if ch is None else (0, ch)
+            kid = kids[k]
+            if materialise:
+                n = kid.nframes
+                if G.isknowninf(n):
+                    n = hi + shift
+                tag = self._materialize(kid, n)
+                return [Piece(lo, hi, a, b, [Instr(OP_LOAD, LEAF_BUF, buf=tag, c_mul=kcm, c_off=kco, i0=shift, i1=n)])]
+            return self.lower(kid, shift, lo, hi, kcm, kco, a, b)
+
+        def build(materialise):
+            out = []
+            for a, b, gcm, gco, root in groups:
+                combos = [(lo, hi, a, b, {})]
+                for key in sorted(_node_args(root, set()), key=repr):
+                    ps = arg_pieces(key, a, b, gcm, gco, key in materialise)
+                    if any(not _isleaf(p.prog) for p in ps):
+                        expressions.add(key)
+                    nxt = []
+                    for c0 in combos:
+                        for p in ps:
+                            r = _intersect(Piece(*c0[:4], None), p)
+                            if r:
+                                nxt.append((*r, {**c0[4], key: p.prog}))
+                    combos = nxt
+                for (plo, phi, pclo, pchi, argprog) in combos:
+                    prog = _traced_program(root, argprog, f32) + tail
+                    if len(prog) > MAX_PROG or _stack_depth(prog) > MAX_STACK:
+                        raise _TooLong
+                    out.append(Piece(plo, phi, pclo, pchi, prog))
+            return out
+
+        expressions = set()
+        try:
+            return build(set())
+        except _TooLong:
+            pass
+        # an argument used several times is evaluated each time: when that does not fit, the arguments that are
+        # expressions of their own are computed once into temps (as As1Channel does) and read back as buffers
+        try:
+            return build(set(expressions))
+        except _TooLong:
+            raise LoweringError(f"OperateOn({name}): the traced expression needs more than {MAX_PROG} operations "
+                                f"or nests deeper than the device stack ({MAX_STACK})") from None
 
     # ---- post passes -----------------------------------------------------------------------
     def _fuse_epilogues(self):

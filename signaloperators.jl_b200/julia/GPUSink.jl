@@ -208,6 +208,12 @@ const F32, F64, I64 = Int32(1), Int32(2), Int32(3)
 const OP_LOAD, OP_ADD, OP_SUB, OP_MUL, OP_DIV = UInt8(1), UInt8(2), UInt8(3), UInt8(4), UInt8(5)
 const OP_PUSH, OP_POPADD, OP_POPSUB, OP_POPMUL, OP_POPDIV = UInt8(6), UInt8(7), UInt8(8), UInt8(9), UInt8(10)
 const OP_NEG, OP_CAST_F32, OP_CAST_I64 = UInt8(11), UInt8(12), UInt8(13)
+const OP_FN1, OP_FN2, OP_POPFN2 = UInt8(14), UInt8(15), UInt8(16)
+# closure functions (SIGOPS_EFN_*): unary codes for FN1, binary codes (from 32) for FN2 / POPFN2
+const EFN = Dict{Symbol,UInt8}(:abs => 1, :sign => 2, :floor => 3, :ceil => 4, :trunc => 5, :round => 6, :sqrt => 7,
+    :clamp => 8, :exp => 9, :exp2 => 10, :expm1 => 11, :log => 12, :log2 => 13, :log10 => 14, :log1p => 15, :sin => 16,
+    :cos => 17, :tan => 18, :tanh => 19, :sinh => 20, :cosh => 21, :atan => 22, :cbrt => 23,
+    :min => 32, :max => 33, :copysign => 34, :rem => 35, :mod => 36, :pow => 37, :hypot => 38)
 const LEAF_NONE, LEAF_CONST, LEAF_BUF, LEAF_CHANSUM, LEAF_GEN = UInt8(0), UInt8(1), UInt8(2), UInt8(3), UInt8(4)
 const LEAF_RAMP_ON, LEAF_RAMP_OFF, LEAF_RMS, LEAF_STAGE, LEAF_RANDN = UInt8(5), UInt8(6), UInt8(7), UInt8(8), UInt8(9)
 const PAD_CONST, PAD_CYCLE, PAD_MIRROR, PAD_LAST = 0, 1, 2, 3
@@ -372,9 +378,97 @@ function stack_depth(prog)
     sp = mx = 0
     for I in prog
         I.op == OP_PUSH && (sp += 1; mx = max(mx, sp))
-        OP_POPADD <= I.op <= OP_POPDIV && (sp -= 1)
+        (OP_POPADD <= I.op <= OP_POPDIV || I.op == OP_POPFN2) && (sp -= 1)
     end
     mx
+end
+withfn(I::Instr, op, fn) = Instr(op, I.leaf, UInt8(fn), I.flags, I.buf, I.c_mul, I.c_off, I.i0, I.i1, I.i2, I.d0, I.d1, I.d2, I.d3, I.d4)
+
+# ---- traced OperateOn closures (host/trace.py) ----------------------------------------------------------------------
+# The closure is called once with `Traced` values standing for the samples; what it returns is an expression DAG over
+# the arguments (`:arg`, key = argument index or (argument, channel)) and Float64 constants.  Anything that needs a
+# sample's value (a comparison, and so `if`, `ifelse`, `isless`) throws a LoweringError naming it.
+struct TNode
+    kind::Symbol
+    args::Vector{TNode}
+    value::Any
+end
+struct Traced <: Real
+    node::TNode
+end
+tnode(x::Traced) = x.node
+tnode(x::Real) = TNode(:const, TNode[], Float64(x))
+traced(kind, xs...; value = nothing) = Traced(TNode(kind, TNode[tnode(x) for x in xs], value))
+for (f, k) in ((:+, :+), (:-, :-), (:*, :*), (:/, :/), (:min, :min), (:max, :max), (:copysign, :copysign), (:rem, :rem),
+               (:mod, :mod), (:hypot, :hypot), (:^, :pow))
+    @eval Base.$f(a::Traced, b::Traced) = traced($(QuoteNode(k)), a, b)
+    @eval Base.$f(a::Traced, b::Real) = traced($(QuoteNode(k)), a, b)
+    @eval Base.$f(a::Real, b::Traced) = traced($(QuoteNode(k)), a, b)
+end
+Base.:-(a::Traced) = traced(:neg, a)
+Base.:+(a::Traced) = a
+for f in (:abs, :sign, :floor, :ceil, :trunc, :sqrt, :exp, :exp2, :expm1, :log, :log2, :log10, :log1p, :sin, :cos, :tan,
+          :tanh, :sinh, :cosh, :atan, :cbrt)
+    @eval Base.$f(a::Traced) = traced($(QuoteNode(f)), a)
+end
+Base.round(a::Traced) = traced(:round, a)
+Base.round(a::Traced, ::RoundingMode{:Nearest}) = traced(:round, a)
+Base.round(a::Traced, ::RoundingMode{:Down}) = traced(:floor, a)
+Base.round(a::Traced, ::RoundingMode{:Up}) = traced(:ceil, a)
+Base.round(a::Traced, ::RoundingMode{:ToZero}) = traced(:trunc, a)
+Base.clamp(a::Traced, lo::Real, hi::Real) = Traced(TNode(:clamp, [tnode(a)], (Float64(lo), Float64(hi))))
+Base.literal_pow(::typeof(^), a::Traced, ::Val{2}) = a * a                  # Julia's x^2 is x*x
+Base.literal_pow(::typeof(^), a::Traced, ::Val{p}) where p = traced(:pow, a, p)
+Base.promote_rule(::Type{Traced}, ::Type{<:Real}) = Traced
+Base.float(a::Traced) = a
+refuse(what) = throw(LoweringError("$what on a traced sample: the GPU sink compiles the closure once for all samples, " *
+                                   "so it cannot depend on a sample's value"))
+for f in (:<, :<=, :isless, :(==), :isequal)
+    @eval Base.$f(::Traced, ::Traced) = refuse("a comparison ($($(string(f))), ifelse, if)")
+    @eval Base.$f(::Traced, ::Real) = refuse("a comparison ($($(string(f))), ifelse, if)")
+    @eval Base.$f(::Real, ::Traced) = refuse("a comparison ($($(string(f))), ifelse, if)")
+end
+Base.isnan(::Traced) = refuse("isnan")
+Base.signbit(::Traced) = refuse("signbit")
+Base.Bool(::Traced) = refuse("a conversion to Bool")
+
+targs!(out, nd::TNode) = (nd.kind === :arg && push!(out, nd.value); foreach(a -> targs!(out, a), nd.args); out)
+
+# accumulator program of a traced expression (lowering.py `_traced_program`): IEEE results kept, only the exact operand
+# swap of + * min max, constants meet Float32 samples as Float32, a Float32 map rounds after every operation
+function traced_program(nd::TNode, argprog, f32::Bool)
+    rnd = f32 ? [Instr(OP_CAST_F32)] : Instr[]
+    cval(v) = f32 ? Float64(Float32(v)) : Float64(v)
+    leaf(p, ok = nothing) = isleaf(p) && (ok === nothing || p[1].leaf in ok)
+    fn2ok = (LEAF_CONST, LEAF_BUF, LEAF_CHANSUM, LEAF_RMS, LEAF_STAGE, LEAF_RANDN)
+    function emit(nd)
+        out = emit1(nd)
+        length(out) > MAX_PROG && throw(LoweringError("traced expression of more than $MAX_PROG operations"))
+        out
+    end
+    function emit1(nd)
+        k = nd.kind
+        k === :arg && return copy(argprog[nd.value])
+        k === :const && return [Instr(OP_LOAD, LEAF_CONST; d0 = cval(nd.value))]
+        k === :neg && return vcat(emit(nd.args[1]), [Instr(OP_NEG)])
+        k === :clamp && return vcat(emit(nd.args[1]), [Instr(OP_FN1; fn = EFN[k], d0 = cval(nd.value[1]), d1 = cval(nd.value[2]))], rnd)
+        length(nd.args) == 1 && return vcat(emit(nd.args[1]), [Instr(OP_FN1; fn = EFN[k])], rnd)
+        pa, pb = emit(nd.args[1]), emit(nd.args[2])
+        if k in (:+, :*, :min, :max) && leaf(pa, (LEAF_CONST,)) && !leaf(pb, (LEAF_CONST,))
+            pa, pb = pb, pa
+        end
+        if k in (:+, :-, :*, :/)
+            f = k === :+ ? (+) : k === :- ? (-) : k === :* ? (*) : (/)
+            leaf(pb) && return vcat(pa, [withop(pb[1], ARITH[f][1])], rnd)
+            leaf(pa) && k in (:+, :*) && return vcat(pb, [withop(pa[1], ARITH[f][1])], rnd)
+            leaf(pa) && k === :- && return vcat(pb, [Instr(OP_NEG), withop(pa[1], OP_ADD)], rnd)
+            return vcat(pa, [Instr(OP_PUSH)], pb, [Instr(ARITH[f][2])], rnd)
+        end
+        leaf(pb, fn2ok) && return vcat(pa, [withfn(pb[1], OP_FN2, EFN[k])], rnd)
+        leaf(pa, fn2ok) && k in (:min, :max) && return vcat(pb, [withfn(pa[1], OP_FN2, EFN[k])], rnd)
+        vcat(pa, [Instr(OP_PUSH)], pb, [Instr(OP_POPFN2; fn = EFN[k])], rnd)
+    end
+    emit(nd)
 end
 function intersect_pieces(a::Piece, b::Piece)
     lo, hi, clo, chi = max(a.lo, b.lo), min(a.hi, b.hi), max(a.clo, b.clo), min(a.chi, b.chi)
@@ -569,7 +663,7 @@ function lower_node(lw, x::MapSignal, shift, lo, hi, cm, co, clo, chi)          
             cast = code == F32 ? OP_CAST_F32 : OP_CAST_I64
             return [Piece(p.lo, p.hi, p.clo, p.chi, vcat(p.prog, [Instr(cast)])) for p in ps]
         end
-        haskey(ARITH, fn) || throw(LoweringError("OperateOn($fn, ...) is not in the enumerated operator set of the GPU sink"))
+        haskey(ARITH, fn) || return lower_traced(lw, x, fn, kids, shift, lo, hi, cm, co, clo, chi)
         acc = lower_node(lw, kids[1], shift, lo, hi, cm, co, clo, chi)
         (length(kids) == 1 && fn === (-)) &&
             return [Piece(p.lo, p.hi, p.clo, p.chi, vcat(p.prog, [Instr(OP_NEG)])) for p in acc]
@@ -626,7 +720,65 @@ function lower_node(lw, x::MapSignal, shift, lo, hi, cm, co, clo, chi)          
         end
         return out
     end
-    throw(LoweringError("whole-frame OperateOn functions other than ToChannels/AddChannel/SelectChannel are not lowered to the GPU sink"))
+    lower_traced(lw, x, fn, kids, shift, lo, hi, cm, co, clo, chi)
+end
+
+# any other OperateOn function: trace it, compile the expression (lowering.py `_lower_traced`)
+function lower_traced(lw, x, fn, kids, shift, lo, hi, cm, co, clo, chi)
+    if x.bychannel
+        r = fn((Traced(TNode(:arg, TNode[], k - 1)) for k in eachindex(kids))...)
+        r isa Traced || throw(LoweringError("OperateOn($fn) did not return one traced value per sample"))
+        groups = [(clo, chi, cm, co, r.node)]
+    else
+        r = fn((Tuple(Traced(TNode(:arg, TNode[], (k - 1, c))) for c in 0:nchannels(kids[k])-1) for k in eachindex(kids))...)
+        roots = r isa Traced ? [r.node] : [tnode(v) for v in r]
+        groups = [(c, c + 1, 0, cm == 0 ? co : c * cm + co, roots[(cm == 0 ? co : c * cm + co) + 1]) for c in clo:chi-1]
+    end
+    T = sampletype(x)
+    f32 = T === Float32
+    tail = T <: Integer ? [Instr(OP_CAST_I64)] : Instr[]
+    function argpieces(key, a, b, gcm, gco, mat)
+        k, ch = x.bychannel ? (key, nothing) : key
+        kcm, kco = ch === nothing ? (gcm, gco) : (0, ch)
+        kid = kids[k+1]
+        if mat
+            n = isknowninf(nframes(kid)) ? hi + shift : nframes(kid)
+            tag = materialize!(lw, kid, n)
+            return [Piece(lo, hi, a, b, [Instr(OP_LOAD, LEAF_BUF; buf = tag, c_mul = kcm, c_off = kco, i0 = shift, i1 = n)])]
+        end
+        lower_node(lw, kid, shift, lo, hi, kcm, kco, a, b)
+    end
+    exprs = Set{Any}()
+    function build(mat)
+        out = Piece[]
+        for (a, b, gcm, gco, root) in groups
+            combos = [(lo, hi, a, b, Dict{Any,Vector{Instr}}())]
+            for key in sort!(collect(targs!(Set{Any}(), root)); by = repr)
+                ps = argpieces(key, a, b, gcm, gco, key in mat)
+                any(p -> !isleaf(p.prog), ps) && push!(exprs, key)
+                nxt = []
+                for c0 in combos, p in ps
+                    r = intersect_pieces(Piece(c0[1], c0[2], c0[3], c0[4], Instr[]), p)
+                    r === nothing || push!(nxt, (r..., merge(c0[5], Dict{Any,Vector{Instr}}(key => p.prog))))
+                end
+                combos = nxt
+            end
+            for (plo, phi, pclo, pchi, argprog) in combos
+                prog = vcat(traced_program(root, argprog, f32), tail)
+                (length(prog) > MAX_PROG || stack_depth(prog) > MAX_STACK) && return nothing
+                push!(out, Piece(plo, phi, pclo, pchi, prog))
+            end
+        end
+        out
+    end
+    out = try build(Set{Any}()) catch e; e isa LoweringError ? nothing : rethrow() end
+    out === nothing || return out
+    # an argument used several times is evaluated each time: when that does not fit, the arguments that are
+    # expressions of their own are computed once into temps and read back as buffers
+    out = try build(copy(exprs)) catch e; e isa LoweringError ? nothing : rethrow() end
+    out === nothing && throw(LoweringError("OperateOn($fn): the traced expression needs more than $MAX_PROG operations " *
+                                           "or nests deeper than the device stack ($MAX_STACK)"))
+    out
 end
 
 lower_node(lw, x, args...) = throw(LoweringError("cannot lower node of type $(typeof(x))"))

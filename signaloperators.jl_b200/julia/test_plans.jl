@@ -3,7 +3,8 @@
 # Run by a maintainer who has Julia, SignalOperators.jl 0.5 and DSP.jl 0.6 (none of which exist in this
 # repository's build image):
 #     julia --project -e 'include("signaloperators.jl_b200/julia/test_plans.jl")'
-# Each graph below is the Julia spelling of the graph of the same name in tests/golden/plans/make_plans.py.
+# Each graph below is the Julia spelling of the graph of the same name in tests/golden/plans/make_plans.py
+# (traced OperateOn closures: tests/golden/plans/make_fn_plans.py).
 # Everything the lowering decides (buffer shapes, instructions, pieces, stage wiring, integer fields) must
 # match exactly; numbers that DSP.jl produces on the Julia side and host/dspjl.py on the Python side (biquad
 # coefficients, polyphase banks, and the gain / rate / phase0 fields of a stage) must agree to 1e-12.
@@ -53,6 +54,13 @@ graphs = Dict(
         a = Signal(Z(50, 3), 10Hz)
         AddChannel(a |> SelectChannel(2), a |> ToChannels(1)) |> ToChannels(2) |> Amplify(2)
     end,
+    "envelope" => () -> OperateOn(abs, Signal(Z(48000, 2), 48kHz)) |> Filt(Lowpass, 50Hz),
+    "softclip" => () -> Signal(zeros(Float32, 48000, 2), 48kHz) |> Filt(Bandpass, 500Hz, 4kHz) |> Operate(v -> tanh(2f0 * v)),
+    "clamp" => () -> begin
+        x = Signal(Z(1000, 1), 10kHz)
+        Mix(OperateOn(v -> clamp(v, -1, 1), x), OperateOn(v -> max(v, 0), x))
+    end,
+    "midside" => () -> OperateOn(f -> (0.5(f[1] + f[2]), 0.5(f[1] - f[2])), Signal(Z(1000, 2), 10kHz), bychannel = false),
 )
 
 # section offsets of a plan (include/signalops.h)
