@@ -18,7 +18,10 @@
 //             Wc frames, where Wc is the number of frames after which that
 //             response has decayed below 2^-64 of its peak (Wc = L if it never
 //             does).  MAIN leaves those frames un-finalised; FIX applies the
-//             fused epilogue to them.
+//             fused epilogue to them.  The generic kernel k_iir instead leaves
+//             them unwritten and FIX reruns the cascade over them from s_in[k]:
+//             its output may be Float32, which cannot hold the zero-state
+//             values exactly until FIX adds the rest.
 // Superposition makes 1+3 equal to the sequential filter up to rounding.
 //
 // Roofline: 16 B/sample HBM (8 in + 8 out); 5 FP64 instructions per section per
@@ -80,20 +83,6 @@ struct Cascade {
         double y = x;
 #pragma unroll
         for (int j = 0; j < M; ++j) {
-            const double xi = y;
-            y = fma(b0[j], xi, s1[j]);
-            s1[j] = fma(-a1[j], y, fma(b1[j], xi, s2[j]));
-            s2[j] = fma(-a2[j], y, b2[j] * xi);
-        }
-        return y;
-    }
-    // same with x == 0 entering the first section
-    __device__ __forceinline__ double step_zero_input() {
-        double y = s1[0];
-        s1[0] = fma(-a1[0], y, s2[0]);
-        s2[0] = -a2[0] * y;
-#pragma unroll
-        for (int j = 1; j < M; ++j) {
             const double xi = y;
             y = fma(b0[j], xi, s1[j]);
             s1[j] = fma(-a1[j], y, fma(b1[j], xi, s2[j]));
@@ -340,25 +329,16 @@ k_iir(const __grid_constant__ IirParams P) {
         for (int r = 0; r < 32; r += kIirV) {
             const int64_t n0 = (chunk0 + r) * P.L + s * 32 + lane;
             double v[kIirV];
-            if (MODE == IIR_MAIN) {
-                if (P.plain_in_buf >= 0) {
-                    const BufRef ib = sbufs[P.plain_in_buf];
-#pragma unroll
-                    for (int j = 0; j < kIirV; ++j) {
-                        const int64_t n = n0 + j * P.L;
-                        v[j] = (n < P.plain_in_len) ? load_elem(ib.ptr, ib.dtype, (int64_t)c * ib.ld + n) : 0.0;
-                    }
-                } else {
-                    eval_program<kIirV>(sprog_in, lc_in, lr_in, P.in_prog_len, env, n0, P.L, c, nullptr, v,
-                                        stack + threadIdx.x, kIirThreads);
-                }
-            } else {
+            if (P.plain_in_buf >= 0) {
+                const BufRef ib = sbufs[P.plain_in_buf];
 #pragma unroll
                 for (int j = 0; j < kIirV; ++j) {
                     const int64_t n = n0 + j * P.L;
-                    v[j] = (n < P.N && chunk0 + r + j >= 1)
-                               ? load_elem(ob.ptr, ob.dtype, (int64_t)c * ob.ld + n) : 0.0;
+                    v[j] = (n < P.plain_in_len) ? load_elem(ib.ptr, ib.dtype, (int64_t)c * ib.ld + n) : 0.0;
                 }
+            } else {
+                eval_program<kIirV>(sprog_in, lc_in, lr_in, P.in_prog_len, env, n0, P.L, c, nullptr, v,
+                                    stack + threadIdx.x, kIirThreads);
             }
 #pragma unroll
             for (int j = 0; j < kIirV; ++j) tile[(r + j) * kTilePitch + lane] = v[j];
@@ -368,13 +348,8 @@ k_iir(const __grid_constant__ IirParams P) {
         // ---- compute phase: lane = chunk, 32 sequential frames
         {
             double* myrow = tile + lane * kTilePitch;
-            if (MODE == IIR_MAIN) {
 #pragma unroll
-                for (int k = 0; k < 32; ++k) myrow[k] = f.step(myrow[k]) * P.gain;
-            } else {
-#pragma unroll
-                for (int k = 0; k < 32; ++k) myrow[k] = fma(f.step_zero_input(), P.gain, myrow[k]);
-            }
+            for (int k = 0; k < 32; ++k) myrow[k] = f.step(myrow[k]) * P.gain;
         }
         __syncwarp();
 
@@ -396,19 +371,11 @@ k_iir(const __grid_constant__ IirParams P) {
             for (int j = 0; j < kIirV; ++j) {
                 const int64_t n = n0 + j * P.L;
                 const int64_t chunk = chunk0 + r + j;
-                if (n >= P.N) continue;
-                if (MODE == IIR_MAIN) {
-                    const bool unfinished = (chunk >= 1) && (s < nsub_raw);
-                    if (unfinished) {
-                        store_elem(ob.ptr, ob.dtype, (int64_t)c * ob.ld + n, y[j]);
-                    } else {
-                        const double w = store_elem(ob.ptr, ob.dtype, (int64_t)c * ob.ld + n, o[j]);
-                        ss += w * w;
-                    }
-                } else if (chunk >= 1) {
-                    const double w = store_elem(ob.ptr, ob.dtype, (int64_t)c * ob.ld + n, o[j]);
-                    ss += w * w;
-                }
+                // MAIN leaves the first Wc frames of chunks >= 1 to FIX; FIX writes nothing else
+                const bool fix_frame = (chunk >= 1) && (s < nsub_raw);
+                if (n >= P.N || fix_frame != (MODE == IIR_FIX)) continue;
+                const double w = store_elem(ob.ptr, ob.dtype, (int64_t)c * ob.ld + n, o[j]);
+                ss += w * w;
             }
         }
         __syncwarp();

@@ -392,7 +392,11 @@ void derive_iir(sigops_plan& p, StageRT& s, int idx) {
         for (int k = 0; k < 5; ++k) c[j][k] = t[j * 5 + k];
     s.iir.unitb = true;
     for (int j = 0; j < st.n_sections; ++j) s.iir.unitb = s.iir.unitb && c[j][0] == 1.0 && c[j][2] == 1.0;
-    s.iir.W = decay_length(c, st.n_sections, st.gain, std::max<int64_t>(32, std::min<int64_t>(st.n_out, 1 << 18)));
+    // The walk is capped (it costs O(cap * M^2) per plan).  A response still alive at the cap, an unstable filter's
+    // included, is taken to never decay: W = n_out keeps every chunker off WARM, and FIX then covers whole chunks.
+    const int64_t cap = std::max<int64_t>(32, std::min<int64_t>(st.n_out, 1 << 18));
+    s.iir.W = decay_length(c, st.n_sections, st.gain, cap);
+    if (s.iir.W >= cap) s.iir.W = std::max<int64_t>(cap, st.n_out);
     if (st.in_prog_len == 1) {
         const sigops_instr& I = p.instrs[st.in_prog_start];
         if (I.op == SIGOPS_OP_LOAD && I.leaf == SIGOPS_LEAF_BUF && I.i0 == 0 && I.c_mul == 1 && I.c_off == 0 &&
@@ -1176,9 +1180,10 @@ void plan_iir_stage(const Wave& w) {
     if (plan_iir_tmap(w, tma)) return;
     // (the program-carrying TMA kernel has no MAIN/FIX form: keep it to chunkings it can run)
     IirLaunch c = tma ? choose_iir_chunking_flat(s, rows, w.sm_count, !s.iir.tma_prog) : choose_iir_chunking(s, rows, w.sm_count);
-    // the program-carrying TMA kernel only exists in the single-launch WARM form
+    // the program-carrying TMA kernel only exists in the single-launch WARM form (for a filter that does not decay
+    // within the row that is one serial chunk per row: the generic kernel's carry pass does better)
     bool tprog = tma && s.iir.tma_prog;
-    if (tprog && c.need_matrix) {
+    if (tprog && (c.need_matrix || s.iir.W >= g.n_out)) {
         tma = tprog = false;
         c = choose_iir_chunking(s, rows, w.sm_count);
     }
