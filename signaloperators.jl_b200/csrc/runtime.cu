@@ -29,6 +29,7 @@
 #include "k_iir_carry.cuh"
 #include "k_fir.cuh"
 #include "k_fir_mma.cuh"
+#include "k_fir_long.cuh"
 #include "k_fir_tmap.cuh"
 #include "k_iir_tmap.cuh"
 #include "k_map.cuh"
@@ -212,6 +213,7 @@ struct FirDerived {
     int64_t period = 0;          // outputs after which index pattern and taps repeat (multiple of 32), 0 = they do not
     int64_t epoch_tiles = 0;     // the Float64 phase accumulator drifts (linearly, ~1e-15 per output): the period table is
     int64_t n_epochs = 0;        // rebuilt every epoch_tiles tiles so that the phase stays within 2e-10 of the table's
+    bool long_bank = false;      // k_fir's shared memory cannot hold the bank: the stage runs on k_fir_long
 };
 
 struct StageRT {
@@ -229,7 +231,8 @@ struct PlanDev {               // device-resident constants of a plan
     std::vector<int32_t*> poff;
     std::vector<double*> alpha;
     std::unordered_map<uint64_t, double*> carry;   // (stage, chunk length) -> device copy of the L-step transition matrix
-    std::unordered_map<uint64_t, double*> bands;   // (stage, ks) -> merged tap bands of one period (k_fir_tmap)
+    std::unordered_map<uint64_t, double*> bands;   // (stage, ks) -> merged tap bands of one period (k_fir_tmap);
+                                                   // (stage, 0) -> B fragments of a single-phase band (k_fir_long)
 };
 
 }  // namespace
@@ -504,6 +507,7 @@ constexpr size_t kFirSmemLimit = 200 * 1024;
 constexpr size_t kFirMmaSmemLimit = 220 * 1024;
 constexpr size_t kFirTmSmemLimit = 232448 - 512;   // 227 KB per block minus the kernel's static barriers
 constexpr int kFirT = 64;     // k_fir's tile (outputs), the table padding granularity (largest tile)
+constexpr int kFirMaxTaps = 65536;   // taps per phase: down-sampling to ~1/1800 of the rate, keeps every index in 32 bits
 
 // k_fir<G, 8> geometry: merged-tap rows, window pitch and dynamic shared memory.  Eight warps make a 64-output
 // tile (measured on B200, config 3: 3.8 ms against 4.7 ms with four warps and 32-output tiles — the smaller tile's
@@ -530,7 +534,8 @@ void derive_fir(sigops_plan& p, StageRT& s, int idx) {
     char what[64];
     snprintf(what, sizeof what, "stage %d (FIR)", idx);
     if (st.taps_per_phase < 1 || st.n_phases < 1) fail(SIGOPS_ERR_INVALID, "%s: empty filter bank", what);
-    if (st.taps_per_phase > 1024) fail(SIGOPS_ERR_UNSUPPORTED, "%s: %d taps per phase (<= 1024 supported)", what, st.taps_per_phase);
+    if (st.taps_per_phase > kFirMaxTaps)
+        fail(SIGOPS_ERR_UNSUPPORTED, "%s: %d taps per phase (<= %d supported)", what, st.taps_per_phase, kFirMaxTaps);
     auto check_table = [&](int id, const char* nm) {
         if (id < 0 || id >= (int)p.tables.size() || p.tables[id].count != (int64_t)st.n_phases * st.taps_per_phase)
             fail(SIGOPS_ERR_INVALID, "%s: %s table must hold n_phases*taps_per_phase doubles", what, nm);
@@ -679,9 +684,14 @@ void derive_fir(sigops_plan& p, StageRT& s, int idx) {
         ring = std::max(ring, need - p0);
     }
     s.fir.ring32 = (int)std::min<int64_t>(ring, 1 << 30);
-    if (fir_smem_bytes(s.fir, st.taps_per_phase, 1, SIGOPS_MAX_STACK) > kFirSmemLimit)
-        fail(SIGOPS_ERR_UNSUPPORTED, "%s: resampling ratio %g with %d taps/phase needs %zu bytes of shared memory per block",
-             what, st.rate, st.taps_per_phase, fir_smem_bytes(s.fir, st.taps_per_phase, 1, SIGOPS_MAX_STACK));
+    // A bank k_fir cannot hold in shared memory runs on k_fir_long, which takes what the lowering emits for such a
+    // stage: Float64 rows, no epilogue or a constant gain.
+    const size_t smem = fir_smem_bytes(s.fir, st.taps_per_phase, 1, SIGOPS_MAX_STACK);
+    s.fir.long_bank = smem > kFirSmemLimit;
+    if (s.fir.long_bank && !(s.fir.epi_const && p.bufs[s.fir.in_buf].dtype == SIGOPS_F64 && p.bufs[st.out_buf].dtype == SIGOPS_F64))
+        fail(SIGOPS_ERR_UNSUPPORTED, "%s: resampling ratio %g with %d taps/phase needs %zu bytes of shared memory per block in the "
+             "scalar kernel, and the long-filter kernel takes Float64 rows with no epilogue or a constant gain only",
+             what, st.rate, st.taps_per_phase, smem);
 }
 
 void parse_plan(sigops_plan& p, const void* bytes, size_t nbytes) {
@@ -1382,8 +1392,78 @@ bool plan_fir_mma(const Wave& w, const FirParams& P) {
     return true;
 }
 
+// B fragments of the band every 8-output group of a single-phase stage shares (k_fir_long, BK_TAB): output n of a
+// group reads q*n positions after output 0, so Band[k][n] = gain * h[k - q*n].  Lane (rr, kk) of chunk c takes
+// Band[8c + kk][rr] and Band[8c + kk + 4][rr].  Built and uploaded once per plan, stage and device.
+const double2* long_band(const Wave& w, int nchunks) {
+    const uint64_t key = (uint64_t)w.si << 16;
+    auto it = w.pd.bands.find(key);
+    if (it != w.pd.bands.end()) return reinterpret_cast<const double2*>(it->second);
+    const sigops_plan& p = w.p;
+    const StageRT& s = p.stages[w.si];
+    const sigops_stage& g = s.st;
+    const double* h = p.blob.data() + p.tables[g.pfb_table].offset;
+    const int64_t q = g.decimation, T = g.taps_per_phase;
+    std::vector<double> tab((size_t)nchunks * 64, 0.0);
+    for (int64_t c = 0; c < nchunks; ++c)
+        for (int lane = 0; lane < 32; ++lane)
+            for (int e = 0; e < 2; ++e) {
+                const int64_t t = 8 * c + (lane & 3) + 4 * e - q * (lane >> 2);
+                if (t >= 0 && t < T) tab[(size_t)(c * 32 + lane) * 2 + e] = h[t] * s.fir.epi_scale;
+            }
+    double* dptr = nullptr;
+    CUDA_OK(cudaMalloc(&dptr, tab.size() * sizeof(double)));
+    CUDA_OK(cudaMemcpy(dptr, tab.data(), tab.size() * sizeof(double), cudaMemcpyHostToDevice));
+    w.pd.bands.emplace(key, dptr);
+    return reinterpret_cast<const double2*>(dptr);
+}
+
+// Long-bank FIR kernel (k_fir_long.cuh): the stages whose bank k_fir cannot hold in shared memory.
+void plan_fir_long(const Wave& w, const FirParams& P) {
+    const StageRT& s = w.p.stages[w.si];
+    const sigops_stage& g = s.st;
+    const int64_t rows = P.nrows;
+    const bool tab = g.fir_kind == SIGOPS_FIR_DECIMATOR;
+    FirLongParams Q{};
+    Q.bufrefs = w.d_refs; Q.scalars = w.scalars; Q.nbuf = w.nbuf; Q.nscalars = w.nscal;
+    Q.in_buf = s.fir.in_buf; Q.out_buf = g.out_buf; Q.sumsq_slot = g.sumsq_slot;
+    Q.in_len = s.fir.in_len; Q.nch = g.nchannels; Q.nrows = rows; Q.n_out = g.n_out;
+    Q.tapsper = g.taps_per_phase;
+    // a group's band: its last output's window ends dpad positions after its first output's
+    const int64_t dpad = tab ? 7 * (int64_t)g.decimation : s.fir.dpad;
+    const int64_t ks = round_up(dpad + g.taps_per_phase, 8);
+    if (ks > (int64_t(1) << 30)) fail(SIGOPS_ERR_UNSUPPORTED, "FIR stage %zu: band of %lld positions", w.si, (long long)ks);
+    Q.nchunks = (int)(ks / 8);
+    Q.xi0 = P.xi0; Q.poff = w.pd.poff[w.si]; Q.alpha = w.pd.alpha[w.si];
+    Q.pfb = P.pfb; Q.dpfb = P.dpfb;
+    Q.band = tab ? long_band(w, Q.nchunks) : nullptr;
+    Q.gain = tab ? 1.0 : s.fir.epi_scale;
+    // rows per block: four 8-row fragments per warp, one where the batch has no more than 8 rows
+    const int MF = rows > 8 ? 4 : 1, RB = 8 * MF;
+    const int64_t tiles = (g.n_out + kFlT - 1) / kFlT, groups = (rows + RB - 1) / RB;
+    if (groups > 65535) fail(SIGOPS_ERR_UNSUPPORTED, "FIR stage over more than %d rows per wave", 65535 * RB);
+    const size_t smem = (size_t)RB * kFlPitch * sizeof(double);
+    dim3 grid((unsigned)tiles, (unsigned)groups);
+    if (getenv("SIGOPS_DEBUG"))
+        fprintf(stderr, "[sigops] FIR stage %zu: long rows=%lld n_out=%lld taps=%d ks=%lld segment=%d grid=%lldx%lld rows/block=%d bank=%s smem=%zu\n",
+                w.si, (long long)rows, (long long)g.n_out, g.taps_per_phase, (long long)ks, kFlSeg, (long long)tiles,
+                (long long)groups, RB, tab ? "table" : (P.dpfb ? "merged" : "gathered"), smem);
+    const bool ssq = g.sumsq_slot >= 0;
+    const int bk = tab ? BK_TAB : (P.dpfb ? BK_MERGE : BK_BANK);
+    using K = void (*)(FirLongParams);
+    static const K kernels[2][3][2] = {
+        {{k_fir_long<1, BK_TAB, false>, k_fir_long<1, BK_TAB, true>},
+         {k_fir_long<1, BK_BANK, false>, k_fir_long<1, BK_BANK, true>},
+         {k_fir_long<1, BK_MERGE, false>, k_fir_long<1, BK_MERGE, true>}},
+        {{k_fir_long<4, BK_TAB, false>, k_fir_long<4, BK_TAB, true>},
+         {k_fir_long<4, BK_BANK, false>, k_fir_long<4, BK_BANK, true>},
+         {k_fir_long<4, BK_MERGE, false>, k_fir_long<4, BK_MERGE, true>}}};
+    const K kernel = kernels[MF == 4][bk][ssq];
+    w.add(KIND_FIR, [=](cudaStream_t st) { launch_dyn_smem(kernel, grid, kFlGroups * 32, smem, st, Q); });
+}
+
 // FIR: the tensor-core kernels for plain Float64 rows on 16-byte boundaries with no epilogue or a constant gain
-// (k_fir_tmap, else k_fir_mma), else the scalar-FMA kernel k_fir.
+// (k_fir_tmap, else k_fir_mma), else the scalar-FMA kernel k_fir; banks k_fir cannot hold take k_fir_long.
 void plan_fir_stage(const Wave& w) {
     const sigops_plan& p = w.p;
     const StageRT& s = p.stages[w.si];
@@ -1401,6 +1481,10 @@ void plan_fir_stage(const Wave& w) {
     P.pfb = w.pd.blob + p.tables[g.pfb_table].offset;
     P.dpfb = g.dpfb_table >= 0 ? w.pd.blob + p.tables[g.dpfb_table].offset : nullptr;
     P.xi0 = w.pd.xi0[w.si]; P.phi = w.pd.phi[w.si];
+    if (s.fir.long_bank) {
+        plan_fir_long(w, P);
+        return;
+    }
     const bool mma = s.fir.epi_const && !getenv("SIGOPS_NO_FIR_MMA") &&
                      p.bufs[s.fir.in_buf].dtype == SIGOPS_F64 && p.bufs[g.out_buf].dtype == SIGOPS_F64 &&
                      rows_aligned(w.refs, w.ninst, w.nbuf, s.fir.in_buf, true) && rows_aligned(w.refs, w.ninst, w.nbuf, g.out_buf, true);
