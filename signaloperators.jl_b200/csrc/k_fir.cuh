@@ -29,7 +29,7 @@
 // FMAs per sample after merging (SURVEY.md §8d).
 #pragma once
 #include "interp.cuh"
-#include "k_iir.cuh"   // cp_async8 / cp_async_wait_all
+#include "ptx.cuh"
 
 namespace sigops {
 
@@ -60,11 +60,6 @@ struct FirParams {
     const double* phi;
     int64_t inst0;             // index of the wave's first instance in the whole call (noise streams)
 };
-
-__device__ __forceinline__ void cp_async16(double* smem_dst, const double* gmem_src, int src_bytes) {
-    const unsigned dst = (unsigned)__cvta_generic_to_shared(smem_dst);
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(gmem_src), "r"(src_bytes) : "memory");
-}
 
 template <int G, int W>
 __global__ void __launch_bounds__(W * 32)
@@ -176,7 +171,7 @@ k_fir(const __grid_constant__ FirParams P) {
         }
     }
     for (int i = tid; i < RB * 8; i += kFirThreads) xs[(size_t)(i >> 3) * P.xpitch + ncopy_e + (i & 7)] = 0.0;
-    asm volatile("cp.async.commit_group;" ::: "memory");
+    cp_async_commit();
 
     // ---- 2. merged taps while the copies fly: 4 threads per output
     for (int i = tid; i < P.epi_prog_len; i += kFirThreads) {
@@ -214,7 +209,8 @@ k_fir(const __grid_constant__ FirParams P) {
             for (int t = sub; t < P.tapsper; t += 4) hrow[base + t] = 0.0;
         }
     }
-    cp_async_wait_all();
+    cp_async_commit();
+    cp_async_wait_group<0>();
     __syncthreads();
 
     // ---- 3. register-tiled dot products: 8 outputs x G rows per thread, two positions per step

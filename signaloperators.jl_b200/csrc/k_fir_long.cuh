@@ -32,8 +32,8 @@
 //                is two DMMAs per chunk (k = outputs 0..3, 4..7) that hand their result straight to the product.
 //     The constant gain of the multi-phase kinds is applied to the finished outputs (once per output, not per tap).
 #pragma once
-#include "k_fir_mma.cuh"   // dmma884, mbar_arrive, mbarrier / bulk-copy helpers
-#include "k_iir.cuh"       // cp_async8
+#include "interp.cuh"
+#include "ptx.cuh"
 
 namespace sigops {
 
@@ -65,10 +65,6 @@ struct FirLongParams {
     const double2* band;    // BK_TAB: [nchunks][32] B fragments of the common band, gain folded in
     double gain;            // constant-gain epilogue of the multi-phase kinds (1.0 = none)
 };
-
-__device__ __forceinline__ void cp_async_mbar_arrive(uint64_t* bar) {
-    asm volatile("cp.async.mbarrier.arrive.shared::cta.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
 
 template <int MF, int BK, bool SSQ>
 __global__ void __launch_bounds__(kFlGroups * 32, 2)
@@ -106,7 +102,7 @@ k_fir_long(const __grid_constant__ FirLongParams P) {
     }
     if (tid == 0) {
         for (int i = 0; i < kFlSlots; ++i) mbar_init(&bar[i], RB);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        fence_mbarrier_init();
     }
     __syncthreads();
 
@@ -233,9 +229,7 @@ k_fir_long(const __grid_constant__ FirLongParams P) {
             }
         }
         if (SSQ) {
-            double ss = (m < P.n_out ? v0 * v0 : 0.0) + (m + 1 < P.n_out ? v1 * v1 : 0.0);
-            ss += __shfl_xor_sync(0xffffffffu, ss, 1);
-            ss += __shfl_xor_sync(0xffffffffu, ss, 2);
+            const double ss = quad_sum((m < P.n_out ? v0 * v0 : 0.0) + (m + 1 < P.n_out ? v1 * v1 : 0.0));
             if (kk == 0 && dst) atomicAdd(P.scalars + (size_t)s_inst[rr + 8 * i] * P.nscalars + P.sumsq_slot, ss);
         }
     }

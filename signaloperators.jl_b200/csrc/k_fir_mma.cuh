@@ -50,7 +50,7 @@
 // k_fir_tmap.cuh instead (tensor-map loads and stores).
 #pragma once
 #include "interp.cuh"
-#include "k_iir_tma.cuh"   // mbarrier / bulk-copy helpers
+#include "ptx.cuh"
 
 namespace sigops {
 
@@ -82,15 +82,6 @@ struct FirMmaParams {
     int tab_doubles;        // nphases*tapsper: both banks are copied to shared memory
     double gain;            // constant-gain epilogue folded into the taps (1.0 = none)
 };
-
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-
-__device__ __forceinline__ void dmma884(double& c0, double& c1, double a, double b) {
-    asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
-                 : "+d"(c0), "+d"(c1) : "d"(a), "d"(b));
-}
 
 // MF = 8-row fragments per compute warp, RH = compute warps per output group (row slices), SSQ =
 // accumulate the sum of squares for a following Normpower (costs the compute warps 2*MF registers):
@@ -148,7 +139,7 @@ k_fir_mma(const __grid_constant__ FirMmaParams P) {
         mbar_init(&bar_taps[1], kAuxThreads);
         mbar_init(&bar_done[0], NCW);
         mbar_init(&bar_done[1], NCW);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        fence_mbarrier_init();
     }
     fence_async_smem();
     __syncthreads();
@@ -399,9 +390,7 @@ k_fir_mma(const __grid_constant__ FirMmaParams P) {
         if (SSQ) {
 #pragma unroll
             for (int i = 0; i < (SSQ ? MF : 1); ++i) {
-                double v = ssq[i];
-                v += __shfl_xor_sync(0xffffffffu, v, 1);
-                v += __shfl_xor_sync(0xffffffffu, v, 2);
+                const double v = quad_sum(ssq[i]);
                 if (kk == 0 && dstp[i]) atomicAdd(P.scalars + (size_t)s_inst[rbase + 8 * i] * P.nscalars + P.sumsq_slot, v);
             }
         }

@@ -41,11 +41,10 @@
 // constant gain, band <= 64 positions, a tile's window within the ring.  Everything else takes
 // k_fir_mma / k_fir.  SIGOPS_NO_FIR_TMAP=1 switches this kernel off.
 #pragma once
-#include <cuda.h>
-
 #include <type_traits>
 
-#include "k_fir_mma.cuh"
+#include "k_fir_mma.cuh"   // kFmT
+#include "ptx.cuh"
 
 namespace sigops {
 
@@ -89,42 +88,8 @@ inline size_t fir_tm_smem_bytes(int nslot, int ks, int tab_doubles, bool has_dpf
 }
 
 // The dynamic shared memory of this kernel is addressed through 32-bit shared-window addresses and
-// explicit ld.shared / st.shared: the 1024-byte alignment of the swizzled boxes is computed on the
-// address, and a pointer rebuilt from it would make every access a generic LD/ST.
-__device__ __forceinline__ void tmap_load_2d(unsigned smem_dst, const CUtensorMap* tm, int c0, int c1, uint64_t* bar) {
-    asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];" ::"r"(smem_dst),
-                 "l"(tm), "r"(c0), "r"(c1), "r"(smem_u32(bar))
-                 : "memory");
-}
-__device__ __forceinline__ void tmap_store_2d(const CUtensorMap* tm, int c0, int c1, unsigned smem_src) {
-    asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%1, %2}], [%3];" ::"l"(tm), "r"(c0), "r"(c1), "r"(smem_src)
-                 : "memory");
-}
-__device__ __forceinline__ double lds_f64(unsigned a) {
-    double v;
-    asm volatile("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"(a));
-    return v;
-}
-__device__ __forceinline__ void sts_f64(unsigned a, double v) { asm volatile("st.shared.f64 [%0], %1;" ::"r"(a), "d"(v) : "memory"); }
-__device__ __forceinline__ void sts_v2f64(unsigned a, double x, double y) {
-    asm volatile("st.shared.v2.f64 [%0], {%1, %2};" ::"r"(a), "d"(x), "d"(y) : "memory");
-}
-
-__device__ __forceinline__ void mbar_wait_a(unsigned bar, unsigned parity) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "LAB_WAIT:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@p bra LAB_DONE;\n"
-        "bra LAB_WAIT;\n"
-        "LAB_DONE:\n"
-        "}\n" ::"r"(bar), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_a(unsigned bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-
+// explicit ld.shared / st.shared (lds_f64, sts_f64, sts_v2f64): the 1024-byte alignment of the swizzled
+// boxes is computed on the address, and a pointer rebuilt from it would make every access a generic LD/ST.
 template <bool SSQ, bool DBG = false>
 __global__ void __launch_bounds__(kFtThreads, 1)
 k_fir_tmap(const __grid_constant__ FirTmParams P, const __grid_constant__ CUtensorMap tm_in,
@@ -163,7 +128,7 @@ k_fir_tmap(const __grid_constant__ FirTmParams P, const __grid_constant__ CUtens
             mbar_init(&bar_stg_full[i], kFtNCW / 2);
             mbar_init(&bar_stg_free[i], 1);
         }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        fence_mbarrier_init();
     }
     fence_async_smem();
     __syncthreads();
@@ -270,7 +235,7 @@ k_fir_tmap(const __grid_constant__ FirTmParams P, const __grid_constant__ CUtens
             // one barrier per tile: the helpers arrive on it once the tile's band is built AND its ring slots
             // have landed (they watch the `full` barriers, off the compute warps' path)
             const long long c0 = DBG ? clock64() : 0;
-            if (!(P.exp & 16)) mbar_wait_a(a_taps + 8u * s, (unsigned)(u >> 1) & 1u);
+            if (!(P.exp & 16)) mbar_wait(a_taps + 8u * s, (unsigned)(u >> 1) & 1u);
             if (DBG) dbg_acc[0] += clock64() - c0;
             load_ops(o, std::integral_constant<int, 0>{});
             if (DBG) dbg_acc[1] += clock64() - cs;
@@ -285,7 +250,7 @@ k_fir_tmap(const __grid_constant__ FirTmParams P, const __grid_constant__ CUtens
         // until they have drained through the LSU queue (~400 cycles per tile, measured).
         auto stage_store = [&](double (&o)[F][2], int u_old) {
             const long long c0 = DBG ? clock64() : 0;
-            if (u_old > 0) mbar_wait_a(a_free, (unsigned)(u_old - 1) & 1u);
+            if (u_old > 0) mbar_wait(a_free, (unsigned)(u_old - 1) & 1u);
             if (DBG) dbg_acc[2] += clock64() - c0;
             if (!(P.exp & 1)) {
                 const unsigned sp = srow + (gw >> 1) * 16384 + ((unsigned)(((gw & 1) * 4 + kk) << 4) ^ key);
@@ -303,7 +268,7 @@ k_fir_tmap(const __grid_constant__ FirTmParams P, const __grid_constant__ CUtens
             const long long c0 = DBG ? clock64() : 0;
             fence_async_smem();
             __syncwarp();
-            if (lead) mbar_arrive_a(a_full);
+            if (lead) mbar_arrive(a_full);
             if (DBG) dbg_acc[3] += clock64() - c0;
         };
         // One tile: its DMMAs accumulate into `acc` while the fragments of the tile before it (`old`) drain to
@@ -373,7 +338,7 @@ k_fir_tmap(const __grid_constant__ FirTmParams P, const __grid_constant__ CUtens
             if (!signalled) stage_signal();               // (tiles of fewer than four blocks)
             __syncwarp();
             if (lead) {
-                mbar_arrive_a(a_done + 8u * (u & 3));
+                mbar_arrive(a_done + 8u * (u & 3));
                 asm volatile("red.release.cta.shared::cta.add.u32 [%0], 1;" ::"r"(a_cnt) : "memory");
             }
         };
@@ -395,9 +360,7 @@ k_fir_tmap(const __grid_constant__ FirTmParams P, const __grid_constant__ CUtens
         if (SSQ) {
 #pragma unroll
             for (int i = 0; i < F; ++i) {
-                double v = ssq[i];
-                v += __shfl_xor_sync(0xffffffffu, v, 1);
-                v += __shfl_xor_sync(0xffffffffu, v, 2);
+                const double v = quad_sum(ssq[i]);
                 const int64_t row = (int64_t)row0 + rloc + 8 * i;
                 if (kk == 0 && row < P.nrows) atomicAdd(P.scalars + (size_t)(row / P.nch) * P.nscalars + P.sumsq_slot, v);
             }
@@ -433,10 +396,7 @@ k_fir_tmap(const __grid_constant__ FirTmParams P, const __grid_constant__ CUtens
                     int64_t ep = t / P.epoch_tiles;
                     ep = ep < P.n_epochs ? ep : P.n_epochs - 1;
                     const double* src = P.bands_g + (size_t)(ep * P.period_tiles + t % P.period_tiles) * (bytes / 8);
-                    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                                     bands + (unsigned)s * band_tile),
-                                 "l"(src), "r"(bytes), "r"(smem_u32(&bar_taps[s]))
-                                 : "memory");
+                    bulk_load(bands + (unsigned)s * band_tile, src, bytes, smem_u32(&bar_taps[s]));
                     while (jwait < hi && !(P.exp & 8)) {                                          // ... and the tile's window has landed
                         mbar_wait(&bar_full[jw_slot], jw_par);
                         ++jwait;

@@ -27,14 +27,15 @@
 // Roofline: 16 B/sample HBM (8 in + 8 out); 5 FP64 instructions per section per
 // sample (SURVEY.md §8d: "FP64 pipe ~ HBM").
 #pragma once
+#include "biquad.cuh"
 #include "interp.cuh"
+#include "ptx.cuh"
 
 namespace sigops {
 
 constexpr int kIirWarps = 4;
 constexpr int kIirThreads = kIirWarps * 32;
 constexpr int kIirV = 4;
-constexpr int kIirMaxSections = 8;
 constexpr int kTilePitch = 33;
 
 struct IirParams {
@@ -66,64 +67,7 @@ struct IirParams {
 
 enum { IIR_MAIN = 0, IIR_FIX = 1, IIR_WARM = 2 };
 
-template <int M>
-struct Cascade {
-    double b0[M], b1[M], b2[M], a1[M], a2[M];
-    double s1[M], s2[M];
-    __device__ __forceinline__ void init(const IirParams& P) {
-#pragma unroll
-        for (int j = 0; j < M; ++j) {
-            b0[j] = P.coef[j][0]; b1[j] = P.coef[j][1]; b2[j] = P.coef[j][2];
-            a1[j] = P.coef[j][3]; a2[j] = P.coef[j][4];
-            s1[j] = 0.0; s2[j] = 0.0;
-        }
-    }
-    // DSP.jl `_filt!` for SecondOrderSections (DF2T), SURVEY.md App. B.2
-    __device__ __forceinline__ double step(double x) {
-        double y = x;
-#pragma unroll
-        for (int j = 0; j < M; ++j) {
-            const double xi = y;
-            y = fma(b0[j], xi, s1[j]);
-            s1[j] = fma(-a1[j], y, fma(b1[j], xi, s2[j]));
-            s2[j] = fma(-a2[j], y, b2[j] * xi);
-        }
-        return y;
-    }
-};
-
-__device__ __forceinline__ void cp_async8(double* smem_dst, const double* gmem_src, bool valid) {
-    const unsigned dst = (unsigned)__cvta_generic_to_shared(smem_dst);
-    const int src_size = valid ? 8 : 0;       // src_size 0 => the 8 bytes are zero-filled, nothing is read
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 8, %2;" ::"r"(dst), "l"(gmem_src), "r"(src_size) : "memory");
-}
-__device__ __forceinline__ void cp_async_wait_all() {
-    asm volatile("cp.async.commit_group;\ncp.async.wait_group 0;" ::: "memory");
-}
-
-// One section update (DSP.jl `_filt!` inner body, SURVEY.md App. B.2).  UNITB: the
-// section has b0 == 1 and b2 == 1 exactly (every zero on the unit circle, which is
-// what the Butterworth/Chebyshev designs give), so `b0*x` and `b2*x` are skipped
-// without changing a single bit of the result.
-template <int M, bool UNITB>
-__device__ __forceinline__ double biquad_step(Cascade<M>& f, int j, double xi) {
-    double y;
-    if (UNITB) {
-        y = xi + f.s1[j];
-        f.s1[j] = fma(-f.a1[j], y, fma(f.b1[j], xi, f.s2[j]));
-        f.s2[j] = fma(-f.a2[j], y, xi);
-    } else {
-        y = fma(f.b0[j], xi, f.s1[j]);
-        f.s1[j] = fma(-f.a1[j], y, fma(f.b1[j], xi, f.s2[j]));
-        f.s2[j] = fma(-f.a2[j], y, f.b2[j] * xi);
-    }
-    return y;
-}
-
-// NT frames of one chunk through the cascade, software-pipelined across sections:
-// at step t section j works on frame t-j, so the M updates of a step are mutually
-// independent (M-way ILP on the FP64 pipe) while every frame still sees exactly the
-// sequential recurrence.  ZERO_IN: the first section's input is 0 (FIX pass).
+// NT frames of one chunk through the cascade (cascade_frames), in place in the lane's shared-memory row.
 // out = in_tile + (cascade * gain) for FIX, (cascade * gain) * sc for MAIN.
 template <int M, int NT, bool ZERO_IN, bool UNITB>
 __device__ __forceinline__ void cascade_tile(Cascade<M>& f, double* myrow, double gain, double sc) {
@@ -133,23 +77,10 @@ __device__ __forceinline__ void cascade_tile(Cascade<M>& f, double* myrow, doubl
 #pragma unroll
     for (int k = 0; k < NT; ++k) xr[k] = myrow[k];
     double pipe[M];
-#pragma unroll
-    for (int t = 0; t < NT + M - 1; ++t) {
-#pragma unroll
-        for (int j = M - 1; j >= 0; --j) {     // descending: section j reads pipe[j-1] of step t-1
-            const int k = t - j;
-            if (k >= 0 && k < NT) {
-                const double in = (j == 0) ? (ZERO_IN ? 0.0 : xr[k]) : pipe[j - 1];
-                pipe[j] = biquad_step<M, UNITB>(f, j, in);
-                if (j == M - 1) myrow[k] = ZERO_IN ? fma(pipe[j], gain, xr[k]) * sc : (pipe[j] * gain) * sc;
-            }
-        }
-    }
+    cascade_frames<M, NT, ZERO_IN, UNITB>(f, xr, pipe, [&](int k, double y) {
+        myrow[k] = ZERO_IN ? fma(y, gain, xr[k]) * sc : (y * gain) * sc;
+    });
 }
-
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait_group() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
 constexpr int kHalfCols = 16;          // frames per half-tile
 constexpr int kHalfPitch = 17;         // doubles; odd pitch keeps lane=row accesses conflict-free
@@ -183,16 +114,8 @@ k_iir_fast(const __grid_constant__ IirParams P) {
     const bool interior = (chunk0 + 32) * P.L <= nvalid;
 
     Cascade<M> f;
-    f.init(P);
-    if (MODE == IIR_FIX && mychunk >= 1) {
-        const double* sin_ = P.carry_is_shift ? P.state_zs : P.state_in;
-        const int64_t src = P.carry_is_shift ? slot - 1 : slot;
-#pragma unroll
-        for (int j = 0; j < M; ++j) {
-            f.s1[j] = sin_[(2 * j) * nslots + src];
-            f.s2[j] = sin_[(2 * j + 1) * nslots + src];
-        }
-    }
+    f.init(P.coef);
+    if (MODE == IIR_FIX && mychunk >= 1) load_carried_state(f, P, nslots, slot);
     const int64_t L = P.L;
     const int64_t nh_raw = P.Wc / kHalfCols;
     const int64_t nh = (MODE == IIR_FIX) ? nh_raw : L / kHalfCols;
@@ -264,13 +187,7 @@ k_iir_fast(const __grid_constant__ IirParams P) {
         __syncwarp();
     }
 
-    if (MODE == IIR_MAIN) {
-#pragma unroll
-        for (int j = 0; j < M; ++j) {
-            P.state_zs[(2 * j) * nslots + slot] = f.s1[j];
-            P.state_zs[(2 * j + 1) * nslots + slot] = f.s2[j];
-        }
-    }
+    if (MODE == IIR_MAIN) store_final_state(f, P.state_zs, nslots, slot);
     if (P.sumsq_slot >= 0) {
         ss = warp_sum(ss);
         if (lane == 0) atomicAdd(P.scalars + (size_t)inst * P.nscalars + P.sumsq_slot, ss);
@@ -307,16 +224,8 @@ k_iir(const __grid_constant__ IirParams P) {
     if (chunk0 * P.L >= P.N) return;      // whole warp past the end (warp-uniform)
 
     Cascade<M> f;
-    f.init(P);
-    if (MODE == IIR_FIX && mychunk >= 1) {
-        const double* sin_ = P.carry_is_shift ? P.state_zs : P.state_in;
-        const int64_t src = P.carry_is_shift ? slot - 1 : slot;
-#pragma unroll
-        for (int j = 0; j < M; ++j) {
-            f.s1[j] = sin_[(2 * j) * nslots + src];
-            f.s2[j] = sin_[(2 * j + 1) * nslots + src];
-        }
-    }
+    f.init(P.coef);
+    if (MODE == IIR_FIX && mychunk >= 1) load_carried_state(f, P, nslots, slot);
 
     const BufRef ob = sbufs[P.out_buf];
     const int64_t nsub_all = P.L / 32, nsub_raw = P.Wc / 32;
@@ -381,13 +290,7 @@ k_iir(const __grid_constant__ IirParams P) {
         __syncwarp();
     }
 
-    if (MODE == IIR_MAIN) {
-#pragma unroll
-        for (int j = 0; j < M; ++j) {
-            P.state_zs[(2 * j) * nslots + slot] = f.s1[j];
-            P.state_zs[(2 * j + 1) * nslots + slot] = f.s2[j];
-        }
-    }
+    if (MODE == IIR_MAIN) store_final_state(f, P.state_zs, nslots, slot);
     if (P.sumsq_slot >= 0) {
         ss = warp_sum(ss);
         if (lane == 0) atomicAdd(P.scalars + (size_t)inst * P.nscalars + P.sumsq_slot, ss);

@@ -1,6 +1,6 @@
 // Cross-chunk state propagation for the MAIN + CARRY + FIX decomposition (see k_iir.cuh).
 #pragma once
-#include "k_iir.cuh"
+#include "biquad.cuh"
 
 namespace sigops {
 

@@ -20,6 +20,7 @@
 // lanes may belong to different channels and the grid can be sized to whole waves.
 #pragma once
 #include "k_iir.cuh"
+#include "ptx.cuh"
 
 namespace sigops {
 
@@ -30,37 +31,8 @@ static_assert(kStageCols % 16 == 0, "stage = whole 16-frame register blocks");
 constexpr int kStagePitch = kStageCols + 2;    // doubles: rows keep 16-B alignment; (cols+2)*2 = 4 mod 32 words makes
                                                // lane=row 128-bit accesses bank-conflict free
 constexpr int kStageBytes = kStageCols * 8;
-
-__device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(uint64_t* bar, int count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, unsigned bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, unsigned parity) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "LAB_WAIT:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@p bra LAB_DONE;\n"
-        "bra LAB_WAIT;\n"
-        "LAB_DONE:\n"
-        "}\n" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void bulk_load(void* smem_dst, const void* gsrc, unsigned bytes, uint64_t* bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(smem_dst)),
-                 "l"(gsrc), "r"(bytes), "r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void bulk_store(void* gdst, const void* smem_src, unsigned bytes) {
-    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gdst), "r"(smem_u32(smem_src)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait_read_all() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-__device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
+// per warp: [stage 0/1][lane][kStagePitch] doubles, then two mbarriers per lane
+constexpr size_t kTmaSmemBytes = (size_t)kTmaThreads * 2 * kStagePitch * sizeof(double) + (size_t)kTmaThreads * 2 * sizeof(uint64_t);
 
 // Fused elementwise programs of the TMA kernel (PROG variants): the input program sees the
 // frame just loaded as LEAF_STAGE (e.g. `load * modulator`), the epilogue sees the filter
@@ -71,7 +43,7 @@ struct TmaProg {
     const sigops_instr* ep_prog;  const double* ep_lc;  const double2* ep_rot;  int ep_len;
 };
 
-// 16 frames (one third of a stage) through the cascade; see cascade_tile in k_iir.cuh.
+// 16 frames (one third of a stage) through the cascade (cascade_frames, out as in cascade_tile of k_iir.cuh).
 // Returns sum(out^2) of the 16 outputs.  n0 = signal frame of p[0], c = channel, keep = the
 // outputs will be stored (PROG only).
 template <int M, bool ZERO_IN, bool UNITB, bool PROG>
@@ -91,18 +63,9 @@ __device__ __forceinline__ double cascade16(Cascade<M>& f, double* p, double gai
         for (int k = 0; k < 16; ++k) xr[k] = t[k];
     }
     double pipe[M], out[16];
-#pragma unroll
-    for (int t = 0; t < 16 + M - 1; ++t) {
-#pragma unroll
-        for (int j = M - 1; j >= 0; --j) {
-            const int k = t - j;
-            if (k >= 0 && k < 16) {
-                const double in = (j == 0) ? (ZERO_IN ? 0.0 : xr[k]) : pipe[j - 1];
-                pipe[j] = biquad_step<M, UNITB>(f, j, in);
-                if (j == M - 1) out[k] = ZERO_IN ? fma(pipe[j], gain, xr[k]) * sc : (pipe[j] * gain) * sc;
-            }
-        }
-    }
+    cascade_frames<M, 16, ZERO_IN, UNITB>(f, xr, pipe, [&](int k, double y) {
+        out[k] = ZERO_IN ? fma(y, gain, xr[k]) * sc : (y * gain) * sc;
+    });
     if (PROG && T.ep_len > 0 && keep) {      // warm-up outputs are discarded: no epilogue
         double t[16];
         Env env{nullptr, nullptr, 0};
@@ -182,22 +145,13 @@ k_iir_tma(const __grid_constant__ IirTmaParams Q) {
 
     mbar_init(&bars[0], 1);
     mbar_init(&bars[1], 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
     fence_async_smem();
     __syncwarp();
 
     Cascade<M> f;
-    f.init(P);
-    if (MODE == IIR_FIX && active && k >= 1) {
-        const int64_t nslots = Q.total_chunks;
-        const double* sin_ = P.carry_is_shift ? P.state_zs : P.state_in;
-        const int64_t src = P.carry_is_shift ? g - 1 : g;
-#pragma unroll
-        for (int j = 0; j < M; ++j) {
-            f.s1[j] = sin_[(2 * j) * nslots + src];
-            f.s2[j] = sin_[(2 * j + 1) * nslots + src];
-        }
-    }
+    f.init(P.coef);
+    if (MODE == IIR_FIX && active && k >= 1) load_carried_state(f, P, Q.total_chunks, g);
     const double sc_final = P.epi_scale[0] * P.epi_scale[1];
     const int64_t raw_frames = (MODE == IIR_MAIN && k >= 1) ? P.Wc : 0;   // MAIN leaves these un-scaled for FIX
     const int64_t skip_frames = pre;                                       // WARM: nothing is stored before this
@@ -268,14 +222,7 @@ k_iir_tma(const __grid_constant__ IirTmaParams Q) {
     }
     bulk_wait_all();
 
-    if (MODE == IIR_MAIN && active && P.state_zs) {
-        const int64_t nslots = Q.total_chunks;
-#pragma unroll
-        for (int j = 0; j < M; ++j) {
-            P.state_zs[(2 * j) * nslots + g] = f.s1[j];
-            P.state_zs[(2 * j + 1) * nslots + g] = f.s2[j];
-        }
-    }
+    if (MODE == IIR_MAIN && active && P.state_zs) store_final_state(f, P.state_zs, Q.total_chunks, g);
     if (P.sumsq_slot >= 0) {
         // lanes of a warp may belong to different instances: one atomic per lane that has data
         if (active && work > 0) atomicAdd(P.scalars + (size_t)inst * P.nscalars + P.sumsq_slot, ss);

@@ -32,19 +32,16 @@
 // wave at base + row*stride (true for staged host batches and for one batch tensor), frame
 // counts that are multiples of 16, WARM mode.
 #pragma once
-#include <cuda.h>
-
-#include "k_iir_tma.cuh"
+#include "biquad.cuh"
+#include "interp.cuh"
+#include "ptx.cuh"
 
 namespace sigops {
 
 constexpr int kTmSub = 16;                       // Float64 frames per 128-byte box row (the widest swizzled row)
-#ifndef TMSUBS
-#define TMSUBS 5                                 // (tuning builds override the shape with -DTMSUBS/-DTMW/-DTMS)
-#endif
 // 80-frame stages: 640 contiguous bytes per row and copy.  An odd number of blocks per row also keeps
 // the swizzle key (blocks*row + block) mod 8 different for 8 consecutive rows (4 blocks: 4-way conflicts).
-constexpr int kTmSubsPerStage = TMSUBS;                  // Float64 shape
+constexpr int kTmSubsPerStage = 5;                       // Float64 shape
 constexpr int kTmStageCols = kTmSub * kTmSubsPerStage;   // Float64 frames per stage
 constexpr int kTmSubBytes = 32 * 128;                    // one box row block: 32 rows x 128 bytes
 // Float32 shape: the bytes per sample halve while the FP64 work per sample stays, so the kernel is
@@ -78,18 +75,6 @@ struct IirTmapParams {
     int n_in_ops, n_ep_ops;
     sigops_instr ops[2 * kTmMaxLeafOps];
 };
-
-__device__ __forceinline__ void tmap_load_3d(void* smem_dst, const CUtensorMap* tm, int c0, int c1, int c2, uint64_t* bar) {
-    asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];" ::"r"(
-                     smem_u32(smem_dst)),
-                 "l"(tm), "r"(c0), "r"(c1), "r"(c2), "r"(smem_u32(bar))
-                 : "memory");
-}
-__device__ __forceinline__ void tmap_store_3d(const CUtensorMap* tm, int c0, int c1, int c2, const void* smem_src) {
-    asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%1, %2, %3}], [%4];" ::"l"(tm), "r"(c0), "r"(c1), "r"(c2),
-                 "r"(smem_u32(smem_src))
-                 : "memory");
-}
 
 // 16 frames of the lane's row through the cascade, in place in a swizzled box.  `row` points at the
 // lane's 128-byte box row, `key` = address bits 7-9 of that row: 16-byte chunk j lives at chunk
@@ -151,18 +136,7 @@ __device__ __forceinline__ double cascade16_swz(Cascade<M>& f, unsigned char* ro
             if (!((skip >> j) & 1u)) apply_leaf16<LV == 2>(P->ops[j], xr, lv + j * lvpitch);
     }
     double pipe[M], out[16];
-#pragma unroll
-    for (int t = 0; t < 16 + M - 1; ++t) {
-#pragma unroll
-        for (int j = M - 1; j >= 0; --j) {
-            const int k = t - j;
-            if (k >= 0 && k < 16) {
-                const double in = (j == 0) ? xr[k] : pipe[j - 1];
-                pipe[j] = biquad_step<M, UNITB>(f, j, in);
-                if (j == M - 1) out[k] = pipe[j] * gain;
-            }
-        }
-    }
+    cascade_frames<M, 16, false, UNITB>(f, xr, pipe, [&](int k, double y) { out[k] = y * gain; });
     // y = ((cascade * gain) * sc) * sc2, the epilogue's constants in order; a factor of exactly 1 is skipped (identity)
     if (sc != 1.0) {
 #pragma unroll
@@ -251,21 +225,13 @@ k_iir_tmap(const __grid_constant__ IirTmapParams P, const __grid_constant__ CUte
 
     if (lane == 0) {
         for (int b = 0; b < NS; ++b) mbar_init(&bars[warp][b], 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        fence_mbarrier_init();
     }
     fence_async_smem();
     __syncwarp();
 
     Cascade<M> f;
-    {
-        // same coefficient set-up as Cascade::init, from this kernel's parameter block
-#pragma unroll
-        for (int j = 0; j < M; ++j) {
-            f.b0[j] = P.coef[j][0]; f.b1[j] = P.coef[j][1]; f.b2[j] = P.coef[j][2];
-            f.a1[j] = P.coef[j][3]; f.a2[j] = P.coef[j][4];
-            f.s1[j] = 0.0; f.s2[j] = 0.0;
-        }
-    }
+    f.init(P.coef);
 
     // One tensor instruction per stage: box = (128 bytes, 5 blocks, 32 rows) of the
     // [row][frame/SUB][SUB] view, i.e. 640 contiguous bytes per row.

@@ -6,33 +6,19 @@ namespace sigops {
 namespace {
 template <int MODE>
 void launch_iir(int M, dim3 grid, size_t smem, cudaStream_t st, const IirParams& P) {
-#define SIGOPS_IIR_CASE(m)                                                                                 \
-    case m:                                                                                                \
-        if (smem > 0) ensure_dyn_smem(k_iir<m, MODE>, smem); \
-        k_iir<m, MODE><<<grid, kIirThreads, smem, st>>>(P);                                                \
-        break;
-    switch (M) {
-        SIGOPS_IIR_CASE(1) SIGOPS_IIR_CASE(2) SIGOPS_IIR_CASE(3) SIGOPS_IIR_CASE(4)
-        SIGOPS_IIR_CASE(5) SIGOPS_IIR_CASE(6) SIGOPS_IIR_CASE(7) SIGOPS_IIR_CASE(8)
-        default: fail(SIGOPS_ERR_UNSUPPORTED, "IIR cascade of %d sections", M);
-    }
-#undef SIGOPS_IIR_CASE
+    with_sections(M, [&](auto m) {
+        if (smem > 0) ensure_dyn_smem(k_iir<m, MODE>, smem);
+        k_iir<m, MODE><<<grid, kIirThreads, smem, st>>>(P);
+    });
     CUDA_OK(cudaGetLastError());
 }
 
 template <int MODE>
 void launch_iir_fast(int M, bool unitb, dim3 grid, cudaStream_t st, const IirParams& P) {
-#define SIGOPS_IIR_CASE(m)                                                  \
-    case m:                                                                 \
-        if (unitb) k_iir_fast<m, MODE, true><<<grid, kIirThreads, 0, st>>>(P);  \
-        else k_iir_fast<m, MODE, false><<<grid, kIirThreads, 0, st>>>(P);       \
-        break;
-    switch (M) {
-        SIGOPS_IIR_CASE(1) SIGOPS_IIR_CASE(2) SIGOPS_IIR_CASE(3) SIGOPS_IIR_CASE(4)
-        SIGOPS_IIR_CASE(5) SIGOPS_IIR_CASE(6) SIGOPS_IIR_CASE(7) SIGOPS_IIR_CASE(8)
-        default: fail(SIGOPS_ERR_UNSUPPORTED, "IIR cascade of %d sections", M);
-    }
-#undef SIGOPS_IIR_CASE
+    with_sections(M, [&](auto m) {
+        if (unitb) k_iir_fast<m, MODE, true><<<grid, kIirThreads, 0, st>>>(P);
+        else k_iir_fast<m, MODE, false><<<grid, kIirThreads, 0, st>>>(P);
+    });
     CUDA_OK(cudaGetLastError());
 }
 

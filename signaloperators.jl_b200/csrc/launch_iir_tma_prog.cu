@@ -9,24 +9,16 @@
 #error "compile with -DSIGOPS_PROG_GROUP=0..3"
 #endif
 
-#define SIGOPS_CAT2(a, b) a##b
-#define SIGOPS_CAT(a, b) SIGOPS_CAT2(a, b)
-
 namespace sigops {
-namespace {
-constexpr size_t kTmaSmemBytes = (size_t)kTmaThreads * 2 * kStagePitch * sizeof(double) + (size_t)kTmaThreads * 2 * sizeof(uint64_t);
 
 template <int M>
-void launch_one(dim3 grid, cudaStream_t st, const IirTmaParams& Q) {
+void launch_iir_tma_prog(dim3 grid, cudaStream_t st, const IirTmaParams& Q) {
     ensure_dyn_smem(k_iir_tma<M, IIR_WARM, false, true>, kTmaSmemBytes);
     k_iir_tma<M, IIR_WARM, false, true><<<grid, kTmaThreads, kTmaSmemBytes, st>>>(Q);
     CUDA_OK(cudaGetLastError());
 }
-}  // namespace
 
-void SIGOPS_CAT(launch_iir_tma_prog_g, SIGOPS_PROG_GROUP)(int M, dim3 grid, cudaStream_t st, const IirTmaParams& Q) {
-    if (M == 2 * SIGOPS_PROG_GROUP + 1) launch_one<2 * SIGOPS_PROG_GROUP + 1>(grid, st, Q);
-    else launch_one<2 * SIGOPS_PROG_GROUP + 2>(grid, st, Q);
-}
+template void launch_iir_tma_prog<2 * SIGOPS_PROG_GROUP + 1>(dim3, cudaStream_t, const IirTmaParams&);
+template void launch_iir_tma_prog<2 * SIGOPS_PROG_GROUP + 2>(dim3, cudaStream_t, const IirTmaParams&);
 
 }  // namespace sigops

@@ -85,17 +85,7 @@ void launch_iir_tmap(bool f32, int M, bool unitb, dim3 grid, cudaStream_t st, co
                      const void* map_out) {
     const CUtensorMap& a = *(const CUtensorMap*)map_in;
     const CUtensorMap& b = *(const CUtensorMap*)map_out;
-    switch (M) {
-        case 1: launch_m<1>(f32, unitb, grid, st, P, a, b); break;
-        case 2: launch_m<2>(f32, unitb, grid, st, P, a, b); break;
-        case 3: launch_m<3>(f32, unitb, grid, st, P, a, b); break;
-        case 4: launch_m<4>(f32, unitb, grid, st, P, a, b); break;
-        case 5: launch_m<5>(f32, unitb, grid, st, P, a, b); break;
-        case 6: launch_m<6>(f32, unitb, grid, st, P, a, b); break;
-        case 7: launch_m<7>(f32, unitb, grid, st, P, a, b); break;
-        case 8: launch_m<8>(f32, unitb, grid, st, P, a, b); break;
-        default: fail(SIGOPS_ERR_UNSUPPORTED, "IIR cascade of %d sections", M);
-    }
+    with_sections(M, [&](auto m) { launch_m<m>(f32, unitb, grid, st, P, a, b); });
     CUDA_OK(cudaGetLastError());
 }
 
