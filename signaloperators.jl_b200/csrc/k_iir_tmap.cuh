@@ -51,6 +51,7 @@ constexpr int kTmSubsPerStageF32 = 3, kTmWarpsF32 = 8;
 // dependency chains are long, so twice the warps on 48-frame stages, like the Float32 shape
 constexpr int kTmSubsPerStageLv = 3, kTmWarpsLv = 8;
 constexpr int kTmMaxLeafOps = 4;                        // fused row-invariant operations before / after the cascade
+constexpr int kTmMaxSubInstrs = 24;                     // instructions of all the sub-programs of a stage's operations
 constexpr size_t tm_smem_bytes(int nw, int ns, int subs, bool lv = false, int sub = kTmSub) {   // + 1024-byte alignment slack
     return (size_t)nw * ns * subs * kTmSubBytes + 1024 + (lv ? (size_t)nw * 2 * kTmMaxLeafOps * subs * sub * sizeof(double) : 0);
 }
@@ -74,6 +75,12 @@ struct IirTmapParams {
     // envelope follower's lowpass, tanh after a filter).
     int n_in_ops, n_ep_ops;
     sigops_instr ops[2 * kTmMaxLeafOps];
+    // (LV = 2) An operation j with sub_len[j] > 0 is `PUSH <sub-program> POPop` of the stage's program: it combines the
+    // sample with the sub-program's value at the frame, sub[sub_start[j] .. + sub_len[j]), whose leaves are again
+    // constants, generators or ramps (e.g. a traced AM envelope 0.5 sin(ϕ) + 0.25 sin(2ϕ) + 0.25).  ops[j] then holds
+    // the operator (ADD..DIV) and no leaf.
+    int sub_start[2 * kTmMaxLeafOps], sub_len[2 * kTmMaxLeafOps];
+    sigops_instr sub[kTmMaxSubInstrs];
 };
 
 // 16 frames of the lane's row through the cascade, in place in a swizzled box.  `row` points at the
@@ -176,6 +183,38 @@ __device__ __forceinline__ double cascade16_swz(Cascade<M>& f, unsigned char* ro
 // value of a row-invariant leaf at frame n (the interpreter's exact per-frame formulas)
 __device__ __forceinline__ double rowinv_leaf(const sigops_instr* I, int64_t n) {
     return I->leaf == SIGOPS_LEAF_CONST ? I->d0 : leaf_value_slow(I, nullptr, n, 0);
+}
+
+// value of a row-invariant sub-program at frame n: a scalar interpreter with eval_program's semantics over constant,
+// generator and ramp leaves.  Out of line for the reason leaf_value_slow is (one copy of the libm code per kernel).
+static __device__ __noinline__ double rowinv_sub_value(const sigops_instr* prog, int len, int64_t n) {
+    double acc = 0.0, stack[SIGOPS_MAX_STACK];
+    int sp = 0;
+    for (int pc = 0; pc < len; ++pc) {
+        const sigops_instr* I = prog + pc;
+        const int op = I->op;
+        if (op <= SIGOPS_OP_DIV || op == SIGOPS_OP_FN2) {
+            const double v = rowinv_leaf(I, n);
+            if (op == SIGOPS_OP_LOAD) acc = v;
+            else if (op == SIGOPS_OP_FN2) efn_vec<1>(I->fn, &acc, [&](int) { return v; }, 0.0);
+            else acc = binop(op, acc, v);
+        } else if (op == SIGOPS_OP_PUSH) {
+            stack[sp++] = acc;
+        } else if (op <= SIGOPS_OP_POPDIV) {
+            acc = binop(op, stack[--sp], acc);
+        } else if (op == SIGOPS_OP_NEG) {
+            acc = -acc;
+        } else if (op == SIGOPS_OP_CAST_F32) {
+            acc = (double)(float)acc;
+        } else if (op == SIGOPS_OP_FN1) {
+            efn_vec<1>(I->fn, &acc, [&](int) { return I->d0; }, I->d1);
+        } else if (op == SIGOPS_OP_POPFN2) {
+            double l = stack[--sp];
+            efn_vec<1>(I->fn, &l, [&](int) { return acc; }, 0.0);
+            acc = l;
+        }
+    }
+    return acc;
 }
 
 template <int M, bool UNITB, int NW, int NS, int SUBS, class T, int LV = 0>
@@ -282,7 +321,9 @@ k_iir_tmap(const __grid_constant__ IirTmapParams P, const __grid_constant__ CUte
                 const int jj = v / SC, fr = v - jj * SC;
                 const int j = jj < P.n_in_ops ? jj : kTmMaxLeafOps + jj - P.n_in_ops;
                 if (((skip >> j) & 1u) || (LV == 2 && P.ops[j].op >= SIGOPS_OP_FN1)) continue;   // (functions: no vector)
-                lvw[j * SC + fr] = ((ones >> j) & 1u) ? 1.0 : rowinv_leaf(&P.ops[j], n0 + fr);
+                // (a sub-program's value is never skipped as "exactly 1": its operation has no ramp leaf)
+                if (LV == 2 && P.sub_len[j] > 0) lvw[j * SC + fr] = rowinv_sub_value(P.sub + P.sub_start[j], P.sub_len[j], n0 + fr);
+                else lvw[j * SC + fr] = ((ones >> j) & 1u) ? 1.0 : rowinv_leaf(&P.ops[j], n0 + fr);
             }
             __syncthreads();
         }

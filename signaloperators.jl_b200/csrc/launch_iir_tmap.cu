@@ -37,8 +37,9 @@ void launch_cfg(bool unitb, dim3 grid, cudaStream_t st, const IirTmapParams& P, 
 template <int M>
 void launch_m(bool f32, bool unitb, dim3 grid, cudaStream_t st, const IirTmapParams& P, const CUtensorMap& a, const CUtensorMap& b) {
     const bool lv = P.n_in_ops + P.n_ep_ops > 0;
-    bool fn = false;                   // a closure function among the fused operations: the variant that applies them
-    for (int j = 0; j < 2 * kTmMaxLeafOps; ++j) fn = fn || P.ops[j].op == SIGOPS_OP_FN1 || P.ops[j].op == SIGOPS_OP_FN2;
+    bool fn = false;   // a closure function or a sub-program among the fused operations: the variant that applies them
+    for (int j = 0; j < 2 * kTmMaxLeafOps; ++j)
+        fn = fn || P.ops[j].op == SIGOPS_OP_FN1 || P.ops[j].op == SIGOPS_OP_FN2 || P.sub_len[j] > 0;
     if (f32) launch_cfg<M, kTmWarpsF32, kTmStages, kTmSubsPerStageF32, float, 0>(unitb, grid, st, P, a, b);
     else if (lv && fn) launch_cfg<M, kTmWarpsLv, kTmStages, kTmSubsPerStageLv, double, 2>(unitb, grid, st, P, a, b);
     else if (lv) launch_cfg<M, kTmWarpsLv, kTmStages, kTmSubsPerStageLv, double, 1>(unitb, grid, st, P, a, b);

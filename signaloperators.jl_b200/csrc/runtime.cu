@@ -190,9 +190,13 @@ struct IirDerived {
     bool fast = false;             // k_iir_fast applies (f64 in/out, constant-gain epilogue)
     bool fast32 = false;           // same shape on Float32 buffers: k_iir_tmap<float> applies
     bool tma_prog = false;         // k_iir_tma<PROG>: one plain f64 buffer + buffer-free programs
+    bool prog_stack = false;       // ... whose programs use the stack: only the row-invariant k_iir_tmap runs them
     int prog_in_start = 0, prog_in_len = 0;   // input program with the buffer leaf turned into LEAF_STAGE
     bool rowinv = false;           // tma_prog whose other leaves depend on the frame only: k_iir_tmap with leaf vectors
     std::vector<sigops_instr> rv_in, rv_ep;   // those operations, in order (<= kTmMaxLeafOps each)
+    std::vector<int> rv_in_sub, rv_ep_sub;    // per operation: start of its sub-program in rv_sub, or -1
+    std::vector<int> rv_sub_len;              // per sub-program (in the order of rv_in_sub then rv_ep_sub)
+    std::vector<sigops_instr> rv_sub;         // the sub-programs (<= kTmMaxSubInstrs in all)
     bool unitb = false;            // every section has b0 == 1 and b2 == 1 exactly
     int n_scale = 0;
     double scale[2] = {1.0, 1.0};
@@ -446,11 +450,11 @@ void derive_iir(sigops_plan& p, StageRT& s, int idx) {
     // in either program touches a buffer or an RMS slot
     if (!s.iir.fast && p.bufs[st.out_buf].dtype == SIGOPS_F64) {
         int nbuf_leaves = 0, bufpc = -1;
-        bool ok = true;
+        bool ok = true, stack = false;
         auto scan = [&](int start, int len, bool is_input) {
             for (int i = 0; i < len; ++i) {
                 const sigops_instr& I = p.instrs[start + i];
-                if (!op_has_leaf(I.op)) { if (I.op == SIGOPS_OP_PUSH) ok = false; continue; }   // no stack in this path
+                if (!op_has_leaf(I.op)) { if (I.op == SIGOPS_OP_PUSH) stack = true; continue; }   // (k_iir_tma: no stack)
                 if (I.leaf == SIGOPS_LEAF_RMS || I.leaf == SIGOPS_LEAF_CHANSUM || I.leaf == SIGOPS_LEAF_RANDN) ok = false;
                 if (I.leaf == SIGOPS_LEAF_BUF) {
                     if (!is_input) { ok = false; continue; }
@@ -478,18 +482,52 @@ void derive_iir(sigops_plan& p, StageRT& s, int idx) {
             if (s.iir.prog_in_len == 1) s.iir.prog_in_len = 0;      // bare load: nothing to evaluate
             // Row-invariant form: `LOAD buffer, (op leaf)*` before and `LOAD stage, (op leaf)*` after the cascade,
             // every leaf a constant, generator or ramp (the same value for all rows at a frame); closure functions
-            // f(acc) and g(acc, constant) take an operation slot and no leaf vector
-            auto rowinv_ops = [&](int start, int len, std::vector<sigops_instr>& ops) {
+            // f(acc) and g(acc, constant) take an operation slot and no leaf vector.  `PUSH <sub-program> POPop` takes
+            // one slot too when the sub-program reads only such leaves (a traced generator closure: its value at the
+            // frame is the slot's vector); at most kTmMaxSubInstrs sub-program instructions per stage.
+            auto rowinv_leaf_ok = [](const sigops_instr& I) {
+                return I.leaf == SIGOPS_LEAF_CONST || I.leaf == SIGOPS_LEAF_GEN || I.leaf == SIGOPS_LEAF_RAMP_ON ||
+                       I.leaf == SIGOPS_LEAF_RAMP_OFF;
+            };
+            auto sub_instr_ok = [&](const sigops_instr& I) {
+                if (I.op >= SIGOPS_OP_LOAD && I.op <= SIGOPS_OP_DIV) return rowinv_leaf_ok(I);
+                if (I.op == SIGOPS_OP_FN2) return I.leaf == SIGOPS_LEAF_CONST;
+                return I.op == SIGOPS_OP_PUSH || (I.op >= SIGOPS_OP_POPADD && I.op <= SIGOPS_OP_POPDIV) ||
+                       I.op == SIGOPS_OP_NEG || I.op == SIGOPS_OP_CAST_F32 || I.op == SIGOPS_OP_FN1 || I.op == SIGOPS_OP_POPFN2;
+            };
+            auto rowinv_ops = [&](int start, int len, std::vector<sigops_instr>& ops, std::vector<int>& subs) {
                 for (int i = 1; i < len; ++i) {
                     const sigops_instr& I = p.instrs[start + i];
+                    if (I.op == SIGOPS_OP_PUSH) {
+                        int e = i + 1, depth = 1;                          // e: the matching pop
+                        for (; e < len; ++e) {
+                            const int op = p.instrs[start + e].op;
+                            depth += op == SIGOPS_OP_PUSH ? 1 : ((op >= SIGOPS_OP_POPADD && op <= SIGOPS_OP_POPDIV) || op == SIGOPS_OP_POPFN2 ? -1 : 0);
+                            if (depth == 0) break;
+                        }
+                        const int n = e - i - 1;
+                        if (e >= len || p.instrs[start + e].op > SIGOPS_OP_POPDIV || n < 1 ||
+                            p.instrs[start + i + 1].op != SIGOPS_OP_LOAD || (int)s.iir.rv_sub.size() + n > kTmMaxSubInstrs)
+                            return false;
+                        subs.push_back((int)s.iir.rv_sub.size());
+                        s.iir.rv_sub_len.push_back(n);
+                        for (int q = i + 1; q < e; ++q) {
+                            if (!sub_instr_ok(p.instrs[start + q])) return false;
+                            s.iir.rv_sub.push_back(p.instrs[start + q]);
+                        }
+                        sigops_instr J{};
+                        J.op = (uint8_t)(p.instrs[start + e].op - SIGOPS_OP_POPADD + SIGOPS_OP_ADD);
+                        J.leaf = SIGOPS_LEAF_NONE;
+                        ops.push_back(J);
+                        i = e;
+                        continue;
+                    }
+                    subs.push_back(-1);
                     if (I.op == SIGOPS_OP_FN1 || (I.op == SIGOPS_OP_FN2 && I.leaf == SIGOPS_LEAF_CONST)) {
                         ops.push_back(I);
                         continue;
                     }
-                    if (I.op < SIGOPS_OP_ADD || I.op > SIGOPS_OP_DIV) return false;
-                    if (I.leaf != SIGOPS_LEAF_CONST && I.leaf != SIGOPS_LEAF_GEN && I.leaf != SIGOPS_LEAF_RAMP_ON &&
-                        I.leaf != SIGOPS_LEAF_RAMP_OFF)
-                        return false;
+                    if (I.op < SIGOPS_OP_ADD || I.op > SIGOPS_OP_DIV || !rowinv_leaf_ok(I)) return false;
                     ops.push_back(I);
                 }
                 return (int)ops.size() <= kTmMaxLeafOps;
@@ -497,8 +535,11 @@ void derive_iir(sigops_plan& p, StageRT& s, int idx) {
             const bool in_first = bufpc == st.in_prog_start && p.instrs[bufpc].op == SIGOPS_OP_LOAD;
             const bool ep_first = st.epi_prog_len == 0 || (p.instrs[st.epi_prog_start].op == SIGOPS_OP_LOAD &&
                                                            p.instrs[st.epi_prog_start].leaf == SIGOPS_LEAF_STAGE);
-            s.iir.rowinv = in_first && ep_first && rowinv_ops(st.in_prog_start, st.in_prog_len, s.iir.rv_in) &&
-                           rowinv_ops(st.epi_prog_start, st.epi_prog_len, s.iir.rv_ep);
+            s.iir.rowinv = in_first && ep_first && rowinv_ops(st.in_prog_start, st.in_prog_len, s.iir.rv_in, s.iir.rv_in_sub) &&
+                           rowinv_ops(st.epi_prog_start, st.epi_prog_len, s.iir.rv_ep, s.iir.rv_ep_sub);
+            // programs with a stack: the row-invariant kernel or none of the TMA ones (k_iir runs them)
+            s.iir.prog_stack = stack;
+            if (stack && !s.iir.rowinv) s.iir.tma_prog = false;
         }
     }
 }
@@ -1161,6 +1202,16 @@ bool plan_iir_tmap(const Wave& w, bool tma) {
         T.n_ep_ops = (int)s.iir.rv_ep.size();
         for (int j = 0; j < T.n_in_ops; ++j) T.ops[j] = s.iir.rv_in[j];
         for (int j = 0; j < T.n_ep_ops; ++j) T.ops[kTmMaxLeafOps + j] = s.iir.rv_ep[j];
+        int q = 0;                        // sub-programs, in the order rowinv_ops recorded them
+        for (int j = 0; j < 2 * kTmMaxLeafOps; ++j) {
+            const int k = j < kTmMaxLeafOps ? j : j - kTmMaxLeafOps;
+            const std::vector<int>& subs = j < kTmMaxLeafOps ? s.iir.rv_in_sub : s.iir.rv_ep_sub;
+            if (k < (int)subs.size() && subs[k] >= 0) {
+                T.sub_start[j] = subs[k];
+                T.sub_len[j] = s.iir.rv_sub_len[q++];
+            }
+        }
+        for (size_t i = 0; i < s.iir.rv_sub.size(); ++i) T.sub[i] = s.iir.rv_sub[i];
     }
     const double* tc = w.p.blob.data() + w.p.tables[g.coef_table].offset;
     for (int j = 0; j < s.iir.M; ++j)
@@ -1188,6 +1239,7 @@ void plan_iir_stage(const Wave& w) {
     bool tma = (s.iir.fast || s.iir.tma_prog) && rows_aligned(w.refs, w.ninst, w.nbuf, s.iir.plain_buf, false) &&
                rows_aligned(w.refs, w.ninst, w.nbuf, g.out_buf, false);
     if (plan_iir_tmap(w, tma)) return;
+    if (s.iir.prog_stack) tma = false;   // (k_iir_tma interprets no stack)
     // (the program-carrying TMA kernel has no MAIN/FIX form: keep it to chunkings it can run)
     IirLaunch c = tma ? choose_iir_chunking_flat(s, rows, w.sm_count, !s.iir.tma_prog) : choose_iir_chunking(s, rows, w.sm_count);
     // the program-carrying TMA kernel only exists in the single-launch WARM form (for a filter that does not decay

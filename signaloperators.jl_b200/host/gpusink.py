@@ -199,14 +199,20 @@ def sink_into(result, x, to):
 
 
 def _build_prefix(lw, x, n, dtype):
-    from .lowering import STAGE_MAP, BufDesc, Stage, dtype_code
+    from .lowering import STAGE_MAP, BufDesc, LoweringError, Stage, dtype_code
     C = x.nchannels
-    lw.plan.outputs.append(BufDesc(n, C, dtype_code(dtype)))
-    lw.plan.framerate = x.framerate
-    pieces = lw.lower(x, 0, 0, n, 1, 0, 0, C) if n > 0 else []
-    lw.plan.stages.append(Stage(STAGE_MAP, ("out", 0), pieces=pieces, nchannels=C, n_out=n))
-    lw._fuse_epilogues()
-    lw._check_limits()
+    try:
+        lw.plan.outputs.append(BufDesc(n, C, dtype_code(dtype)))
+        lw.plan.framerate = x.framerate
+        pieces = lw.lower(x, 0, 0, n, 1, 0, 0, C) if n > 0 else []
+        lw.plan.stages.append(Stage(STAGE_MAP, ("out", 0), pieces=pieces, nchannels=C, n_out=n))
+        lw._fuse_epilogues()
+        lw._check_limits()
+    except LoweringError:
+        nxt = lw.fallback()          # traced generators over a device limit: lower them the next way
+        if nxt is None:
+            raise
+        return _build_prefix(nxt, x, n, dtype)
     return lw.plan
 
 
@@ -216,8 +222,14 @@ def sink_batch(xs, to):
     constants) and differ only in the arrays they read."""
     if not xs:
         return []
-    plans = [Lowerer(instance_index=k).build(x) for k, x in enumerate(xs)]
+    lws = [Lowerer(instance_index=k) for k in range(len(xs))]
+    plans = [lw.build(x) for lw, x in zip(lws, xs)]
     ref = plans[0].tobytes()
+    if any(lw.traced_generators for lw in lws) and any(p.tobytes() != ref for p in plans[1:]):
+        # closure generators whose traced programs differ between elements (other ω, ϕ or constants): evaluated on
+        # the host, their frames are input buffers and the plans agree again
+        plans = [Lowerer(instance_index=k, generators="host").build(x) for k, x in enumerate(xs)]
+        ref = plans[0].tobytes()
     for k, p in enumerate(plans[1:], 1):
         if p.tobytes() != ref:
             raise G.SignalError(f"batch element {k} does not lower to the same plan as element 0")

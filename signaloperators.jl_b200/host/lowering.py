@@ -22,9 +22,9 @@ from dataclasses import dataclass, field, replace
 import numpy as np
 
 from . import dspjl, graph as G
-from .functors import functor_code
+from .functors import functor_code, generator_shape
 from .philox import PhiloxRNG
-from .trace import TraceError, trace
+from .trace import TraceError, same, trace, trace_generator
 from .wav import WavSignal
 
 # ---- constants mirrored from include/signalops.h -------------------------------
@@ -304,9 +304,17 @@ def _intersect(a: Piece, b: Piece):
     return None
 
 
+# How the closures of `Signal(fn, ...)` that trace are lowered: in line as device programs, each computed once into a
+# temp by a MAP stage of its own, or evaluated on the host as before tracing.  Lowering starts with the first and takes
+# the next one when the plan exceeds a device limit (a long traced expression inside a long program).
+GENERATOR_MODES = ("device", "temp", "host")
+
+
 class Lowerer:
-    def __init__(self, instance_index=0):
+    def __init__(self, instance_index=0, generators="device"):
         self.instance_index = instance_index     # position of this graph in a batch call (device noise streams)
+        self.generators = generators             # GENERATOR_MODES
+        self.traced_generators = False           # a closure generator became a device program
         self.plan = Plan()
         self._input_ids = {}      # id(ndarray) -> input index
         self._barrier_memo = {}   # id(node) -> (buf tag, frames materialised, stage)
@@ -368,8 +376,25 @@ class Lowerer:
         self.plan.n_scalars += 1
         return self.plan.n_scalars - 1
 
+    def fallback(self):
+        """A fresh Lowerer for the next generator mode, or None when this one traced no generator (nothing to change)."""
+        if not self.traced_generators or self.generators == GENERATOR_MODES[-1]:
+            return None
+        return Lowerer(self.instance_index, GENERATOR_MODES[GENERATOR_MODES.index(self.generators) + 1])
+
     # ---- entry point ------------------------------------------------------------
     def build(self, x, nframes=None, nchannels=None, out_dtype=None):
+        try:
+            return self._build(x, nframes, nchannels, out_dtype)
+        except LoweringError:
+            nxt = self.fallback()
+            if nxt is None:
+                raise
+        self.plan = nxt.build(x, nframes, nchannels, out_dtype)
+        self.traced_generators = nxt.traced_generators
+        return self.plan
+
+    def _build(self, x, nframes, nchannels, out_dtype):
         x = G.process_sink_params(x)
         N = x.nframes if nframes is None else int(nframes)
         if nchannels is not None:
@@ -474,15 +499,38 @@ class Lowerer:
         code = None if isinstance(x.fn, G.RandFn) else functor_code(x.fn)
         if code is not None and x.nchannels == 1:
             fn, a, b = code
-            return [Piece(lo, hi, clo, chi, [Instr(
-                OP_LOAD, LEAF_GEN, fn=fn, flags=FLAG_HAS_OMEGA if x.omega is not None else 0,
-                i0=shift + 1, d0=float(fs), d1=float(x.omega or 0.0), d2=x.phi, d3=a, d4=b)])]
+            return [Piece(lo, hi, clo, chi, [_gen_leaf(x, shift, fn, a, b)])]
+        progs = None if isinstance(x.fn, G.RandFn) or self.generators == "host" else _generator_programs(x, shift)
+        if progs is not None:
+            self.traced_generators = True
+            if self.generators == "temp" and any(not _isleaf(pr) for pr in progs):
+                return self._materialize_generator(x, shift, lo, hi, cm, co, clo, chi)
+            if cm == 0 or len(progs) == 1:
+                return [Piece(lo, hi, clo, chi, progs[co if cm == 0 else 0])]
+            return [Piece(lo, hi, c, c + 1, progs[c * cm + co]) for c in range(clo, chi)]
         # not expressible on the device: evaluate this leaf on the host with the
         # reference's formula and feed it as an input buffer (SURVEY.md §7.3-5/6)
         vals = host_function_frames(x, lo + shift + 1, hi + shift + 1)
         tag = self.add_input(vals)
         return [Piece(lo, hi, clo, chi, [Instr(OP_LOAD, LEAF_BUF, buf=tag, c_mul=cm, c_off=co,
                                                i0=-lo, i1=hi - lo)])]
+
+    def _materialize_generator(self, x, shift, lo, hi, cm, co, clo, chi):
+        """A traced generator computed once into a temp by a MAP stage of its own (frames [0, n) of the node), read
+        back as a buffer: the program that reads it keeps one instruction for it."""
+        n = hi + shift
+        key = ("gen", id(x))
+        memo = self._barrier_memo.get(key)
+        if not (memo and memo[1] >= n):
+            C = x.nchannels
+            tag = self.add_temp(n, C, x.sampletype)
+            progs = _generator_programs(x, 0)
+            pieces = [Piece(0, n, c, c + 1, progs[c]) for c in range(C)]
+            self.plan.stages.append(Stage(STAGE_MAP, tag, pieces=pieces, nchannels=C, n_out=n))
+            memo = (tag, n, None)
+            self._barrier_memo[key] = memo
+            self._keepalive.append(x)
+        return [Piece(lo, hi, clo, chi, [Instr(OP_LOAD, LEAF_BUF, buf=memo[0], c_mul=cm, c_off=co, i0=shift, i1=memo[1])])]
 
     def _lower_ramp(self, x, shift, lo, hi, clo, chi):
         L = x.resolvelen()
@@ -998,6 +1046,48 @@ class Lowerer:
                     raise LoweringError(f"fused expression of {len(prog)} operations exceeds {MAX_PROG}")
                 if _stack_depth(prog) > MAX_STACK:
                     raise LoweringError("expression nests deeper than the device stack")
+
+
+def _gen_leaf(x, shift, fn, a=0.0, b=0.0):
+    """The device generator leaf of SignalFunction `x` (src/functions.jl:53-60): `fn` of 2π((k/fs·ω + ϕ) % 1) with ω,
+    of k/fs + ϕ without, at 1-based frame k = n + shift + 1."""
+    return Instr(OP_LOAD, LEAF_GEN, fn=fn, flags=FLAG_HAS_OMEGA if x.omega is not None else 0,
+                 i0=shift + 1, d0=float(x.framerate), d1=float(x.omega or 0.0), d2=x.phi, d3=a, d4=b)
+
+
+def _generator_programs(x, shift):
+    """One device program per channel computing the generator closure of SignalFunction `x`, or None when the closure
+    has to run on the host.  The closure is traced (host/trace.py) on a tracer standing for the generator's argument,
+    the FN_IDENTITY leaf; an expression that is exactly one of the enumerated generators becomes that leaf
+    (functors.generator_shape), so it keeps the angle-addition fast path.  The closure is traced twice: the reference
+    calls it once per frame, so a closure whose two traces differ (it draws random numbers, or reads state it changes)
+    or that ignores its argument would be frozen into a constant, and stays on the host.  So does a closure the tracer
+    refuses (comparisons, `math` functions, ...) and one whose program does not fit a device program."""
+    try:
+        roots = trace_generator(x.fn, x.nchannels)
+        again = trace_generator(x.fn, x.nchannels)
+    except Exception:          # any error of a closure that needs a number: it still runs on the host, as before
+        return None
+    if not all(same(a, b) and _node_args(a, set()) for a, b in zip(roots, again)):
+        return None
+    T = np.dtype(x.sampletype)
+    f32 = T == np.float32
+    tail = [Instr(op=OP_CAST_I64)] if T.kind in "iub" else []
+    arg = {0: [_gen_leaf(x, shift, FN_IDENTITY)]}
+    progs = []
+    for root in roots:
+        shape = generator_shape(root) if T == np.float64 else None
+        if shape is not None:
+            progs.append([_gen_leaf(x, shift, *shape)])
+            continue
+        try:
+            prog = _traced_program(root, arg, f32) + tail
+        except _TooLong:
+            return None
+        if len(prog) > MAX_PROG or _stack_depth(prog) > MAX_STACK:
+            return None
+        progs.append(prog)
+    return progs
 
 
 def host_function_frames(x, k_lo, k_hi):

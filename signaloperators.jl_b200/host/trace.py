@@ -160,6 +160,20 @@ def _unpack(v, n_out, what):
     return tuple(_node(e, what) for e in vs)
 
 
+def same(a, b):
+    """Whether two traced expressions are the same expression (constants compared bit for bit)."""
+    return (a.kind == b.kind and a.key == b.key and repr(a.value) == repr(b.value) and len(a.args) == len(b.args)
+            and all(same(p, q) for p, q in zip(a.args, b.args)))
+
+
+def trace_generator(fn, nchannels):
+    """Call the generator closure of `Signal(fn, ...)` on one tracer value standing for its argument (the phase or the
+    time of a frame) and return one Node per channel.  Raises whatever `fn` raises on a tracer: a TraceError for what
+    a traced sample cannot stand for, or any other error of a closure that needs a number."""
+    name = getattr(fn, "__name__", repr(fn))
+    return _unpack(fn(Sym(Node("arg", key=0))), nchannels, f"Signal({name})")
+
+
 def trace(fn, nargs, channels=None):
     """Call `fn` on tracer values.  bychannel (channels is None): one Sym per argument, returns one Node.  Otherwise
     `channels[k]` channels of argument k arrive as a tuple of Sym, and a tuple of Nodes (one per output channel) is

@@ -140,6 +140,9 @@ end
 function SignalOperators.sink(xs::AbstractVector, to::GPUSink)
     xs = process_sink_params.(xs)
     plans = [lower(x; instance_index = i - 1) for (i, x) in enumerate(xs)]
+    # closure generators whose traced programs differ between elements (other ω, ϕ or constants): on the CPU sink,
+    # their frames are input buffers and the plans agree again
+    all(p -> p.bytes == plans[1].bytes, plans) || (plans = [lower(x; instance_index = i - 1, generators = :host) for (i, x) in enumerate(xs)])
     all(p -> p.bytes == plans[1].bytes, plans) || error("batch elements do not lower to the same plan")
     results = [pinned_matrix(to, p.outtype, nframes(x), nchannels(x)) for (x, p) in zip(xs, plans)]
     (isempty(xs) || nframes(xs[1]) == 0) || run!(to, plans, results)
@@ -230,8 +233,9 @@ end
 Base.showerror(io::IO, e::LoweringError) = print(io, "GPUSinks: ", e.msg)
 
 # ---- GPU-aware generator functions (host/functors.py) -------------------------------------------------------
-# `Signal(fn, ω=...)` with one of these lowers to a device generator; any other callable is evaluated on the
-# host with the reference's own formula (src/functions.jl:53-60) and fed as an input buffer.
+# `Signal(fn, ω=...)` with one of these lowers to a device generator; any other closure is traced into a device
+# program (`generator_programs` below), and what does not trace is evaluated by the reference's own CPU sink
+# (src/functions.jl:53-60) and fed as an input buffer.
 struct Sawtooth end
 (::Sawtooth)(x) = x / π - 1
 struct AffineSin; a::Float64; b::Float64; end
@@ -315,8 +319,10 @@ mutable struct Lowerer
     input_ids::Dict{UInt,Int}
     memo::Dict{Any,Any}
     instance_index::Int          # position of this graph in a batch call (device noise streams)
-    Lowerer(instance_index = 0) = new(BufDesc[], Array[], BufDesc[], BufDesc[], 0, Vector{Float64}[], Stage[], Dict{UInt,Int}(),
-                                      Dict{Any,Any}(), instance_index)
+    generators::Symbol           # closure generators that trace: :device (in line), :temp (own MAP stage), :host (CPU sink)
+    traced_generators::Bool      # a closure generator became a device program
+    Lowerer(instance_index = 0, generators = :device) = new(BufDesc[], Array[], BufDesc[], BufDesc[], 0, Vector{Float64}[], Stage[],
+                                                            Dict{UInt,Int}(), Dict{Any,Any}(), instance_index, generators, false)
 end
 
 # `Signal(randn; rng = PhiloxRNG(seed, stream))`: noise drawn ON THE DEVICE (src/functions.jl:98-114 with a
@@ -470,22 +476,115 @@ function traced_program(nd::TNode, argprog, f32::Bool)
     end
     emit(nd)
 end
+# ---- generator closures `Signal(ϕ -> …)` (lowering.py `_generator_programs`, functors.py `generator_shape`) ----------
+gen_leaf(x, fs, shift, fn, a = 0.0, b = 0.0) =
+    Instr(OP_LOAD, LEAF_GEN; fn = fn, flags = ismissing(x.ω) ? 0x00 : FLAG_HAS_OMEGA, i0 = shift + 1, d0 = Float64(fs),
+          d1 = ismissing(x.ω) ? 0.0 : Float64(x.ω), d2 = x.ϕ, d3 = a, d4 = b)
+same_tnode(a::TNode, b::TNode) = a.kind === b.kind && isequal(a.value, b.value) && length(a.args) == length(b.args) &&
+                                 all(same_tnode(p, q) for (p, q) in zip(a.args, b.args))
+isconstnode(nd, v = nothing) = nd.kind === :const && (v === nothing || nd.value == v)
+isargnode(nd) = nd.kind === :arg
+function scaled_gen(nd, f)                # `a*f(arg)` or `f(arg)*a` -> a; `f(arg)` -> 1
+    nd.kind === f && isargnode(nd.args[1]) && return 1.0
+    if nd.kind === :*
+        p, q = nd.args
+        isconstnode(p) && q.kind === f && isargnode(q.args[1]) && return p.value
+        isconstnode(q) && p.kind === f && isargnode(p.args[1]) && return q.value
+    end
+    nothing
+end
+# (code, a, b) of the device generator a traced expression is exactly, or nothing; only rewrites that keep every bit
+function generator_shape(nd::TNode)
+    isargnode(nd) && return (FN_IDENTITY, 0.0, 0.0)
+    if nd.kind === :- && isconstnode(nd.args[2], 1.0) && nd.args[1].kind === :/
+        p, q = nd.args[1].args
+        isargnode(p) && isconstnode(q, Float64(π)) && return (FN_SAW, 0.0, 0.0)
+    end
+    nd.kind === :cos && isargnode(nd.args[1]) && return (FN_COS, 0.0, 0.0)
+    nd.kind === :sin && isargnode(nd.args[1]) && return (FN_AFFINE_SIN, 1.0, 0.0)     # not FN_SIN: that is `sinpi`
+    if nd.kind === :+ || nd.kind === :-
+        p, q = nd.args
+        nd.kind === :+ && isconstnode(p) && ((p, q) = (q, p))
+        if isconstnode(q)
+            b = nd.kind === :+ ? q.value : -q.value
+            for (f, code) in ((:sin, FN_AFFINE_SIN), (:cos, FN_AFFINE_COS))
+                a = scaled_gen(p, f)
+                a === nothing || return (code, Float64(a), Float64(b))
+            end
+        end
+    end
+    nothing
+end
+function trace_generator(fn)
+    r = fn(Traced(TNode(:arg, TNode[], 0)))
+    r isa Traced ? [r.node] : [tnode(v) for v in r]
+end
+# one device program per channel, or nothing when the closure stays on the CPU sink: the tracer refuses it, its two
+# traces differ (it draws random numbers or changes state), it ignores its argument, or it does not fit a program
+function generator_programs(x, fs, shift)
+    traces = try
+        (trace_generator(x.fn), trace_generator(x.fn))
+    catch
+        return nothing
+    end
+    roots, again = traces
+    (length(roots) == length(again) == nchannels(x)) || return nothing
+    all(same_tnode(a, b) && !isempty(targs!(Set{Any}(), a)) for (a, b) in zip(roots, again)) || return nothing
+    T = sampletype(x)
+    f32 = T === Float32
+    tail = T <: Integer ? [Instr(OP_CAST_I64)] : Instr[]
+    arg = Dict{Any,Vector{Instr}}(0 => [gen_leaf(x, fs, shift, FN_IDENTITY)])
+    progs = Vector{Instr}[]
+    for root in roots
+        shape = T === Float64 ? generator_shape(root) : nothing
+        if shape !== nothing
+            push!(progs, [gen_leaf(x, fs, shift, shape...)])
+            continue
+        end
+        prog = try vcat(traced_program(root, arg, f32), tail) catch e; e isa LoweringError ? nothing : rethrow() end
+        (prog === nothing || length(prog) > MAX_PROG || stack_depth(prog) > MAX_STACK) && return nothing
+        push!(progs, prog)
+    end
+    progs
+end
+# a traced generator computed once into a temp by a MAP stage of its own, read back as a buffer
+function materialize_generator!(lw, x, fs, shift, lo, hi, cm, co, clo, chi)
+    n = hi + shift
+    key = (:gen, objectid(x))
+    memo = get(lw.memo, key, nothing)
+    if memo === nothing || memo[2] < n
+        C = nchannels(x)
+        tag = add_temp!(lw, n, C, sampletype(x))
+        progs = generator_programs(x, fs, 0)
+        push!(lw.stages, Stage(kind = STAGE_MAP, out_buf = tag, pieces = [Piece(0, n, c, c + 1, progs[c+1]) for c in 0:C-1],
+                               nchannels = C, n_out = n))
+        memo = lw.memo[key] = (tag, n)
+    end
+    [Piece(lo, hi, clo, chi, [Instr(OP_LOAD, LEAF_BUF; buf = memo[1], c_mul = cm, c_off = co, i0 = shift, i1 = memo[2])])]
+end
+
 function intersect_pieces(a::Piece, b::Piece)
     lo, hi, clo, chi = max(a.lo, b.lo), min(a.hi, b.hi), max(a.clo, b.clo), min(a.chi, b.chi)
     (lo < hi && clo < chi) ? (lo, hi, clo, chi) : nothing
 end
 
 # ---- entry point (`Lowerer.build`) -------------------------------------------------------------------------------
-function lower(x; nframes = SignalOperators.nframes(x), outtype = nothing, instance_index = 0)
-    lw = Lowerer(instance_index)
+# `generators` (internal): how closure generators that trace are lowered; over a device limit the next way is taken
+function lower(x; nframes = SignalOperators.nframes(x), outtype = nothing, instance_index = 0, generators = :device)
+    lw = Lowerer(instance_index, generators)
     N, C = Int(nframes), nchannels(x)
     S = sampletype(x)
     T = outtype !== nothing ? outtype : S <: Union{Integer,Bool} ? Int64 : S <: Union{Float32,Float64} ? S : Float64
-    push!(lw.outputs, BufDesc(N, C, dtypecode(T)))
-    pieces = N > 0 ? lower_node(lw, x, 0, 0, N, 1, 0, 0, C) : Piece[]
-    push!(lw.stages, Stage(kind = STAGE_MAP, out_buf = (:out, 0), pieces = pieces, nchannels = C, n_out = N))
-    fuse_epilogues!(lw)
-    check_limits(lw)
+    try
+        push!(lw.outputs, BufDesc(N, C, dtypecode(T)))
+        pieces = N > 0 ? lower_node(lw, x, 0, 0, N, 1, 0, 0, C) : Piece[]
+        push!(lw.stages, Stage(kind = STAGE_MAP, out_buf = (:out, 0), pieces = pieces, nchannels = C, n_out = N))
+        fuse_epilogues!(lw)
+        check_limits(lw)
+    catch e
+        (e isa LoweringError && lw.traced_generators && generators !== :host) || rethrow()
+        return lower(x; nframes, outtype, instance_index, generators = generators === :device ? :temp : :host)
+    end
     Plan(tobytes(lw), lw.input_arrays, T)
 end
 
@@ -515,10 +614,15 @@ function lower_node(lw, x::SignalFunction, shift, lo, hi, cm, co, clo, chi)     
     end
     code = x.fn isa RandFn ? nothing : functor_code(x.fn)
     if code !== nothing && nchannels(x) == 1
-        fn, a, b = code
-        return [Piece(lo, hi, clo, chi, [Instr(OP_LOAD, LEAF_GEN; fn = fn, flags = ismissing(x.ω) ? 0x00 : FLAG_HAS_OMEGA,
-                                               i0 = shift + 1, d0 = Float64(fs), d1 = ismissing(x.ω) ? 0.0 : Float64(x.ω),
-                                               d2 = x.ϕ, d3 = a, d4 = b)])]
+        return [Piece(lo, hi, clo, chi, [gen_leaf(x, fs, shift, code...)])]
+    end
+    progs = x.fn isa RandFn || lw.generators === :host ? nothing : generator_programs(x, fs, shift)
+    if progs !== nothing
+        lw.traced_generators = true
+        lw.generators === :temp && any(p -> !isleaf(p), progs) &&
+            return materialize_generator!(lw, x, fs, shift, lo, hi, cm, co, clo, chi)
+        (cm == 0 || length(progs) == 1) && return [Piece(lo, hi, clo, chi, progs[(cm == 0 ? co : 0) + 1])]
+        return [Piece(lo, hi, c, c + 1, progs[c * cm + co + 1]) for c in clo:chi-1]
     end
     # not expressible on the device: frames lo+shift+1 .. hi+shift by the reference's own CPU sink
     vals = sink(Until(x, (hi + shift) * SignalOperators.frames), Array)[lo + shift + 1:hi + shift, :]
