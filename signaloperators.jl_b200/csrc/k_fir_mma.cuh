@@ -78,7 +78,6 @@ struct FirMmaParams {
     const int64_t* xi0;     // padded to a multiple of 64 entries
     const int32_t* poff;    // [m] (phase index - 1) * tapsper: row of output m in the banks
     const double* alpha;    // [m] fractional phase (0 for the rational kernels)
-    long long* dbg;         // optional [gridDim.x * gridDim.y][8] cycle counters (tuning aid), or nullptr
     int tab_doubles;        // nphases*tapsper: both banks are copied to shared memory
     double gain;            // constant-gain epilogue folded into the taps (1.0 = none)
 };
@@ -158,7 +157,6 @@ k_fir_mma(const __grid_constant__ FirMmaParams P) {
         const double* const src = lane < RPA ? s_src[myrow] : nullptr;
         double* const rrow = ring + (size_t)(lane < RPA ? myrow : 0) * P.pitch;
         int64_t have = pos_base;                        // positions below `have` are in the ring (or on their way)
-        long long dbg_acc[3] = {0, 0, 0};
         int wi = 0;                                     // ring index of position `have`
 
         // Extend the ring to position `need` (exclusive, even); completion is signalled on `bar`, where
@@ -222,13 +220,10 @@ k_fir_mma(const __grid_constant__ FirMmaParams P) {
             const int off_l = po_l - sh_l;
             const int lo_l = m_l < P.n_out ? sh_l : P.ks;                 // band rows [lo, sh + tapsper) hold taps
             // tile t-2 must be finished: its ring slots and its tap buffer are about to be overwritten
-            const long long c0 = P.dbg ? clock64() : 0;
             if (u >= 2) mbar_wait(&bar_done[s], (unsigned)((u >> 1) - 1) & 1u);
-            const long long c1 = P.dbg ? clock64() : 0;
 
             // ---- ring: the positions tile t+1 adds, requested a whole tile ahead of their use
             if (t + 1 < t1) extend(need, &bar_data[(u + 1) & 3]);
-            const long long c2 = P.dbg ? clock64() : 0;
 
             // ---- tap band of group `aux` for tile t: lanes along the band rows.  No FP64 instruction
             // other than the merges themselves, and those back to back: a DFMA issued from this warp
@@ -291,13 +286,7 @@ k_fir_mma(const __grid_constant__ FirMmaParams P) {
                 }
             }
             mbar_arrive(&bar_taps[s]);
-            if (P.dbg) {
-                const long long c3 = clock64();
-                dbg_acc[0] += c1 - c0; dbg_acc[1] += c2 - c1; dbg_acc[2] += c3 - c2;
-            }
         }
-        if (P.dbg && warp == NCW && lane == 0)
-            for (int i = 0; i < 3; ++i) P.dbg[((size_t)blockIdx.y * gridDim.x + blockIdx.x) * 8 + i] = dbg_acc[i];
     } else {
         // ---------------- DMMA ----------------
         const int g = warp & 3, half = warp >> 2;
@@ -319,7 +308,6 @@ k_fir_mma(const __grid_constant__ FirMmaParams P) {
         int64_t qprev = pos_base;
         int qidx = 0;                                   // ring index of position qprev
         int64_t q_nx = __ldg(P.xi0 + t0 * kFmT + 8 * g) - P.tapsper + 1;   // read one tile ahead
-        long long dbg_acc[4] = {0, 0, 0, 0};
         double prev[MF][2];                              // fragments of the previous tile, not yet stored
         int64_t mprev = -1;
         bool prev_full = false;                          // both outputs of the pending fragments exist
@@ -344,11 +332,8 @@ k_fir_mma(const __grid_constant__ FirMmaParams P) {
             double acc[MF][2];
 #pragma unroll
             for (int i = 0; i < MF; ++i) acc[i][0] = acc[i][1] = 0.0;
-            const long long c0 = P.dbg ? clock64() : 0;
             mbar_wait(&bar_taps[s], (unsigned)((t - t0) >> 1) & 1u);
-            const long long c1 = P.dbg ? clock64() : 0;
             mbar_wait(&bar_data[(t - t0) & 3], (unsigned)((t - t0) >> 2) & 1u);
-            const long long c2 = P.dbg ? clock64() : 0;
             auto step = [&](int ks) {
                 const double b = bp[ks * 4 * kFmHbPitch];
                 const double* ap = arow + idx;
@@ -378,15 +363,9 @@ k_fir_mma(const __grid_constant__ FirMmaParams P) {
 #pragma unroll
                 for (int i = 0; i < MF; ++i) ssq[i] = fma(acc[i][0], acc[i][0], fma(acc[i][1], acc[i][1], ssq[i]));
             }
-            if (P.dbg) {
-                const long long c3 = clock64();
-                dbg_acc[0] += c1 - c0; dbg_acc[1] += c2 - c1; dbg_acc[2] += c3 - c2;
-            }
         }
 #pragma unroll
         for (int i = 0; i < MF; ++i) store_frag(dstp[i], mprev, mprev + 1 < P.n_out, prev[i][0], prev[i][1]);
-        if (P.dbg && warp == 0 && lane == 0)
-            for (int i = 0; i < 4; ++i) P.dbg[((size_t)blockIdx.y * gridDim.x + blockIdx.x) * 8 + 3 + i] = dbg_acc[i];
         if (SSQ) {
 #pragma unroll
             for (int i = 0; i < (SSQ ? MF : 1); ++i) {

@@ -77,9 +77,6 @@ struct FirTmParams {
     int period_tiles;
     int64_t epoch_tiles;    // one period table per epoch of this many tiles (the phase accumulator's drift), n_epochs of them
     int n_epochs;
-    long long* dbg;         // optional [blocks][8] cycle counters (tuning aid, SIGOPS_FIR_DBG=1), or nullptr
-    int exp;                // tuning experiments (SIGOPS_FIR_EXP bit mask; wrong results): 1 no staging stores, 2 no tensor
-                            // stores, 4 no tap-band building, 8 no ring loads, 16 compute warps do not wait for bands / data
 };
 
 inline size_t fir_tm_smem_bytes(int nslot, int ks, int tab_doubles, bool has_dpfb) {
@@ -90,7 +87,7 @@ inline size_t fir_tm_smem_bytes(int nslot, int ks, int tab_doubles, bool has_dpf
 // The dynamic shared memory of this kernel is addressed through 32-bit shared-window addresses and
 // explicit ld.shared / st.shared (lds_f64, sts_f64, sts_v2f64): the 1024-byte alignment of the swizzled
 // boxes is computed on the address, and a pointer rebuilt from it would make every access a generic LD/ST.
-template <bool SSQ, bool DBG = false>
+template <bool SSQ>
 __global__ void __launch_bounds__(kFtThreads, 1)
 k_fir_tmap(const __grid_constant__ FirTmParams P, const __grid_constant__ CUtensorMap tm_in,
            const __grid_constant__ CUtensorMap tm_out) {
@@ -177,7 +174,6 @@ k_fir_tmap(const __grid_constant__ FirTmParams P, const __grid_constant__ CUtens
             x7_nx = __ldg(xp + (int64_t)u * kFmT + 7);
         };
         fetch_idx(0);
-        long long dbg_acc[5] = {0, 0, 0, 0, 0};   // (DBG) wait taps, set-up, wait staging, staging, -
 
         // The band starts at the group's own first window position, so every lane tracks its own position
         // p = first + kk + 4b.  Four blocks are 16 positions = one ring slot: within a tile, block b = 4c + J sits
@@ -208,7 +204,6 @@ k_fir_tmap(const __grid_constant__ FirTmParams P, const __grid_constant__ CUtens
         // Set tile t up (index arithmetic, barrier wait) and load the operands of its first block into `o`.
         // Runs underneath the last block of the tile before it.
         auto setup = [&](int u, Ops& o) {
-            const long long cs = DBG ? clock64() : 0;
             const int s = u & 1;
             const int r = (int)(xq_nx - P.tapsper + 1 - pos_base) + kk;            // >= 0: my position of block 0
             int n = (int)(x7_nx - xq_nx) + P.tapsper + 3;
@@ -234,11 +229,8 @@ k_fir_tmap(const __grid_constant__ FirTmParams P, const __grid_constant__ CUtens
             bq = bands + s * band_tile + bcol;
             // one barrier per tile: the helpers arrive on it once the tile's band is built AND its ring slots
             // have landed (they watch the `full` barriers, off the compute warps' path)
-            const long long c0 = DBG ? clock64() : 0;
-            if (!(P.exp & 16)) mbar_wait(a_taps + 8u * s, (unsigned)(u >> 1) & 1u);
-            if (DBG) dbg_acc[0] += clock64() - c0;
+            mbar_wait(a_taps + 8u * s, (unsigned)(u >> 1) & 1u);
             load_ops(o, std::integral_constant<int, 0>{});
-            if (DBG) dbg_acc[1] += clock64() - cs;
         };
         auto mma_block = [&](double (&acc)[F][2], const Ops& o) {
 #pragma unroll
@@ -249,27 +241,20 @@ k_fir_tmap(const __grid_constant__ FirTmParams P, const __grid_constant__ CUtens
         // arrival two blocks later — issued right behind the stores the fence would hold the warp (and its DMMAs)
         // until they have drained through the LSU queue (~400 cycles per tile, measured).
         auto stage_store = [&](double (&o)[F][2], int u_old) {
-            const long long c0 = DBG ? clock64() : 0;
             if (u_old > 0) mbar_wait(a_free, (unsigned)(u_old - 1) & 1u);
-            if (DBG) dbg_acc[2] += clock64() - c0;
-            if (!(P.exp & 1)) {
-                const unsigned sp = srow + (gw >> 1) * 16384 + ((unsigned)(((gw & 1) * 4 + kk) << 4) ^ key);
+            const unsigned sp = srow + (gw >> 1) * 16384 + ((unsigned)(((gw & 1) * 4 + kk) << 4) ^ key);
 #pragma unroll
-                for (int i = 0; i < F; ++i) sts_v2f64(sp + i * 1024, o[i][0], o[i][1]);
-            }
+            for (int i = 0; i < F; ++i) sts_v2f64(sp + i * 1024, o[i][0], o[i][1]);
             if (SSQ) {
                 // outputs past n_out have all-zero taps, rows past the last read zeros: exactly 0
 #pragma unroll
                 for (int i = 0; i < F; ++i) ssq[i] = fma(o[i][0], o[i][0], fma(o[i][1], o[i][1], ssq[i]));
             }
-            if (DBG) dbg_acc[3] += clock64() - c0;
         };
         auto stage_signal = [&]() {
-            const long long c0 = DBG ? clock64() : 0;
             fence_async_smem();
             __syncwarp();
             if (lead) mbar_arrive(a_full);
-            if (DBG) dbg_acc[3] += clock64() - c0;
         };
         // One tile: its DMMAs accumulate into `acc` while the fragments of the tile before it (`old`) drain to
         // the staging boxes underneath its first block and, during the last block, the next tile is set up and its
@@ -345,14 +330,9 @@ k_fir_tmap(const __grid_constant__ FirTmParams P, const __grid_constant__ CUtens
 
         double accA[F][2], accB[F][2];
         setup(0, o0);
-        const long long cstart = DBG ? clock64() : 0;
         for (int u = 0; u < nt; u += 2) {
             tile(accA, accB, u);
             if (u + 1 < nt) tile(accB, accA, u + 1);
-        }
-        if (DBG && warp == 0 && lane == 0) {
-            long long* d = P.dbg + ((size_t)blockIdx.y * gridDim.x + blockIdx.x) * 8;
-            d[0] = dbg_acc[0]; d[1] = dbg_acc[1]; d[2] = dbg_acc[2]; d[3] = clock64() - cstart; d[6] = dbg_acc[3];
         }
         if (nt & 1) stage_store(accA, nt - 1);
         else stage_store(accB, nt - 1);
@@ -397,7 +377,7 @@ k_fir_tmap(const __grid_constant__ FirTmParams P, const __grid_constant__ CUtens
                     ep = ep < P.n_epochs ? ep : P.n_epochs - 1;
                     const double* src = P.bands_g + (size_t)(ep * P.period_tiles + t % P.period_tiles) * (bytes / 8);
                     bulk_load(bands + (unsigned)s * band_tile, src, bytes, smem_u32(&bar_taps[s]));
-                    while (jwait < hi && !(P.exp & 8)) {                                          // ... and the tile's window has landed
+                    while (jwait < hi) {                                                          // ... and the tile's window has landed
                         mbar_wait(&bar_full[jw_slot], jw_par);
                         ++jwait;
                         if (++jw_slot == P.nslot) { jw_slot = 0; jw_par ^= 1u; }
@@ -411,7 +391,6 @@ k_fir_tmap(const __grid_constant__ FirTmParams P, const __grid_constant__ CUtens
         const unsigned pf_tab = tabs, dpf_tab = tabs + 8u * P.tab_doubles;
         const bool has_d = P.dpfb != nullptr;
         const int nblk = P.ks >> 3;                        // 8-row band blocks (ks is a multiple of 8 here)
-        long long hdbg[2] = {0, 0};
         int64_t jwait = 0;                              // ring slots [0, jwait) have been seen to land
         int jw_slot = 0;
         unsigned jw_par = 0;
@@ -447,14 +426,11 @@ k_fir_tmap(const __grid_constant__ FirTmParams P, const __grid_constant__ CUtens
             const double b0v = (kk == rr) ? al_b : 0.0, b1v = (4 + kk == rr) ? al_b : 0.0;
             const unsigned band = bands + s * band_tile + (unsigned)(grp * P.ks) * 64u;
             // tile t-2 must be finished: its band buffer is about to be overwritten
-            const long long c0 = DBG ? clock64() : 0;
             if (u >= 2) mbar_wait(&bar_done[(u - 2) & 3], (unsigned)((u - 2) >> 2) & 1u);
-            const long long c1 = DBG ? clock64() : 0;
-            if (DBG) hdbg[0] += c1 - c0;
             // batches of four 8-row blocks: all table look-ups first, then the (independent) DMMAs, then the stores —
             // a helper's instructions queue behind the compute warps' DMMA stream, so a dependent
             // look-up -> DMMA -> DMMA -> store chain per block would pay that queueing four times per block
-            for (int b0 = 0; b0 < ((P.exp & 4) ? 0 : nblk); b0 += 4) {
+            for (int b0 = 0; b0 < nblk; b0 += 4) {
                 double cv0[4], cv1[4], a0[4], a1[4];
 #pragma unroll
                 for (int i = 0; i < 4; ++i) {
@@ -483,24 +459,19 @@ k_fir_tmap(const __grid_constant__ FirTmParams P, const __grid_constant__ CUtens
                 }
             }
             // ... and the tile's window has landed in the ring
-            while (jwait < hi && !(P.exp & 8)) {
+            while (jwait < hi) {
                 mbar_wait(&bar_full[jw_slot], jw_par);
                 ++jwait;
                 if (++jw_slot == P.nslot) { jw_slot = 0; jw_par ^= 1u; }
             }
             mbar_arrive(&bar_taps[s]);
-            if (DBG) hdbg[1] += clock64() - c1;
-        }
-        if (DBG && grp == 0 && lane == 0) {
-            long long* d = P.dbg + ((size_t)blockIdx.y * gridDim.x + blockIdx.x) * 8;
-            d[4] = hdbg[0]; d[5] = hdbg[1];
         }
     } else {
       // (one setmaxnreg for the whole fourth warpgroup: producer, store and two warps that only give registers away)
       asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(kFtRegsMisc));
       if (warp == kFtNCW + kFtNAW) {
         // ---------------- producer: one tensor copy per ring slot, as far ahead as the ring allows ----------------
-        if (lane == 0 && !(P.exp & 8)) {
+        if (lane == 0) {
             const int64_t last_need = __ldg(P.xi0 + (t1 - 1) * kFmT + kFmT - 1) + 4;
             const int64_t nslots_total = (last_need - pos_base + (kFtSlotPos - 1)) >> 4;
             auto lo_of = [&](int64_t t) { return (__ldg(P.xi0 + t * kFmT) - P.tapsper + 1 - pos_base) >> 4; };
@@ -517,11 +488,10 @@ k_fir_tmap(const __grid_constant__ FirTmParams P, const __grid_constant__ CUtens
                     }
                     const unsigned target = (unsigned)(tp - t0 + 1) * kFtNCW;
                     unsigned seen;
-                    // (polled with a pause: a spinning warp takes issue slots from the compute warps of its sub-partition)
+                    // (polled in a tight spin, no pause between reads)
                     while (true) {
                         asm volatile("ld.acquire.cta.shared::cta.u32 %0, [%1];" : "=r"(seen) : "r"(smem_u32(&done_count)) : "memory");
                         if (seen >= target) break;
-                        if (P.exp & 32) __nanosleep(64);
                     }
                 }
                 mbar_expect_tx(&bar_full[s], kFtSlotBytes);
@@ -538,7 +508,7 @@ k_fir_tmap(const __grid_constant__ FirTmParams P, const __grid_constant__ CUtens
                 const int64_t u = t - t0;
                 mbar_wait(&bar_stg_full[h], (unsigned)u & 1u);
                 const int64_t m0 = t * kFmT;
-                if (!(P.exp & 2) && rows_live) {
+                if (rows_live) {
                     tmap_store_2d(&tm_out, (int)m0, row0 + 64 * h, stg + 8192u * h);
                     if (m0 + 16 < P.n_out) tmap_store_2d(&tm_out, (int)(m0 + 16), row0 + 64 * h, stg + 16384 + 8192u * h);
                 }

@@ -4,7 +4,6 @@
 // sharding over devices (no collectives: instances are independent, SURVEY.md
 // §8e) and the host<->device pipeline of `sigops_plan_run`.
 #include <algorithm>
-#include <array>
 #include <atomic>
 #include <chrono>
 #include <cmath>
@@ -1003,7 +1002,6 @@ struct Wave {                 // what the wave knows when its stages are planned
     int64_t ninst, inst0;
     size_t si;                // stage being planned
     Arena& arena;             // IIR state
-    cudaStream_t stream;      // (the synchronous SIGOPS_FIR_DBG launches)
     std::vector<Slot::Prepared>& launches;
     void add(int kind, std::function<void(cudaStream_t)> fn) const { launches.push_back({kind, std::move(fn)}); }
 };
@@ -1083,26 +1081,6 @@ const double* period_bands(const Wave& w, int ks) {
     CUDA_OK(cudaMemcpy(dptr, tab.data(), tab.size() * sizeof(double), cudaMemcpyHostToDevice));
     w.pd.bands.emplace(key, dptr);
     return dptr;
-}
-
-// Tuning aid (SIGOPS_FIR_DBG=1): `launch` runs a FIR kernel once with per-block cycle counters ([nblocks][8]); the
-// counters summed over the blocks, per tile.
-std::array<double, 8> fir_cycles_per_tile(cudaStream_t stream, size_t nblocks, int64_t tiles_per_seg,
-                                          const std::function<void(long long*)>& launch) {
-    long long* dbg = nullptr;
-    CUDA_OK(cudaMalloc(&dbg, nblocks * 8 * sizeof(long long)));
-    CUDA_OK(cudaMemset(dbg, 0, nblocks * 8 * sizeof(long long)));
-    launch(dbg);
-    CUDA_OK(cudaStreamSynchronize(stream));
-    std::vector<long long> h(nblocks * 8);
-    CUDA_OK(cudaMemcpy(h.data(), dbg, h.size() * sizeof(long long), cudaMemcpyDeviceToHost));
-    cudaFree(dbg);
-    std::array<double, 8> sum{};
-    for (size_t b = 0; b < nblocks; ++b)
-        for (int k = 0; k < 8; ++k) sum[k] += (double)h[b * 8 + k];
-    const double per = 1.0 / ((double)nblocks * (double)tiles_per_seg);
-    for (double& v : sum) v *= per;
-    return sum;
 }
 
 // One launch with `smem` bytes of dynamic shared memory (opted in once per kernel, size and device).
@@ -1360,7 +1338,6 @@ bool plan_fir_tmap(const Wave& w, const FirParams& P) {
     T.bands_g = bands_g; T.period_tiles = period_tiles;
     T.epoch_tiles = s.fir.epoch_tiles; T.n_epochs = (int)s.fir.n_epochs;
     T.gain = s.fir.epi_scale;
-    if (const char* e = getenv("SIGOPS_FIR_EXP")) T.exp = atoi(e);
     const int64_t groups = (rows + kFtRows - 1) / kFtRows;
     if (groups > 65535) return false;
     T.tiles_per_seg = choose_tiles_per_segment(T.ntiles, groups, w.sm_count);
@@ -1372,16 +1349,6 @@ bool plan_fir_tmap(const Wave& w, const FirParams& P) {
                 w.si, (long long)rows, (long long)g.n_out, T.tapsper, ks, nslot, win_slots, (long long)nseg, (long long)groups,
                 (long long)T.tiles_per_seg, smem, T.gain, (long long)s.fir.period, bands_g ? " (tap bands from the period tables)" : "");
         if (bands_g) fprintf(stderr, "[sigops]   %lld epochs of %lld tiles\n", (long long)s.fir.n_epochs, (long long)s.fir.epoch_tiles);
-    }
-    if (getenv("SIGOPS_FIR_DBG")) {
-        const auto c = fir_cycles_per_tile(w.stream, (size_t)nseg * groups, T.tiles_per_seg, [&](long long* dbg) {
-            FirTmParams D = T;
-            D.dbg = dbg;
-            launch_dyn_smem(k_fir_tmap<false, true>, tgrid, kFtThreads, smem, w.stream, D, *(const CUtensorMap*)&mi,
-                            *(const CUtensorMap*)&mo);
-        });
-        fprintf(stderr, "[sigops] FIR tmap cycles/tile  compute: set-up %.0f (of it wait_taps %.0f) staging %.0f (of it wait_stg %.0f) total %.0f | helper: wait_done %.0f build %.0f\n",
-                c[1], c[0], c[6], c[2], c[3], c[4], c[5]);
     }
     const auto kernel = g.sumsq_slot >= 0 ? k_fir_tmap<true> : k_fir_tmap<false>;
     w.add(KIND_FIR, [=](cudaStream_t st) {
@@ -1427,15 +1394,6 @@ bool plan_fir_mma(const Wave& w, const FirParams& P) {
         fprintf(stderr, "[sigops] FIR stage %zu: mma rows=%lld n_out=%lld taps=%d ks=%d ring=%d pitch=%d rows/block=%d grid=%lldx%lld tiles/seg=%lld smem=%zu\n",
                 w.si, (long long)rows, (long long)g.n_out, Q.tapsper, Q.ks, Q.ring, Q.pitch, RB, (long long)nseg,
                 (long long)groups, (long long)Q.tiles_per_seg, smem);
-    if (getenv("SIGOPS_FIR_DBG")) {
-        const auto c = fir_cycles_per_tile(w.stream, (size_t)nseg * groups, Q.tiles_per_seg, [&](long long* dbg) {
-            FirMmaParams D = Q;
-            D.dbg = dbg;
-            if (RB == 128) launch_dyn_smem(k_fir_mma<8, 2, false>, grid, 16 * 32, smem, w.stream, D);
-        });
-        fprintf(stderr, "[sigops] FIR cycles/tile  aux: wait_done %.0f extend %.0f taps %.0f | compute: wait_taps %.0f wait_data %.0f dmma %.0f store %.0f\n",
-                c[0], c[1], c[2], c[3], c[4], c[5], c[6]);
-    }
     const bool ssq = Q.sumsq_slot >= 0;
     const auto kernel = RB == 128 ? (ssq ? k_fir_mma<8, 2, true> : k_fir_mma<8, 2, false>)
                       : RB == 64  ? (ssq ? k_fir_mma<4, 2, true> : k_fir_mma<4, 2, false>)
@@ -1666,7 +1624,7 @@ int64_t enqueue_wave(sigops_plan& p, int di, Slot& slot, cudaStream_t stream, co
     slot.cache_plan = 0;
     // (slot.last_table now holds this wave's table)
     Wave w{p, pd, dev.sm_count, (const BufRef*)slot.last_table.data(), d_refs, scalars, nbuf, nscal, ninst, io.inst0, 0,
-           slot.arena, stream, slot.cache_launches};
+           slot.arena, slot.cache_launches};
     for (w.si = 0; w.si < p.stages.size(); ++w.si) {
         switch (p.stages[w.si].st.kind) {
             case SIGOPS_STAGE_MAP: plan_map_stage(w); break;
@@ -1823,7 +1781,6 @@ void parallel_copy(const std::vector<CopyPiece>& pieces, int nthreads) {
 }
 
 int copy_threads(int ndev) {
-    if (const char* e = getenv("SIGOPS_COPY_THREADS")) return std::max(1, atoi(e));
     const int hw = (int)std::thread::hardware_concurrency();
     return std::max(1, std::min(8, (hw > 0 ? hw : 8) / std::max(1, ndev)));
 }
