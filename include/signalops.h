@@ -100,6 +100,20 @@ void sigops_plan_destroy(sigops_plan* plan);
 int sigops_plan_run(sigops_plan* plan, int64_t ninst,
                     const sigops_buffer* in, sigops_buffer* out, sigops_stats* stats);
 
+/* Ragged batch: `ninst` instances of a plan built for the longest of them, each with its own lengths.  Every
+ * host buffer may hold fewer frames than the plan declares (`nframes` <= the plan's; same channels and sample
+ * type, no SIGOPS_INTERLEAVED); `temp_frames` holds ninst*n_temps valid frame counts of the temps, instance-
+ * major.  An instance's results are the first frames of what the plan computes from its inputs extended with
+ * zeros, with every buffer read as zero past the instance's valid frames and each sum of squares taken over the
+ * instance's valid frames of its stage's output: exactly the instance's own plan, for plans whose lengths are
+ * the only difference (the host lowering checks that).  Each RMS leaf divides by d0 * (the instance's frames x
+ * channels) / (the plan's), so every RMS leaf of one scalar slot must carry the same d0.  Instances run longest
+ * first (in the caller's order when the plan draws device noise) and devices take about equal output samples.
+ * Only the instance's valid output frames are written.  Costs over an equal-length batch: one reduction pass
+ * per sum of squares, the zero tails and the frames each wave computes past its shorter instances' lengths. */
+int sigops_plan_run_ragged(sigops_plan* plan, int64_t ninst, const sigops_buffer* in, sigops_buffer* out,
+                           const int64_t* temp_frames, sigops_stats* stats);
+
 /* Page-locked host memory for sample buffers.  `sigops_plan_run` accepts ANY host pointer: page-locked
  * memory (from here, cudaHostAlloc or cudaHostRegister) is read and written by the DMA engines directly;
  * pageable memory (a plain Julia `Array`, malloc) is staged through the library's own pinned ring by a few

@@ -32,6 +32,7 @@
 #include "k_fir_tmap.cuh"
 #include "k_iir_tmap.cuh"
 #include "k_map.cuh"
+#include "k_ragged.cuh"
 #include "k_wav.cuh"
 
 static_assert(sizeof(sigops_instr) == 80, "ABI: sigops_instr");
@@ -262,6 +263,7 @@ struct sigops_plan {
     int max_stack = 0;
     bool has_randn = false;        // some program draws device noise (LEAF_RANDN): launches depend on the wave's first instance index
     bool has_fn = false;           // some program applies closure functions (FN1 / FN2 / POPFN2): k_map's variant with them
+    std::vector<double> slot_d0;   // per scalar slot: d0 of the RMS leaves reading it (0 = none, NaN = they disagree)
     uint64_t uid = 0;
 };
 
@@ -807,9 +809,14 @@ void parse_plan(sigops_plan& p, const void* bytes, size_t nbytes) {
         } else
             fail(SIGOPS_ERR_INVALID, "%s: unknown kind %d", what, g.kind);
     }
+    p.slot_d0.assign(p.h.n_scalars, 0.0);
     for (const sigops_instr& I : p.instrs) {
         if (op_has_leaf(I.op) && I.leaf == SIGOPS_LEAF_RANDN) p.has_randn = true;
         if (I.op >= SIGOPS_OP_FN1) p.has_fn = true;
+        if (op_has_leaf(I.op) && I.leaf == SIGOPS_LEAF_RMS) {
+            double& d = p.slot_d0[I.buf];
+            d = d == 0.0 || d == I.d0 ? I.d0 : NAN;
+        }
     }
 }
 
@@ -882,8 +889,7 @@ struct IirLaunch {
 //                         chunks of a row (one 2Mx2M mat-vec each, ~3 frame-times) and two more launches
 // Measured on B200 (README scene, W = 3307: WARM L = 3360 -> 0.375 ms, MAIN/CARRY/FIX L = 240 ->
 // 0.035 + 0.042 + 0.034 ms; 512 such rows: 0.735 ms vs 0.29 ms).
-IirLaunch choose_iir_chunking_flat(const StageRT& s, int64_t rows, int sm_count, bool allow_matrix = true) {
-    const int64_t N = s.st.n_out;
+IirLaunch choose_iir_chunking_flat(const StageRT& s, int64_t N, int64_t rows, int sm_count, bool allow_matrix = true) {
     const int64_t W64 = round_up(std::max<int64_t>(s.iir.W, 1), kStageCols);
     const int64_t jmax = std::max<int64_t>(1, (N + kStageCols - 1) / kStageCols);
     double best = 1e300;
@@ -930,8 +936,7 @@ IirLaunch choose_tmap_chunking(int64_t N, int64_t rows, int64_t stage_cols, int6
     return IirLaunch{0, bestL, Wst, bestL ? (N + bestL - 1) / bestL : 0, false, best};
 }
 
-IirLaunch choose_iir_chunking(const StageRT& s, int64_t rows, int sm_count) {
-    const int64_t N = s.st.n_out;
+IirLaunch choose_iir_chunking(const StageRT& s, int64_t N, int64_t rows, int sm_count) {
     const int64_t W32 = round_up(std::max<int64_t>(s.iir.W, 1), 32);
     const int64_t target_blocks = (int64_t)sm_count * 4;
     int bpr = 1;
@@ -957,6 +962,8 @@ struct WaveIO {
     const sigops_buffer* in;   // device pointers, [ninst][n_inputs]
     const sigops_buffer* out;  // [ninst][n_outputs]
     int64_t inst0 = 0;         // index of the wave's first instance in the whole call (LEAF_RANDN streams)
+    const int64_t* temp_frames = nullptr;   // ragged run: valid frames of every temp, [ninst][n_temps]; the valid frames
+                                            // of inputs and outputs are their buffers' nframes
 };
 
 size_t temp_bytes_per_instance(const sigops_plan& p) {
@@ -968,23 +975,26 @@ size_t temp_bytes_per_instance(const sigops_plan& p) {
     return total;
 }
 
-size_t iir_state_bytes(const sigops_plan& p, int64_t ninst, int sm_count) {
+// `n`: frames of every stage in the wave (a ragged wave's prefixes), nullptr = the plan's
+size_t iir_state_bytes(const sigops_plan& p, int64_t ninst, int sm_count, const int64_t* n = nullptr) {
     size_t total = 0;   // every IIR stage of a wave takes its own state arrays from the arena
-    for (auto& s : p.stages) {
+    for (size_t si = 0; si < p.stages.size(); ++si) {
+        const StageRT& s = p.stages[si];
         if (s.st.kind != SIGOPS_STAGE_IIR) continue;
-        const int64_t rows = ninst * s.st.nchannels;
-        const IirLaunch a = choose_iir_chunking(s, rows, sm_count);
+        const int64_t rows = ninst * s.st.nchannels, N = n ? n[si] : s.st.n_out;
+        const IirLaunch a = choose_iir_chunking(s, N, rows, sm_count);
         size_t slots = (size_t)rows * a.blocks_per_row * kIirThreads;
-        if (s.iir.fast || s.iir.tma_prog) slots = std::max(slots, (size_t)rows * choose_iir_chunking_flat(s, rows, sm_count).nchunks);
+        if (s.iir.fast || s.iir.tma_prog) slots = std::max(slots, (size_t)rows * choose_iir_chunking_flat(s, N, rows, sm_count).nchunks);
         total += (size_t)2 * (2 * s.iir.M) * slots * sizeof(double) + 4096 + 1024;
     }
     return total;
 }
 
-size_t wave_workspace_bytes(const sigops_plan& p, int64_t ninst, int sm_count) {
-    return temp_bytes_per_instance(p) * ninst + iir_state_bytes(p, ninst, sm_count) +
-           (size_t)ninst * p.nbuf() * sizeof(BufRef) + (size_t)ninst * std::max<uint32_t>(p.h.n_scalars, 1) * sizeof(double) +
-           (1 << 16);
+// `n` as for iir_state_bytes; a ragged wave (n given) also uploads its table of valid frames
+size_t wave_workspace_bytes(const sigops_plan& p, int64_t ninst, int sm_count, const int64_t* n = nullptr) {
+    return temp_bytes_per_instance(p) * ninst + iir_state_bytes(p, ninst, sm_count, n) +
+           (size_t)ninst * p.nbuf() * (sizeof(BufRef) + (n ? sizeof(int64_t) : 0)) +
+           (size_t)ninst * std::max<uint32_t>(p.h.n_scalars, 1) * sizeof(double) + (1 << 16);
 }
 
 // ---- stage launch planning ------------------------------------------------------
@@ -1003,8 +1013,18 @@ struct Wave {                 // what the wave knows when its stages are planned
     size_t si;                // stage being planned
     Arena& arena;             // IIR state
     std::vector<Slot::Prepared>& launches;
+    // the stage's frames and sum-of-squares slot in this wave: the plan's, except in a ragged run, where a stage
+    // computes the prefix its longest instance needs and its sums of squares are taken by k_sumsq_rows
+    int64_t n_out = 0;
+    int sumsq_slot = -1;
     void add(int kind, std::function<void(cudaStream_t)> fn) const { launches.push_back({kind, std::move(fn)}); }
 };
+
+// Frames a ragged wave computes for stage `si`: the prefix its longest instance needs (`vmax` valid frames of the
+// stage's output), rounded up to 16 frames within the plan's.
+int64_t ragged_stage_frames(const sigops_plan& p, size_t si, int64_t vmax) {
+    return std::min(p.bufs[p.stages[si].st.out_buf].nframes, round_up(vmax, 16));
+}
 
 // Every instance's rows of buffer `buf` start on a 16-byte boundary (several channels: an even number of
 // elements apart), and with `f64` hold Float64: what the bulk copies of the TMA and tensor-core kernels need.
@@ -1096,18 +1116,22 @@ void plan_map_stage(const Wave& w) {
     MapParams P{};
     P.instrs = w.pd.instrs; P.bufrefs = w.d_refs; P.scalars = w.scalars; P.inst0 = w.inst0;
     P.nbuf = w.nbuf; P.nscalars = w.nscal;
-    P.out_buf = g.out_buf; P.sumsq_slot = g.sumsq_slot; P.out_nch = p.bufs[g.out_buf].nchannels;
+    P.out_buf = g.out_buf; P.sumsq_slot = w.sumsq_slot; P.out_nch = p.bufs[g.out_buf].nchannels;
     P.n_pieces = g.n_pieces;
+    // pieces clipped to the wave's frames
+    for (int k = 0; k < g.n_pieces; ++k) {
+        P.pieces[k] = p.pieces[g.piece_start + k];
+        P.pieces[k].out_len = std::max<int64_t>(0, std::min(P.pieces[k].out_len, w.n_out - P.pieces[k].out_start));
+    }
     // frames per block: four 2048-frame passes amortise the per-block set-up, unless that would
     // leave the GPU with fewer than a few blocks per SM
     int64_t subs = 0;
     for (int k = 0; k < g.n_pieces; ++k)
-        subs += (p.pieces[g.piece_start + k].out_len + kMapSub - 1) / kMapSub * p.pieces[g.piece_start + k].ch_count;
+        subs += (P.pieces[k].out_len + kMapSub - 1) / kMapSub * P.pieces[k].ch_count;
     P.passes = subs * w.ninst >= (int64_t)kMapPasses * w.sm_count * 8 ? kMapPasses : 1;
     const int64_t per_block = (int64_t)kMapSub * P.passes;
     int tiles = 0;
     for (int k = 0; k < g.n_pieces; ++k) {
-        P.pieces[k] = p.pieces[g.piece_start + k];
         P.tile_prefix[k] = tiles;
         tiles += (int)((P.pieces[k].out_len + per_block - 1) / per_block);
     }
@@ -1141,16 +1165,16 @@ bool plan_iir_tmap(const Wave& w, bool tma) {
     const int esz = f32 ? 4 : 8;
     const int stage_cols = f32 ? 32 * kTmSubsPerStageF32 : (rowinv ? kTmSub * kTmSubsPerStageLv : kTmStageCols);
     if (!((tma && s.iir.fast) || f32 || rowinv) || getenv("SIGOPS_NO_TMAP") || !iir_tmap_available() ||
-        !(rows % 32 == 0 || rows >= 256) || rows * 32 >= (int64_t(1) << 31) || g.n_out >= (int64_t(1) << 30))
+        !(rows % 32 == 0 || rows >= 256) || rows * 32 >= (int64_t(1) << 31) || w.n_out >= (int64_t(1) << 30))
         return false;
     char *bin = nullptr, *bout = nullptr;
     int64_t sin_ = 0, sout = 0;
     const int dtype = f32 ? SIGOPS_F32 : SIGOPS_F64;
     const int64_t Wst = round_up(std::max<int64_t>(s.iir.W, 1), stage_cols);
     if (!strided_matrix(w.refs, w.ninst, w.nbuf, s.iir.plain_buf, esz, dtype, &bin, &sin_) ||
-        !strided_matrix(w.refs, w.ninst, w.nbuf, g.out_buf, esz, dtype, &bout, &sout) || 2 * Wst > g.n_out)
+        !strided_matrix(w.refs, w.ninst, w.nbuf, g.out_buf, esz, dtype, &bout, &sout) || 2 * Wst > w.n_out)
         return false;
-    const int64_t N = g.n_out, groups = (rows + 31) / 32;
+    const int64_t N = w.n_out, groups = (rows + 31) / 32;
     const int nw = f32 ? kTmWarpsF32 : (rowinv ? kTmWarpsLv : kTmWarps);
     const IirLaunch c = choose_tmap_chunking(N, rows, stage_cols, Wst, nw, rowinv, w.sm_count);
     // A slowly decaying filter is better served by k_iir_tma's short chunks and carry pass.
@@ -1158,7 +1182,7 @@ bool plan_iir_tmap(const Wave& w, bool tma) {
     // cycles (measured: 210 with 256 lanes, 102 with 128), which makes them comparable.
     auto frame_cycles = [](int lanes) { return std::max(100.0, 0.82 * lanes); };
     const bool tmap_wins = c.cost * frame_cycles(32 * nw) <=
-                           choose_iir_chunking_flat(s, rows, w.sm_count).cost * frame_cycles(32 * kTmaWarps);
+                           choose_iir_chunking_flat(s, w.n_out, rows, w.sm_count).cost * frame_cycles(32 * kTmaWarps);
     TensorMapBlob mi, mo;
     // (a Float32 stage has no other fast kernel to fall back on: take this one whenever it applies)
     if (!(c.L > Wst && (tmap_wins || f32 || rowinv) &&
@@ -1167,7 +1191,7 @@ bool plan_iir_tmap(const Wave& w, bool tma) {
         return false;
     IirTmapParams T{};
     T.bufrefs = w.d_refs; T.scalars = w.scalars; T.nbuf = w.nbuf; T.nscalars = w.nscal;
-    T.out_buf = g.out_buf; T.sumsq_slot = g.sumsq_slot; T.nch = g.nchannels; T.nrows = rows;
+    T.out_buf = g.out_buf; T.sumsq_slot = w.sumsq_slot; T.nch = g.nchannels; T.nrows = rows;
     T.N = N; T.L = c.L; T.Wc = Wst;
     T.cpr = c.nchunks;
     T.nunits = groups * T.cpr;
@@ -1211,7 +1235,7 @@ void plan_iir_stage(const Wave& w) {
     const sigops_plan& p = w.p;
     const StageRT& s = p.stages[w.si];
     const sigops_stage& g = s.st;
-    if (g.n_out == 0) return;
+    if (w.n_out == 0) return;
     const int64_t rows = w.ninst * g.nchannels;
     // TMA path: fast-path stage whose every channel starts on a 16-byte boundary
     bool tma = (s.iir.fast || s.iir.tma_prog) && rows_aligned(w.refs, w.ninst, w.nbuf, s.iir.plain_buf, false) &&
@@ -1219,24 +1243,24 @@ void plan_iir_stage(const Wave& w) {
     if (plan_iir_tmap(w, tma)) return;
     if (s.iir.prog_stack) tma = false;   // (k_iir_tma interprets no stack)
     // (the program-carrying TMA kernel has no MAIN/FIX form: keep it to chunkings it can run)
-    IirLaunch c = tma ? choose_iir_chunking_flat(s, rows, w.sm_count, !s.iir.tma_prog) : choose_iir_chunking(s, rows, w.sm_count);
+    IirLaunch c = tma ? choose_iir_chunking_flat(s, w.n_out, rows, w.sm_count, !s.iir.tma_prog) : choose_iir_chunking(s, w.n_out, rows, w.sm_count);
     // the program-carrying TMA kernel only exists in the single-launch WARM form (for a filter that does not decay
     // within the row that is one serial chunk per row: the generic kernel's carry pass does better)
     bool tprog = tma && s.iir.tma_prog;
-    if (tprog && (c.need_matrix || s.iir.W >= g.n_out)) {
+    if (tprog && (c.need_matrix || s.iir.W >= w.n_out)) {
         tma = tprog = false;
-        c = choose_iir_chunking(s, rows, w.sm_count);
+        c = choose_iir_chunking(s, w.n_out, rows, w.sm_count);
     }
     IirParams P{};
     P.instrs = w.pd.instrs; P.bufrefs = w.d_refs; P.scalars = w.scalars; P.inst0 = w.inst0;
     P.nbuf = w.nbuf; P.nscalars = w.nscal;
-    P.out_buf = g.out_buf; P.sumsq_slot = g.sumsq_slot;
+    P.out_buf = g.out_buf; P.sumsq_slot = w.sumsq_slot;
     P.in_prog_start = g.in_prog_start; P.in_prog_len = g.in_prog_len;
     P.epi_prog_start = g.epi_prog_start; P.epi_prog_len = g.epi_prog_len;
     P.plain_in_buf = (s.iir.plain_in || tprog) ? s.iir.plain_buf : -1;
     P.plain_in_len = s.iir.plain_len;
     P.nch = g.nchannels; P.blocks_per_row = c.blocks_per_row;
-    P.N = g.n_out; P.L = c.L; P.Wc = c.Wc;
+    P.N = w.n_out; P.L = c.L; P.Wc = c.Wc;
     P.slots_per_row = tma ? c.nchunks : (int64_t)c.blocks_per_row * kIirThreads;
     P.M = s.iir.M; P.gain = g.gain;
     const double* t = p.blob.data() + p.tables[g.coef_table].offset;
@@ -1257,7 +1281,7 @@ void plan_iir_stage(const Wave& w) {
     }
     if (getenv("SIGOPS_DEBUG"))
         fprintf(stderr, "[sigops] IIR stage %zu: %s rows=%lld N=%lld M=%d W=%lld L=%lld chunks/row=%lld Wc=%lld matrix=%d\n", w.si,
-                tma ? "tma" : (s.iir.fast ? "cp.async" : "generic"), (long long)rows, (long long)g.n_out, s.iir.M,
+                tma ? "tma" : (s.iir.fast ? "cp.async" : "generic"), (long long)rows, (long long)w.n_out, s.iir.M,
                 (long long)s.iir.W, (long long)c.L, (long long)c.nchunks, (long long)c.Wc, (int)c.need_matrix);
     const int64_t tma_blocks = ((Q.total_chunks + 31) / 32 + kTmaWarps - 1) / kTmaWarps;
     dim3 grid((unsigned)(tma ? tma_blocks : rows * c.blocks_per_row));
@@ -1302,7 +1326,7 @@ bool plan_fir_tmap(const Wave& w, const FirParams& P) {
     const sigops_stage& g = s.st;
     const int64_t rows = P.nrows;
     if (rows <= 64 || getenv("SIGOPS_NO_FIR_TMAP") || !iir_tmap_available() || rows >= (int64_t(1) << 31) ||
-        g.n_out >= (int64_t(1) << 31) || s.fir.in_len >= (int64_t(1) << 31))
+        w.n_out >= (int64_t(1) << 31) || s.fir.in_len >= (int64_t(1) << 31))
         return false;
     // a group's band starts at its first window position; the helpers build it in blocks of 8 rows
     const int ks = (int)round_up(s.fir.dpad + g.taps_per_phase, 8);
@@ -1312,7 +1336,7 @@ bool plan_fir_tmap(const Wave& w, const FirParams& P) {
     // memory then, which buys one more ring slot
     const double* bands_g = nullptr;
     int period_tiles = 0;
-    if (s.fir.period > 0 && g.sumsq_slot < 0 && !getenv("SIGOPS_NO_FIR_BANDS") &&
+    if (s.fir.period > 0 && w.sumsq_slot < 0 && !getenv("SIGOPS_NO_FIR_BANDS") &&
         (size_t)(s.fir.period / 8) * ks * 64 * (size_t)s.fir.n_epochs <= (size_t(96) << 20)) {
         bands_g = period_bands(w, ks);
         period_tiles = (int)(s.fir.period / kFmT);
@@ -1327,12 +1351,12 @@ bool plan_fir_tmap(const Wave& w, const FirParams& P) {
           strided_matrix(w.refs, w.ninst, w.nbuf, s.fir.in_buf, 8, SIGOPS_F64, &bin, &sin_) &&
           strided_matrix(w.refs, w.ninst, w.nbuf, g.out_buf, 8, SIGOPS_F64, &bout, &sout) && s.fir.in_len >= 1 &&
           tmap_encode_2d_f64(&mi, bin, s.fir.in_len, rows, sin_, kFtSlotPos, kFtRows) &&
-          tmap_encode_2d_f64(&mo, bout, g.n_out, rows, sout, 16, kFtRows / 2)))
+          tmap_encode_2d_f64(&mo, bout, w.n_out, rows, sout, 16, kFtRows / 2)))
         return false;
     FirTmParams T{};
-    T.scalars = w.scalars; T.nscalars = w.nscal; T.sumsq_slot = g.sumsq_slot; T.nch = g.nchannels;
-    T.nrows = rows; T.n_out = g.n_out; T.tapsper = g.taps_per_phase; T.ks = ks; T.nslot = nslot;
-    T.ntiles = (g.n_out + kFmT - 1) / kFmT;
+    T.scalars = w.scalars; T.nscalars = w.nscal; T.sumsq_slot = w.sumsq_slot; T.nch = g.nchannels;
+    T.nrows = rows; T.n_out = w.n_out; T.tapsper = g.taps_per_phase; T.ks = ks; T.nslot = nslot;
+    T.ntiles = (w.n_out + kFmT - 1) / kFmT;
     T.pfb = P.pfb; T.dpfb = P.dpfb; T.xi0 = P.xi0; T.poff = w.pd.poff[w.si]; T.alpha = w.pd.alpha[w.si];
     T.tab_doubles = (int)tabd;
     T.bands_g = bands_g; T.period_tiles = period_tiles;
@@ -1346,11 +1370,11 @@ bool plan_fir_tmap(const Wave& w, const FirParams& P) {
     dim3 tgrid((unsigned)nseg, (unsigned)groups);
     if (getenv("SIGOPS_DEBUG")) {
         fprintf(stderr, "[sigops] FIR stage %zu: tensor-map rows=%lld n_out=%lld taps=%d ks=%d slots=%d (window %d) grid=%lldx%lld tiles/seg=%lld smem=%zu gain=%g period=%lld outputs%s\n",
-                w.si, (long long)rows, (long long)g.n_out, T.tapsper, ks, nslot, win_slots, (long long)nseg, (long long)groups,
+                w.si, (long long)rows, (long long)w.n_out, T.tapsper, ks, nslot, win_slots, (long long)nseg, (long long)groups,
                 (long long)T.tiles_per_seg, smem, T.gain, (long long)s.fir.period, bands_g ? " (tap bands from the period tables)" : "");
         if (bands_g) fprintf(stderr, "[sigops]   %lld epochs of %lld tiles\n", (long long)s.fir.n_epochs, (long long)s.fir.epoch_tiles);
     }
-    const auto kernel = g.sumsq_slot >= 0 ? k_fir_tmap<true> : k_fir_tmap<false>;
+    const auto kernel = w.sumsq_slot >= 0 ? k_fir_tmap<true> : k_fir_tmap<false>;
     w.add(KIND_FIR, [=](cudaStream_t st) {
         launch_dyn_smem(kernel, tgrid, kFtThreads, smem, st, T, *(const CUtensorMap*)&mi, *(const CUtensorMap*)&mo);
     });
@@ -1364,14 +1388,14 @@ bool plan_fir_mma(const Wave& w, const FirParams& P) {
     const int64_t rows = P.nrows;
     FirMmaParams Q{};
     Q.bufrefs = w.d_refs; Q.scalars = w.scalars; Q.nbuf = w.nbuf; Q.nscalars = w.nscal;
-    Q.in_buf = s.fir.in_buf; Q.out_buf = g.out_buf; Q.sumsq_slot = g.sumsq_slot;
-    Q.in_len = s.fir.in_len; Q.nch = g.nchannels; Q.nrows = rows; Q.n_out = g.n_out;
+    Q.in_buf = s.fir.in_buf; Q.out_buf = g.out_buf; Q.sumsq_slot = w.sumsq_slot;
+    Q.in_len = s.fir.in_len; Q.nch = g.nchannels; Q.nrows = rows; Q.n_out = w.n_out;
     Q.tapsper = g.taps_per_phase;
     Q.ks = (int)round_up(s.fir.dpad + g.taps_per_phase, 4);
     Q.ring = s.fir.ring32;
     Q.pitch = Q.ring + ((4 - Q.ring % 16) + 16) % 16;
     Q.pfb = P.pfb; Q.dpfb = P.dpfb; Q.xi0 = P.xi0; Q.poff = w.pd.poff[w.si]; Q.alpha = w.pd.alpha[w.si];
-    Q.ntiles = (g.n_out + kFmT - 1) / kFmT;
+    Q.ntiles = (w.n_out + kFmT - 1) / kFmT;
     Q.gain = s.fir.epi_scale;
     // both polyphase banks ride along in shared memory when that leaves the ring its room
     const int64_t tabd = (int64_t)g.n_phases * g.taps_per_phase;
@@ -1392,7 +1416,7 @@ bool plan_fir_mma(const Wave& w, const FirParams& P) {
     dim3 grid((unsigned)nseg, (unsigned)groups);
     if (getenv("SIGOPS_DEBUG"))
         fprintf(stderr, "[sigops] FIR stage %zu: mma rows=%lld n_out=%lld taps=%d ks=%d ring=%d pitch=%d rows/block=%d grid=%lldx%lld tiles/seg=%lld smem=%zu\n",
-                w.si, (long long)rows, (long long)g.n_out, Q.tapsper, Q.ks, Q.ring, Q.pitch, RB, (long long)nseg,
+                w.si, (long long)rows, (long long)w.n_out, Q.tapsper, Q.ks, Q.ring, Q.pitch, RB, (long long)nseg,
                 (long long)groups, (long long)Q.tiles_per_seg, smem);
     const bool ssq = Q.sumsq_slot >= 0;
     const auto kernel = RB == 128 ? (ssq ? k_fir_mma<8, 2, true> : k_fir_mma<8, 2, false>)
@@ -1436,8 +1460,8 @@ void plan_fir_long(const Wave& w, const FirParams& P) {
     const bool tab = g.fir_kind == SIGOPS_FIR_DECIMATOR;
     FirLongParams Q{};
     Q.bufrefs = w.d_refs; Q.scalars = w.scalars; Q.nbuf = w.nbuf; Q.nscalars = w.nscal;
-    Q.in_buf = s.fir.in_buf; Q.out_buf = g.out_buf; Q.sumsq_slot = g.sumsq_slot;
-    Q.in_len = s.fir.in_len; Q.nch = g.nchannels; Q.nrows = rows; Q.n_out = g.n_out;
+    Q.in_buf = s.fir.in_buf; Q.out_buf = g.out_buf; Q.sumsq_slot = w.sumsq_slot;
+    Q.in_len = s.fir.in_len; Q.nch = g.nchannels; Q.nrows = rows; Q.n_out = w.n_out;
     Q.tapsper = g.taps_per_phase;
     // a group's band: its last output's window ends dpad positions after its first output's
     const int64_t dpad = tab ? 7 * (int64_t)g.decimation : s.fir.dpad;
@@ -1450,15 +1474,15 @@ void plan_fir_long(const Wave& w, const FirParams& P) {
     Q.gain = tab ? 1.0 : s.fir.epi_scale;
     // rows per block: four 8-row fragments per warp, one where the batch has no more than 8 rows
     const int MF = rows > 8 ? 4 : 1, RB = 8 * MF;
-    const int64_t tiles = (g.n_out + kFlT - 1) / kFlT, groups = (rows + RB - 1) / RB;
+    const int64_t tiles = (w.n_out + kFlT - 1) / kFlT, groups = (rows + RB - 1) / RB;
     if (groups > 65535) fail(SIGOPS_ERR_UNSUPPORTED, "FIR stage over more than %d rows per wave", 65535 * RB);
     const size_t smem = (size_t)RB * kFlPitch * sizeof(double);
     dim3 grid((unsigned)tiles, (unsigned)groups);
     if (getenv("SIGOPS_DEBUG"))
         fprintf(stderr, "[sigops] FIR stage %zu: long rows=%lld n_out=%lld taps=%d ks=%lld segment=%d grid=%lldx%lld rows/block=%d bank=%s smem=%zu\n",
-                w.si, (long long)rows, (long long)g.n_out, g.taps_per_phase, (long long)ks, kFlSeg, (long long)tiles,
+                w.si, (long long)rows, (long long)w.n_out, g.taps_per_phase, (long long)ks, kFlSeg, (long long)tiles,
                 (long long)groups, RB, tab ? "table" : (P.dpfb ? "merged" : "gathered"), smem);
-    const bool ssq = g.sumsq_slot >= 0;
+    const bool ssq = w.sumsq_slot >= 0;
     const int bk = tab ? BK_TAB : (P.dpfb ? BK_MERGE : BK_BANK);
     using K = void (*)(FirLongParams);
     static const K kernels[2][3][2] = {
@@ -1478,15 +1502,15 @@ void plan_fir_stage(const Wave& w) {
     const sigops_plan& p = w.p;
     const StageRT& s = p.stages[w.si];
     const sigops_stage& g = s.st;
-    if (g.n_out == 0) return;
+    if (w.n_out == 0) return;
     const int64_t rows = w.ninst * g.nchannels;
     FirParams P{};
     P.instrs = w.pd.instrs; P.bufrefs = w.d_refs; P.scalars = w.scalars; P.inst0 = w.inst0;
     P.nbuf = w.nbuf; P.nscalars = w.nscal;
-    P.out_buf = g.out_buf; P.sumsq_slot = g.sumsq_slot;
+    P.out_buf = g.out_buf; P.sumsq_slot = w.sumsq_slot;
     P.in_buf = s.fir.in_buf; P.in_len = s.fir.in_len;
     P.epi_prog_start = g.epi_prog_start; P.epi_prog_len = g.epi_prog_len;
-    P.nch = g.nchannels; P.nrows = rows; P.n_out = g.n_out;
+    P.nch = g.nchannels; P.nrows = rows; P.n_out = w.n_out;
     P.tapsper = g.taps_per_phase;
     P.pfb = w.pd.blob + p.tables[g.pfb_table].offset;
     P.dpfb = g.dpfb_table >= 0 ? w.pd.blob + p.tables[g.dpfb_table].offset : nullptr;
@@ -1505,13 +1529,13 @@ void plan_fir_stage(const Wave& w) {
     const FirGeom geo = fir_geometry(s.fir, g.taps_per_phase, G, p.max_stack);
     P.hbase = geo.hbase; P.tpad = geo.tpad; P.xpitch = geo.xpitch;
     const size_t smem = geo.smem;
-    const int64_t tiles = (g.n_out + kFirT - 1) / kFirT;
+    const int64_t tiles = (w.n_out + kFirT - 1) / kFirT;
     const int64_t groups = (rows + 32 * G - 1) / (32 * G);
     if (groups > 65535) fail(SIGOPS_ERR_UNSUPPORTED, "FIR stage over more than %d rows per wave", 65535 * 32 * G);
     dim3 grid((unsigned)tiles, (unsigned)groups);
     if (getenv("SIGOPS_DEBUG"))
         fprintf(stderr, "[sigops] FIR stage %zu: scalar rows=%lld n_out=%lld taps=%d G=%d tiles=%lld smem=%zu\n", w.si,
-                (long long)rows, (long long)g.n_out, g.taps_per_phase, G, (long long)tiles, smem);
+                (long long)rows, (long long)w.n_out, g.taps_per_phase, G, (long long)tiles, smem);
     const auto kernel = G == 4 ? k_fir<4, 8> : (G == 2 ? k_fir<2, 8> : k_fir<1, 8>);
     w.add(KIND_FIR, [=](cudaStream_t st) { launch_dyn_smem(kernel, grid, 256, smem, st, P); });
 }
@@ -1523,15 +1547,20 @@ int64_t enqueue_wave(sigops_plan& p, int di, Slot& slot, cudaStream_t stream, co
     const int nbuf = p.nbuf();
     const int64_t ninst = io.ninst;
     const int nscal = std::max<uint32_t>(p.h.n_scalars, 1);
+    const bool ragged = io.temp_frames != nullptr;
     // -- workspace carve-up
     const size_t temp_stride = temp_bytes_per_instance(p);
     char* temps = temp_stride ? (char*)slot.arena.take(temp_stride * ninst) : nullptr;
     double* scalars = (double*)slot.arena.take((size_t)ninst * nscal * sizeof(double));
-    BufRef* d_refs = (BufRef*)slot.arena.take((size_t)ninst * nbuf * sizeof(BufRef));
+    // (a ragged wave's table of valid frames, [ninst][nbuf] int64, follows the BufRef table in the same upload, so
+    // that prepared launches and graphs are replayed only for the same lengths too)
+    const size_t refs_bytes = (size_t)ninst * nbuf * sizeof(BufRef);
+    const size_t table_bytes = refs_bytes + (ragged ? (size_t)ninst * nbuf * sizeof(int64_t) : 0);
+    BufRef* d_refs = (BufRef*)slot.arena.take(table_bytes);
+    const int64_t* d_valid = (const int64_t*)((const char*)d_refs + refs_bytes);
     CUDA_OK(cudaMemsetAsync(scalars, 0, (size_t)ninst * nscal * sizeof(double), stream));
 
     // -- BufRef table (instance-major)
-    const size_t table_bytes = (size_t)ninst * nbuf * sizeof(BufRef);
     std::vector<char> table(table_bytes);
     BufRef* refs = (BufRef*)table.data();
     for (int64_t i = 0; i < ninst; ++i) {
@@ -1553,6 +1582,15 @@ int64_t enqueue_wave(sigops_plan& p, int di, Slot& slot, cudaStream_t stream, co
                 r.ptr = ob.ptr; r.ld = ob.ld; r.dtype = ob.dtype; r.nch = ob.nchannels;
             }
         }
+    }
+    if (ragged) {
+        int64_t* valid = (int64_t*)(table.data() + refs_bytes);
+        const uint32_t nin = p.h.n_inputs, ntmp = p.h.n_temps;
+        for (int64_t i = 0; i < ninst; ++i)
+            for (int b = 0; b < nbuf; ++b)
+                valid[i * nbuf + b] = b < (int)nin ? io.in[i * nin + b].nframes
+                                    : b < (int)(nin + ntmp) ? io.temp_frames[i * ntmp + (b - nin)]
+                                    : io.out[i * p.h.n_outputs + (b - nin - ntmp)].nframes;
     }
     bool table_changed = false;
     if (slot.last_table_dev != (void*)d_refs || slot.last_table != table) {
@@ -1625,13 +1663,52 @@ int64_t enqueue_wave(sigops_plan& p, int di, Slot& slot, cudaStream_t stream, co
     // (slot.last_table now holds this wave's table)
     Wave w{p, pd, dev.sm_count, (const BufRef*)slot.last_table.data(), d_refs, scalars, nbuf, nscal, ninst, io.inst0, 0,
            slot.arena, slot.cache_launches};
+    const int64_t* valid = ragged ? (const int64_t*)(slot.last_table.data() + refs_bytes) : nullptr;
+    // ragged run: frames [valid, ld) of buffer b of every instance set to zero (launch skipped when no row has a tail)
+    auto zero_tails = [&](int b) {
+        int64_t tail = 0;
+        for (int64_t i = 0; i < ninst; ++i) tail = std::max(tail, w.refs[i * nbuf + b].ld - valid[i * nbuf + b]);
+        if (tail <= 0) return;
+        RaggedParams R{d_refs, d_valid, scalars, nbuf, nscal, b, -1, ninst, 0.0};
+        const dim3 grid((unsigned)((tail + kRgSpan - 1) / kRgSpan), (unsigned)std::min<int64_t>(ninst, 65535));
+        w.add(KIND_MAP, [=](cudaStream_t st) { k_tail_zero<<<grid, kRgThreads, 0, st>>>(R); });
+    };
+    int64_t computed = 0, useful = 0;
+    if (ragged)
+        for (uint32_t b = 0; b < p.h.n_inputs; ++b) zero_tails((int)b);
     for (w.si = 0; w.si < p.stages.size(); ++w.si) {
-        switch (p.stages[w.si].st.kind) {
+        const sigops_stage& g = p.stages[w.si].st;
+        const sigops_bufdesc& ob = p.bufs[g.out_buf];
+        w.n_out = ob.nframes;
+        w.sumsq_slot = g.sumsq_slot;
+        int64_t vmax = 0;
+        if (ragged) {
+            // the prefix the wave's longest instance needs (rounded up to 16 frames within the plan's), no fused sum of
+            // squares
+            for (int64_t i = 0; i < ninst; ++i) {
+                vmax = std::max(vmax, valid[i * nbuf + g.out_buf]);
+                useful += valid[i * nbuf + g.out_buf] * ob.nchannels;
+            }
+            w.n_out = ragged_stage_frames(p, w.si, vmax);
+            w.sumsq_slot = -1;
+            computed += w.n_out * ob.nchannels * ninst;
+        }
+        switch (g.kind) {
             case SIGOPS_STAGE_MAP: plan_map_stage(w); break;
             case SIGOPS_STAGE_IIR: plan_iir_stage(w); break;
             default: plan_fir_stage(w);
         }
+        if (!ragged) continue;
+        if (g.sumsq_slot >= 0 && vmax > 0) {
+            RaggedParams R{d_refs, d_valid, scalars, nbuf, nscal, g.out_buf, g.sumsq_slot, ninst, p.slot_d0[g.sumsq_slot]};
+            const dim3 grid((unsigned)((vmax + kRgSpan - 1) / kRgSpan), (unsigned)std::min<int64_t>(ninst, 65535));
+            w.add(KIND_MAP, [=](cudaStream_t st) { k_sumsq_rows<<<grid, kRgThreads, 0, st>>>(R); });
+        }
+        if (g.out_buf < (int)(p.h.n_inputs + p.h.n_temps)) zero_tails(g.out_buf);
     }
+    if (ragged && getenv("SIGOPS_DEBUG"))
+        fprintf(stderr, "[sigops] ragged wave: instances=%lld frames computed=%lld useful=%lld (%.3f)\n", (long long)ninst,
+                (long long)computed, (long long)useful, useful ? (double)computed / useful : 0.0);
     slot.cache_plan = p.uid;
     slot.cache_ninst = ninst;
     slot.cache_inst0 = io.inst0;
@@ -1719,7 +1796,9 @@ int64_t copy_runs(const sigops_buffer* host, const sigops_buffer* dev, int64_t w
             }
             const size_t bytes = (size_t)hb.nframes * hb.nchannels * es;
             int64_t j = i + 1;
-            while (merge && j < w && (char*)host[j * nb + b].ptr == (char*)hb.ptr + (j - i) * bytes &&
+            // (the next instance must be dense too: in a ragged run it may hold fewer frames than its rows)
+            while (merge && j < w && host[j * nb + b].nframes == hb.nframes && host[j * nb + b].ld == hb.nframes &&
+                   dev[j * nb + b].ld == hb.nframes && (char*)host[j * nb + b].ptr == (char*)hb.ptr + (j - i) * bytes &&
                    (char*)dev[j * nb + b].ptr == (char*)db.ptr + (j - i) * bytes)
                 ++j;
             if (to_device) CUDA_OK(cudaMemcpyAsync(db.ptr, hb.ptr, bytes * (j - i), cudaMemcpyHostToDevice, st));
@@ -1785,8 +1864,9 @@ int copy_threads(int ndev) {
     return std::max(1, std::min(8, (hw > 0 ? hw : 8) / std::max(1, ndev)));
 }
 
+// `temp_frames`: a ragged run (sigops_plan_run_ragged), [instance][n_temps] valid frames of the temps.
 void run_host_on_device(sigops_plan& p, int di, int64_t i_begin, int64_t i_end, const sigops_buffer* in,
-                        sigops_buffer* out, HostRunResult& res) {
+                        sigops_buffer* out, HostRunResult& res, const int64_t* temp_frames = nullptr) {
     Device& dev = p.ctx->devs[di];
     try {
         CUDA_OK(cudaSetDevice(dev.ordinal));
@@ -1817,7 +1897,26 @@ void run_host_on_device(sigops_plan& p, int di, int64_t i_begin, int64_t i_end, 
         if (getenv("SIGOPS_FORCE_STAGING")) pinned_in = pinned_out = false;
         const size_t budget = p.ctx->ws_budget / kHostSlots;
         int64_t wave = ninst;
-        auto need_for = [&](int64_t w) { return wave_workspace_bytes(p, w, dev.sm_count) + io_bytes * w + (size_t)w * (nin + nout) * sizeof(sigops_buffer); };
+        auto need_for = [&](int64_t w) {
+            const size_t io = io_bytes * w + (size_t)w * (nin + nout) * sizeof(sigops_buffer);
+            if (!temp_frames) return wave_workspace_bytes(p, w, dev.sm_count) + io;
+            // ragged: the IIR chunkings follow each wave's prefixes, so take the largest wave of this size exactly
+            size_t most = 0;
+            std::vector<int64_t> n(p.stages.size());
+            for (int64_t i0 = 0; i0 < ninst; i0 += w) {
+                const int64_t wn = std::min(w, ninst - i0);
+                for (size_t si = 0; si < p.stages.size(); ++si) {
+                    const int b = p.stages[si].st.out_buf;
+                    int64_t vmax = 0;
+                    for (int64_t i = i_begin + i0; i < i_begin + i0 + wn; ++i)
+                        vmax = std::max(vmax, b < (int)(nin + p.h.n_temps) ? temp_frames[i * p.h.n_temps + (b - nin)]
+                                                                           : out[i * nout + (b - nin - p.h.n_temps)].nframes);
+                    n[si] = ragged_stage_frames(p, si, vmax);
+                }
+                most = std::max(most, wave_workspace_bytes(p, wn, dev.sm_count, n.data()));
+            }
+            return most + io;
+        };
         // several waves when the batch allows it, so that H2D of wave k+1, the kernels of wave k and D2H of wave
         // k-1 overlap (the first H2D and the last D2H are exposed: 1/nwaves of the copy time)
         int nwaves = 16;
@@ -1877,7 +1976,7 @@ void run_host_on_device(sigops_plan& p, int di, int64_t i_begin, int64_t i_end, 
                     sigops_buffer& db = dbufs[i * nb + b];
                     db = ub;
                     db.dtype = bd.dtype;
-                    db.ld = round_up(std::max<int64_t>(ub.nframes, 1), 16);
+                    db.ld = round_up(std::max<int64_t>(bd.nframes, 1), 16);     // (a ragged instance's rows are the plan's length)
                     db.ptr = slot.arena.take_packed((size_t)db.ld * ub.nchannels * elem_size(bd.dtype));
                     cu[i * nb + b] = ub;
                     cd[i * nb + b] = db;
@@ -1948,7 +2047,7 @@ void run_host_on_device(sigops_plan& p, int di, int64_t i_begin, int64_t i_end, 
             // ---- stages on the slot's stream (WAV-layout inputs are transposed / decoded first, outputs encoded last)
             CUDA_OK(cudaStreamWaitEvent(slot.stream, dev.ev_in[s], 0));
             for (auto& j : wav_in) launch_wav(false, j.P, slot.stream);
-            WaveIO io{w, din.data(), dout.data(), i_begin + i0};
+            WaveIO io{w, din.data(), dout.data(), i_begin + i0, temp_frames ? temp_frames + (i_begin + i0) * p.h.n_temps : nullptr};
             res.launches += enqueue_wave(p, di, slot, slot.stream, io) + (int64_t)wav_in.size() + (int64_t)wav_out.size();
             for (auto& j : wav_out) launch_wav(true, j.P, slot.stream);
             CUDA_OK(cudaGetLastError());
@@ -1985,6 +2084,38 @@ void run_host_on_device(sigops_plan& p, int di, int64_t i_begin, int64_t i_end, 
         for (int s = 0; s < kHostSlots; ++s) cudaStreamSynchronize(dev.slots[s].stream);
         cudaStreamSynchronize(dev.s_in);
         cudaStreamSynchronize(dev.s_out);
+    }
+}
+
+// Host-buffer run over the context's devices, one thread each: device d takes instances [bounds[d], bounds[d+1]).
+void run_host_sharded(sigops_plan& p, const std::vector<int64_t>& bounds, const sigops_buffer* in, sigops_buffer* out,
+                      const int64_t* temp_frames, int64_t out_samples, sigops_stats* stats) {
+    std::unique_lock<std::mutex> lk(p.ctx->mu);
+    auto t0 = std::chrono::steady_clock::now();
+    const int nd = (int)p.ctx->devs.size();
+    std::vector<HostRunResult> res(nd);
+    std::vector<std::thread> th;
+    for (int d = 0; d < nd; ++d) {
+        const int64_t b = bounds[d], e = bounds[d + 1];
+        if (nd == 1) run_host_on_device(p, d, b, e, in, out, res[d], temp_frames);
+        else th.emplace_back([&, d, b, e] { run_host_on_device(p, d, b, e, in, out, res[d], temp_frames); });
+    }
+    for (auto& t : th) t.join();
+    lk.unlock();
+    for (auto& r : res)
+        if (r.code) throw Failure{r.code, r.msg};
+    if (stats) {
+        memset(stats, 0, sizeof *stats);
+        for (auto& r : res) {
+            stats->gpu_ms = std::max(stats->gpu_ms, r.gpu_ms);
+            stats->h2d_ms = std::max(stats->h2d_ms, r.h2d_ms);
+            stats->d2h_ms = std::max(stats->d2h_ms, r.d2h_ms);
+            stats->launches += r.launches;
+            stats->h2d_bytes += r.h2d;
+            stats->d2h_bytes += r.d2h;
+        }
+        stats->out_samples = out_samples;
+        stats->wall_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
     }
 }
 
@@ -2195,33 +2326,67 @@ int sigops_plan_run(sigops_plan* plan, int64_t ninst, const sigops_buffer* in, s
     return guarded(plan->ctx, [&] {
         sigops_ctx* ctx = plan->ctx;
         validate_io(*plan, ninst, in, out, true);
-        std::unique_lock<std::mutex> lk(ctx->mu);
-        auto t0 = std::chrono::steady_clock::now();
         const int nd = (int)ctx->devs.size();
-        std::vector<HostRunResult> res(nd);
-        std::vector<std::thread> th;
-        for (int d = 0; d < nd; ++d) {
-            const int64_t b = ninst * d / nd, e = ninst * (d + 1) / nd;
-            if (nd == 1) run_host_on_device(*plan, d, b, e, in, out, res[d]);
-            else th.emplace_back([&, d, b, e] { run_host_on_device(*plan, d, b, e, in, out, res[d]); });
-        }
-        for (auto& t : th) t.join();
-        lk.unlock();
-        for (auto& r : res)
-            if (r.code) throw Failure{r.code, r.msg};
-        if (stats) {
-            memset(stats, 0, sizeof *stats);
-            for (auto& r : res) {
-                stats->gpu_ms = std::max(stats->gpu_ms, r.gpu_ms);
-                stats->h2d_ms = std::max(stats->h2d_ms, r.h2d_ms);
-                stats->d2h_ms = std::max(stats->d2h_ms, r.d2h_ms);
-                stats->launches += r.launches;
-                stats->h2d_bytes += r.h2d;
-                stats->d2h_bytes += r.d2h;
+        std::vector<int64_t> bounds(nd + 1);
+        for (int d = 0; d <= nd; ++d) bounds[d] = ninst * d / nd;
+        run_host_sharded(*plan, bounds, in, out, nullptr, count_out_samples(*plan, ninst), stats);
+    });
+}
+
+int sigops_plan_run_ragged(sigops_plan* plan, int64_t ninst, const sigops_buffer* in, sigops_buffer* out,
+                           const int64_t* temp_frames, sigops_stats* stats) {
+    if (!plan) return SIGOPS_ERR_INVALID;
+    return guarded(plan->ctx, [&] {
+        sigops_ctx* ctx = plan->ctx;
+        const sigops_plan& p = *plan;
+        const uint32_t nin = p.h.n_inputs, ntmp = p.h.n_temps, nout = p.h.n_outputs;
+        if (ninst < 0) fail(SIGOPS_ERR_INVALID, "negative instance count");
+        if (ninst > 0 && ((nin && !in) || !out || (ntmp && !temp_frames))) fail(SIGOPS_ERR_INVALID, "null buffer array");
+        for (int64_t i = 0; i < ninst; ++i) {
+            for (uint32_t b = 0; b < nin + nout; ++b) {
+                const bool isin = b < nin;
+                const sigops_buffer& ub = isin ? in[i * nin + b] : out[i * nout + (b - nin)];
+                const sigops_bufdesc& bd = isin ? p.bufs[b] : p.bufs[ntmp + b];
+                if (ub.nframes < 0 || ub.nframes > bd.nframes || ub.nchannels != bd.nchannels || ub.dtype != bd.dtype)
+                    fail(SIGOPS_ERR_INVALID, "instance %lld %s %u: buffer is %lldx%d type %d, plan expects at most %lldx%d type %d "
+                         "(ragged runs take no WAV-layout buffers)", (long long)i, isin ? "input" : "output", isin ? b : b - nin,
+                         (long long)ub.nframes, ub.nchannels, ub.dtype, (long long)bd.nframes, bd.nchannels, bd.dtype);
+                if (ub.ld < ub.nframes) fail(SIGOPS_ERR_INVALID, "instance %lld: ld %lld < nframes %lld", (long long)i, (long long)ub.ld, (long long)ub.nframes);
+                if (!ub.ptr && ub.nframes > 0) fail(SIGOPS_ERR_INVALID, "instance %lld: null buffer pointer", (long long)i);
             }
-            stats->out_samples = count_out_samples(*plan, ninst);
-            stats->wall_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+            for (uint32_t t = 0; t < ntmp; ++t)
+                if (temp_frames[i * ntmp + t] < 0 || temp_frames[i * ntmp + t] > p.bufs[nin + t].nframes)
+                    fail(SIGOPS_ERR_INVALID, "instance %lld temp %u: %lld valid frames of %lld", (long long)i, t,
+                         (long long)temp_frames[i * ntmp + t], (long long)p.bufs[nin + t].nframes);
         }
+        for (const StageRT& s : p.stages)
+            if (s.st.sumsq_slot >= 0 && std::isnan(p.slot_d0[s.st.sumsq_slot]))
+                fail(SIGOPS_ERR_UNSUPPORTED, "scalar slot %d is read by RMS leaves with different divisors", s.st.sumsq_slot);
+        // Longest first, so that every wave computes about the frames its instances need; a plan with device noise
+        // keeps the caller's order (an instance's noise stream is its index in the call).
+        std::vector<int64_t> order(ninst);
+        for (int64_t i = 0; i < ninst; ++i) order[i] = i;
+        if (!p.has_randn)
+            std::stable_sort(order.begin(), order.end(), [&](int64_t a, int64_t b) { return out[a * nout].nframes > out[b * nout].nframes; });
+        std::vector<sigops_buffer> pin((size_t)ninst * nin), pout((size_t)ninst * nout);
+        std::vector<int64_t> ptmp(std::max<size_t>(1, (size_t)ninst * ntmp)), cum(ninst + 1, 0);   // (never empty: non-null marks the run ragged)
+        for (int64_t k = 0; k < ninst; ++k) {
+            const int64_t i = order[k];
+            std::copy(in + i * nin, in + (i + 1) * nin, pin.begin() + k * nin);
+            std::copy(out + i * nout, out + (i + 1) * nout, pout.begin() + k * nout);
+            std::copy(temp_frames + i * ntmp, temp_frames + (i + 1) * ntmp, ptmp.begin() + k * ntmp);
+            cum[k + 1] = cum[k];
+            for (uint32_t b = 0; b < nout; ++b) cum[k + 1] += out[i * nout + b].nframes * out[i * nout + b].nchannels;
+        }
+        // devices take contiguous ranges of about equal output samples
+        const int nd = (int)ctx->devs.size();
+        std::vector<int64_t> bounds(nd + 1, 0);
+        for (int d = 0; d < nd; ++d) {
+            int64_t e = bounds[d];
+            while (e < ninst && (d == nd - 1 || cum[e + 1] * nd <= cum[ninst] * (d + 1))) ++e;
+            bounds[d + 1] = e;
+        }
+        run_host_sharded(*plan, bounds, pin.data(), pout.data(), ptmp.data(), cum[ninst], stats);
     });
 }
 

@@ -17,7 +17,7 @@ SYMBOLS = ["sigops_abi_version", "sigops_device_count", "sigops_ctx_create", "si
            "sigops_last_error", "sigops_plan_create", "sigops_plan_destroy", "sigops_plan_run",
            "sigops_plan_run_device", "sigops_plan_launch_count", "sigops_plan_algorithmic_bytes",
            "sigops_measure_peaks", "sigops_ctx_set_profiling", "sigops_profile_collect",
-           "sigops_host_alloc", "sigops_host_free"]
+           "sigops_host_alloc", "sigops_host_free", "sigops_plan_run_ragged"]
 KERNEL_KINDS = ["map", "iir_main", "iir_carry", "iir_fix", "fir"]
 
 
@@ -67,6 +67,7 @@ def load():
     lib.sigops_plan_destroy.argtypes = [vp]
     lib.sigops_plan_destroy.restype = None
     lib.sigops_plan_run.argtypes = [vp, i64, C.POINTER(Buffer), C.POINTER(Buffer), C.POINTER(Stats)]
+    lib.sigops_plan_run_ragged.argtypes = [vp, i64, C.POINTER(Buffer), C.POINTER(Buffer), C.POINTER(i64), C.POINTER(Stats)]
     lib.sigops_plan_run_device.argtypes = [vp, C.c_int, i64, C.POINTER(Buffer), C.POINTER(Buffer),
                                            vp, C.POINTER(Stats)]
     lib.sigops_plan_launch_count.argtypes = [vp, C.POINTER(i64)]
@@ -242,6 +243,17 @@ class CompiledPlan:
         outs = self.host_buffers(out_arrays)
         st = Stats()
         _check(self.lib, self.ctx.handle, self.lib.sigops_plan_run(self.handle, ninst, ins, outs, C.byref(st)))
+        return st.asdict()
+
+    def run_ragged(self, ninst, in_arrays, out_arrays, temp_frames):
+        """Instances of different lengths (include/signalops.h `sigops_plan_run_ragged`): each array holds the
+        instance's own frames; `temp_frames` [ninst][n_temps] the valid frames of the plan's temps."""
+        ins = self.host_buffers(in_arrays)
+        outs = self.host_buffers(out_arrays)
+        tf = np.ascontiguousarray(temp_frames, dtype=np.int64)
+        st = Stats()
+        _check(self.lib, self.ctx.handle, self.lib.sigops_plan_run_ragged(
+            self.handle, ninst, ins, outs, tf.ctypes.data_as(C.POINTER(C.c_int64)), C.byref(st)))
         return st.asdict()
 
     def run_device(self, ninst, in_bufs, out_bufs, stream=None, dev_index=0, want_stats=False):

@@ -14,7 +14,7 @@ import hashlib
 import numpy as np
 
 from . import cabi, graph as G
-from .lowering import Lowerer, np_dtype
+from .lowering import Lowerer, np_dtype, ragged_plan
 from .wav import WavRaw, write_wav
 from .lowering import dtype_code as dtype_code_of
 
@@ -219,20 +219,20 @@ def _build_prefix(lw, x, n, dtype):
 def sink_batch(xs, to):
     """Materialise many structurally identical graphs in one call.  Every graph is
     lowered; the plans must agree byte for byte (same operators, lengths and
-    constants) and differ only in the arrays they read."""
+    constants) and differ only in the arrays they read — or differ in lengths alone
+    (a ragged batch: `_sink_ragged`)."""
     if not xs:
         return []
     lws = [Lowerer(instance_index=k) for k in range(len(xs))]
     plans = [lw.build(x) for lw, x in zip(lws, xs)]
     ref = plans[0].tobytes()
-    if any(lw.traced_generators for lw in lws) and any(p.tobytes() != ref for p in plans[1:]):
+    if any(lw.traced_generators for lw in lws) and any(_unlike(p, plans[0]) for p in plans[1:]):
         # closure generators whose traced programs differ between elements (other ω, ϕ or constants): evaluated on
         # the host, their frames are input buffers and the plans agree again
         plans = [Lowerer(instance_index=k, generators="host").build(x) for k, x in enumerate(xs)]
         ref = plans[0].tobytes()
-    for k, p in enumerate(plans[1:], 1):
-        if p.tobytes() != ref:
-            raise G.SignalError(f"batch element {k} does not lower to the same plan as element 0")
+    if any(p.tobytes() != ref for p in plans[1:]):
+        return _sink_ragged(plans, to)
     out = plans[0].outputs[0]
     datas = [to.alloc_result((out.nframes, out.nchannels), np_dtype(out.dtype)) for _ in xs]
     if out.nframes > 0:
@@ -240,3 +240,39 @@ def sink_batch(xs, to):
         ins = [_colmajor(a) for p in plans for a in p.input_arrays]
         to.last_stats = cp.run_host(len(xs), ins, datas)
     return [_wrap(plans[0], d, to) for d in datas]
+
+
+def _unlike(p, ref):
+    """Do two plans differ in more than their lengths?"""
+    try:
+        ragged_plan([ref, p])
+        return False
+    except G.SignalError:
+        return True
+
+
+def _sink_ragged(plans, to):
+    """Elements whose plans differ in lengths alone (include/signalops.h `sigops_plan_run_ragged`): one plan, the
+    field-wise maximum of theirs, runs every element at its own lengths; each result has its own frame count.
+    Elements of no frames take no part in the comparison (their plans have no pieces): they run as instances whose
+    buffers are all empty, which keeps every other element's index in the call (its noise stream)."""
+    live = [k for k, p in enumerate(plans) if p.outputs[0].nframes > 0]
+    if not live:
+        return [_wrap(p, to.alloc_result((0, p.outputs[0].nchannels), np_dtype(p.outputs[0].dtype)), to) for p in plans]
+    mplan, tf = ragged_plan([plans[k] for k in live])
+    if any(isinstance(a, WavRaw) for p in plans for a in p.input_arrays):
+        raise G.SignalError("a batch of signals of different lengths cannot read WAV-layout buffers (WAV files, C-ordered "
+                            "matrices): give the elements one length, or pass column-major arrays")
+    temp_frames = np.zeros((len(plans), len(mplan.temps)), dtype=np.int64)
+    temp_frames[live] = tf
+    ins, datas = [], []
+    for k, p in enumerate(plans):
+        if k in live:
+            ins += [_colmajor(a) for a in p.input_arrays]
+        else:
+            ins += [np.empty((0, b.nchannels), dtype=np_dtype(b.dtype), order="F") for b in mplan.inputs]
+        o = mplan.outputs[0]
+        datas.append(to.alloc_result((p.outputs[0].nframes, o.nchannels), np_dtype(o.dtype)))
+    cp = to.compiled(mplan.tobytes())
+    to.last_stats = cp.run_ragged(len(plans), ins, datas, temp_frames)
+    return [_wrap(p, d, to) for p, d in zip(plans, datas)]

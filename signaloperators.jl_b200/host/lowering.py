@@ -1115,3 +1115,157 @@ def host_function_frames(x, k_lo, k_hi):
 
 def lower(x, **kw):
     return Lowerer().build(x, **kw)
+
+
+# ---- ragged batches -------------------------------------------------------------------------
+# Elements of a batch whose plans differ only in lengths run as instances of one plan: the field-wise maximum of
+# theirs (include/signalops.h `sigops_plan_run_ragged`).  Every stage is prefix-stable, so that is exact when each
+# instance reads zero past its own frames, sums its own frames for a Normpower and keeps its own frames of the
+# result: the runtime sees to all three.  The pieces of a MAP stage are taken from the element that computes the most
+# frames; another element's pieces must compute the same values as those over its own frames, where a zero it reads
+# as a constant (a zero pad: `Pad(x, 0)`, a shorter signal in a `Mix`) may stand for a zero-padded buffer read past
+# the element's frames.  What this cannot express is a length that moves a position rather than an end: a fade-out's
+# start, the start of an appended piece, or a non-zero pad a shorter instance reaches.
+
+_PAD_NAMES = {PAD_CYCLE: "Pad(x, cycle)", PAD_MIRROR: "Pad(x, mirror)", PAD_LAST: "Pad(x, lastframe)"}
+
+
+def _length_masked(I):
+    if I.leaf in (LEAF_BUF, LEAF_CHANSUM, LEAF_STAGE):         # (a fused epilogue's stage leaf keeps the load's i1, unread)
+        return replace(I, i1=0)
+    if I.leaf == LEAF_RMS:
+        return replace(I, d0=0.0)
+    return I
+
+
+def _describe(plan):
+    """Everything of a plan but its lengths and its MAP pieces (tables included)."""
+    return ([(b.nchannels, b.dtype) for b in plan.inputs + plan.temps + plan.outputs], plan.n_scalars,
+            [t.shape for t in plan.tables],
+            [(st.kind, st.out_buf, st.sumsq_slot, st.nchannels, st.n_sections, st.coef_table, st.gain, st.fir_kind,
+              st.n_phases, st.taps_per_phase, st.pfb_table, st.dpfb_table, st.interpolation, st.decimation,
+              st.input_deficit, st.rate, st.phase0, len(st.in_prog), len(st.epi_prog)) for st in plan.stages])
+
+
+def _zero_pad_read(J):
+    return J.leaf in (LEAF_BUF, LEAF_CHANSUM) and (J.flags >> 1) & 3 == PAD_CONST and J.d0 == 0.0
+
+
+class _Unlike(Exception):
+    pass
+
+
+def _match(prog, ref, a, b, k, plan, reads):
+    """Does program `prog` of element `k` compute, over frames [a, b), what `ref` of the ragged plan computes for
+    that element?  Records in `reads` (keyed by instruction position) the leaves whose lengths go into the plan."""
+    if len(prog) != len(ref):
+        raise _Unlike
+    for q, (I, J) in enumerate(zip(prog, ref)):
+        if I.leaf == J.leaf == LEAF_RAMP_OFF and I.i1 != J.i1:
+            raise G.SignalError(f"batch element {k}: a ramp ends at the element's length (Ramp, RampOff or FadeTo over a "
+                                "signal of ragged length); such a batch needs one length")
+        if _length_masked(I) == _length_masked(J):
+            if I.leaf in (LEAF_BUF, LEAF_CHANSUM, LEAF_STAGE, LEAF_RMS):
+                reads.setdefault(q, []).append((k, I, a, b))
+            continue
+        if I.leaf == LEAF_CONST and I.op == J.op and _zero_pad_read(J):
+            if I.d0 != 0.0:
+                raise G.SignalError(f"batch element {k}: a pad with the constant {I.d0:g} (Pad(x, one), or Amplify / * of "
+                                    "signals of different lengths) extends a signal of ragged length; such a batch needs "
+                                    "one length")
+            if a + J.i0 >= _bufdesc(plan, J.buf).nframes:
+                continue                        # the buffer reads zero there for this element (its tail, then the pad)
+        raise _Unlike
+
+
+def ragged_plan(plans):
+    """The plan that runs `plans` (all lowered from one graph shape, lengths aside) as one ragged batch, and the
+    valid frames of every temp per element ([element][temp]).  Raises SignalError naming what stops it."""
+    ref_k = max(range(len(plans)), key=lambda k: ([st.n_out for st in plans[k].stages],
+                                                   sum(b.nframes for b in plans[k].inputs)))
+    ref = plans[ref_k]
+    for k, p in enumerate(plans):
+        if _describe(p) != _describe(ref) or not all(np.array_equal(a, b) for a, b in zip(p.tables, ref.tables)):
+            raise G.SignalError(f"batch element {k} does not lower to the same plan as element {ref_k}")
+    mx = lambda get: max(get(p) for p in plans)                                   # noqa: E731
+    out = Plan()
+    out.__dict__.update({k: v for k, v in ref.__dict__.items()})
+    out.inputs, out.temps, out.outputs = ([BufDesc(mx(lambda p, a=a, i=i: getattr(p, a)[i].nframes), b.nchannels, b.dtype)
+                                           for i, b in enumerate(getattr(ref, a))] for a in ("inputs", "temps", "outputs"))
+    out.stages = []
+    for si, st in enumerate(ref.stages):
+        s2 = replace(st, n_in=mx(lambda p: p.stages[si].n_in), n_out=mx(lambda p: p.stages[si].n_out))
+        end = _bufdesc(ref, st.out_buf).nframes
+        # the pieces of the element with the most frames; the one ending with its output takes every element's end
+        s2.pieces = [Piece(pc.lo, s2.n_out if pc.hi == end else pc.hi, pc.clo, pc.chi, pc.prog) for pc in st.pieces]
+        progs = [(s2.in_prog, "in_prog", lambda p: p.n_in), (s2.epi_prog, "epi_prog", lambda p: p.n_out)]
+        progs = [(pc.prog, None, pc) for pc in s2.pieces] + progs
+        new = []
+        for prog0, attr, ext in progs:
+            reads = {}
+            for k, p in enumerate(plans):
+                pk = p.stages[si]
+                try:
+                    if attr is not None:
+                        _match(getattr(pk, attr), prog0, 0, ext(pk), k, p, reads)
+                        continue
+                    for pc in pk.pieces:
+                        a, b = max(pc.lo, ext.lo), min(pc.hi, ext.hi)
+                        if a < b and max(pc.clo, ext.clo) < min(pc.chi, ext.chi):
+                            _match(pc.prog, prog0, a, b, k, p, reads)
+                except _Unlike:
+                    if attr is None and [pc.lo for pc in pk.pieces] != [pc.lo for pc in st.pieces]:
+                        raise G.SignalError(
+                            f"batch element {k}: a part of the signal starts at a frame that depends on the element's "
+                            "length (Append after a signal of ragged length); such a batch needs one length") from None
+                    raise G.SignalError(f"batch element {k} does not lower to the same plan as element {ref_k}") from None
+            new.append(_max_prog(prog0, reads, plans))
+        if st.kind == STAGE_MAP:
+            for k, p in enumerate(plans):                       # every element's frames lie in the plan's pieces
+                for pc in p.stages[si].pieces:
+                    cover = sum(max(0, min(pc.hi, q.hi) - max(pc.lo, q.lo)) * max(0, min(pc.chi, q.chi) - max(pc.clo, q.clo))
+                                for q in s2.pieces)
+                    if cover != (pc.hi - pc.lo) * (pc.chi - pc.clo):
+                        raise G.SignalError(
+                            f"batch element {k}: a part of the signal starts at a frame that depends on the element's "
+                            "length (Append after a signal of ragged length); such a batch needs one length")
+        for pc, prog in zip(s2.pieces, new):
+            pc.prog = prog
+        s2.in_prog, s2.epi_prog = new[-2], new[-1]
+        out.stages.append(s2)
+    temp_frames = np.array([[t.nframes for t in p.temps] for p in plans], dtype=np.int64).reshape(len(plans), -1)
+    return out, temp_frames
+
+
+def _bufdesc(plan, tag):
+    kind, k = tag
+    return {"in": plan.inputs, "tmp": plan.temps, "out": plan.outputs}[kind][k]
+
+
+def _max_prog(prog, reads, plans):
+    """`prog` with the largest valid length (and RMS divisor) any element gives each of its leaves.  A buffer leaf
+    whose valid length varies reads zero past it for the longest element: fine for a zero pad that starts where the
+    element's buffer ends, wrong for any other pad an element reaches."""
+    out = list(prog)
+    for q, rs in reads.items():
+        I0 = prog[q]
+        if I0.leaf == LEAF_RMS:
+            out[q] = replace(I0, d0=max(I.d0 for _, I, _, _ in rs))
+            continue
+        top = max(I.i1 for _, I, _, _ in rs)
+        out[q] = replace(I0, i1=top)
+        if I0.leaf == LEAF_STAGE:
+            continue
+        for k, I, a, b in rs:
+            if I.i1 == top or b + I.i0 <= I.i1:
+                continue                                     # pads as in the plan, or never reads past its valid frames
+            pad = (I.flags >> 1) & 3
+            if pad != PAD_CONST or I.d0 != 0.0:
+                name = _PAD_NAMES.get(pad, f"a pad with the constant {I.d0:g} (Pad(x, one), or Amplify / * of "
+                                            "signals of different lengths)")
+                raise G.SignalError(f"batch element {k}: {name} extends a signal of ragged length; such a batch "
+                                    "needs one length")
+            if I.i1 < _bufdesc(plans[k], I.buf).nframes:
+                raise G.SignalError(f"batch element {k}: reads a buffer past a valid length shorter than the "
+                                    "buffer; such a batch needs one length")
+    return out

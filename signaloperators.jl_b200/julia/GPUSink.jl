@@ -142,11 +142,213 @@ function SignalOperators.sink(xs::AbstractVector, to::GPUSink)
     plans = [lower(x; instance_index = i - 1) for (i, x) in enumerate(xs)]
     # closure generators whose traced programs differ between elements (other ω, ϕ or constants): on the CPU sink,
     # their frames are input buffers and the plans agree again
-    all(p -> p.bytes == plans[1].bytes, plans) || (plans = [lower(x; instance_index = i - 1, generators = :host) for (i, x) in enumerate(xs)])
-    all(p -> p.bytes == plans[1].bytes, plans) || error("batch elements do not lower to the same plan")
+    unlike(p) = try ragged_plan([plans[1].bytes, p.bytes]); false catch e; e isa ErrorException || rethrow(); true end
+    any(unlike, plans) && (plans = [lower(x; instance_index = i - 1, generators = :host) for (i, x) in enumerate(xs)])
     results = [pinned_matrix(to, p.outtype, nframes(x), nchannels(x)) for (x, p) in zip(xs, plans)]
-    (isempty(xs) || nframes(xs[1]) == 0) || run!(to, plans, results)
+    if all(p -> p.bytes == plans[1].bytes, plans)
+        (isempty(xs) || nframes(xs[1]) == 0) || run!(to, plans, results)
+    else
+        run_ragged!(to, xs, plans, results)
+    end
     [wrapresult(x, refineroot(root(x)), r) for (x, r) in zip(xs, results)]
+end
+
+# ---- ragged batches (include/signalops.h `sigops_plan_run_ragged`; host/lowering.py `ragged_plan`) ---------------------
+# Elements whose plans differ in lengths alone run as instances of the field-wise maximum of their plans.  Elements of
+# no frames take no part in the comparison: they run as instances whose buffers are all empty (their index in the call,
+# which is their noise stream, is kept).  The comparison works on the plan bytes: the length fields are bufdesc
+# nframes, stage n_in / n_out, piece out_len, i1 of BUF / CHANSUM / STAGE leaves and d0 of RMS leaves.
+function run_ragged!(to::GPUSink, xs, plans, results)
+    live = [k for k in eachindex(xs) if nframes(xs[k]) > 0]
+    isempty(live) && return nothing
+    mbytes, tf = ragged_plan([plans[k].bytes for k in live])
+    L = plan_layout(mbytes)
+    temp_frames = zeros(Int64, L.ntmp, length(xs))                  # column k: element k's temps (instance-major bytes)
+    temp_frames[:, live] = tf
+    ins = SigopsBuffer[]
+    for (k, p) in enumerate(plans)
+        if k in live
+            append!(ins, [buffer(a) for a in p.inputs])
+        else
+            for b in 0:L.nin-1
+                push!(ins, SigopsBuffer(C_NULL, 0, rd(Int32, mbytes, L.o_buf + 16b + 8), rd(Int32, mbytes, L.o_buf + 16b + 12), 0))
+            end
+        end
+    end
+    outs = [buffer(r) for r in results]
+    handle = compiled(to, mbytes)
+    stats = SigopsStats()
+    GC.@preserve plans results temp_frames begin
+        check(to, ccall((:sigops_plan_run_ragged, libsignalops), Cint,
+                        (Ptr{Cvoid}, Int64, Ptr{SigopsBuffer}, Ptr{SigopsBuffer}, Ptr{Int64}, Ref{SigopsStats}),
+                        handle, length(results), ins, outs, temp_frames, stats))
+    end
+    stats
+end
+
+rd(::Type{T}, b, o) where T = ltoh(reinterpret(T, b[o+1:o+sizeof(T)])[1])
+wr!(b, o, v) = (b[o+1:o+sizeof(v)] .= reinterpret(UInt8, [htol(v)]); b)
+
+function plan_layout(b)
+    h = [Int(rd(UInt32, b, 4k)) for k in 0:9]
+    nin, ntmp, nout, ntab, nins, npc, nst = h[3], h[4], h[5], h[7], h[8], h[9], h[10]
+    o_buf = 48
+    o_ins = o_buf + 16 * (nin + ntmp + nout) + 16 * ntab
+    o_pc = o_ins + 80 * nins
+    o_st = o_pc + 32 * npc
+    (; nin, ntmp, nb = nin + ntmp + nout, nins, npc, nst, o_buf, o_ins, o_pc, o_st)
+end
+
+# Stage fields: kind 0, out_buf 4, piece_start 12, n_pieces 16, in_prog 20/24, epi_prog 28/32, n_in 40, n_out 48.
+# Piece: out_start 0, out_len 8, ch_start 16, ch_count 20, prog 24/28.  Instr: op 0, leaf 1, flags 3, buf 4, i0 16, i1 24, d0 40.
+stage(b, L, s) = L.o_st + 128s
+piece(b, L, p) = L.o_pc + 32p
+instr(b, L, i) = L.o_ins + 80i
+hasleaf(op) = OP_LOAD <= op <= OP_DIV || op == OP_FN2
+bufframes(b, L, id) = rd(Int64, b, L.o_buf + 16id)
+
+# everything of a plan but its lengths and its MAP pieces: buffer shapes, tables, the stages without their lengths and
+# instruction / piece positions
+function describe(b, L)
+    h = [rd(UInt32, b, 4k) for k in (0, 1, 2, 3, 4, 5, 6, 9)]
+    bufs = [b[L.o_buf+16k+9:L.o_buf+16k+16] for k in 0:L.nb-1]
+    tabs = b[L.o_buf+16L.nb+1:L.o_ins]
+    blob = b[L.o_st+128L.nst+1:end]
+    sts = map(0:L.nst-1) do s
+        c = b[stage(b, L, s)+1:stage(b, L, s)+128]
+        for (o, T) in ((12, Int32), (16, Int32), (20, Int32), (28, Int32), (40, Int64), (48, Int64)); wr!(c, o, zero(T)); end
+        c
+    end
+    (h, bufs, tabs, blob, sts)
+end
+
+masked(b, o) = (c = b[o+1:o+80]; leaf = c[2];
+                hasleaf(c[1]) && leaf in (LEAF_BUF, LEAF_CHANSUM, LEAF_STAGE) && wr!(c, 24, Int64(0));
+                hasleaf(c[1]) && leaf == LEAF_RMS && wr!(c, 40, 0.0); c)
+zero_pad_read(b, o) = b[o+2] in (LEAF_BUF, LEAF_CHANSUM) && (b[o+4] >> 1) & 3 == PAD_CONST && rd(Float64, b, o + 40) == 0.0
+
+struct Unlike <: Exception end
+
+# Does the program of element k at instructions [pk, pk+n) compute, over frames [a, b), what the reference's program
+# at [pr, pr+n) computes for that element?  Records the leaves whose lengths go into the plan in `reads`.
+function match!(reads, bk, Lk, pk, br, Lr, pr, n, a, bb, k)
+    for q in 0:n-1
+        I, J = instr(bk, Lk, pk + q), instr(br, Lr, pr + q)
+        bk[I+2] == br[J+2] == LEAF_RAMP_OFF && rd(Int64, bk, I + 24) != rd(Int64, br, J + 24) &&
+            error("batch element $(k-1): a ramp ends at the element's length (Ramp, RampOff or FadeTo over a signal of " *
+                  "ragged length); such a batch needs one length")
+        if masked(bk, I) == masked(br, J)
+            hasleaf(bk[I+1]) && bk[I+2] in (LEAF_BUF, LEAF_CHANSUM, LEAF_STAGE, LEAF_RMS) && push!(get!(reads, q, []), (k, I, a, bb))
+            continue
+        end
+        if hasleaf(bk[I+1]) && bk[I+2] == LEAF_CONST && bk[I+1] == br[J+1] && zero_pad_read(br, J)
+            d0 = rd(Float64, bk, I + 40)
+            d0 != 0.0 && error("batch element $(k-1): a pad with the constant $d0 (Pad(x, one), or Amplify / * of signals " *
+                               "of different lengths) extends a signal of ragged length; such a batch needs one length")
+            a + rd(Int64, br, J + 16) >= bufframes(bk, Lk, rd(Int32, br, J + 4)) && continue
+        end
+        throw(Unlike())
+    end
+end
+
+function ragged_plan(bs)
+    Ls = [plan_layout(b) for b in bs]
+    key(k) = ([rd(Int64, bs[k], stage(bs[k], Ls[k], s) + 48) for s in 0:Ls[k].nst-1],
+              sum(bufframes(bs[k], Ls[k], i) for i in 0:Ls[k].nin-1; init = 0))
+    r = argmax(key, eachindex(bs))
+    ref, L = bs[r], Ls[r]
+    for k in eachindex(bs)
+        (Ls[k].nb == L.nb && Ls[k].nst == L.nst && describe(bs[k], Ls[k]) == describe(ref, L)) ||
+            error("batch element $(k-1) does not lower to the same plan as element $(r-1)")
+    end
+    out = copy(ref)
+    for i in 0:L.nb-1; wr!(out, L.o_buf + 16i, maximum(bufframes(b, Lk, i) for (b, Lk) in zip(bs, Ls))); end
+    for s in 0:L.nst-1
+        so = stage(ref, L, s)
+        nmax = maximum(rd(Int64, b, stage(b, Lk, s) + 48) for (b, Lk) in zip(bs, Ls))
+        wr!(out, so + 40, maximum(rd(Int64, b, stage(b, Lk, s) + 40) for (b, Lk) in zip(bs, Ls)))
+        wr!(out, so + 48, nmax)
+        finish = bufframes(ref, L, rd(Int32, ref, so + 4))
+        ps, np = rd(Int32, ref, so + 12), rd(Int32, ref, so + 16)
+        ext = map(ps:ps+np-1) do p                                   # (lo, hi, clo, chi, prog start, len) of the plan's pieces
+            o = piece(ref, L, p)
+            lo, hi = rd(Int64, ref, o), rd(Int64, ref, o) + rd(Int64, ref, o + 8)
+            hi == finish && (hi = nmax; wr!(out, o + 8, nmax - lo))   # the piece ending with the output takes every end
+            (lo, hi, rd(Int32, ref, o + 16), rd(Int32, ref, o + 16) + rd(Int32, ref, o + 20), rd(Int32, ref, o + 24), rd(Int32, ref, o + 28))
+        end
+        progs = [(e[5], e[6], e) for e in ext]
+        rd(Int32, ref, so) == STAGE_MAP || append!(progs, [(rd(Int32, ref, so + 20), rd(Int32, ref, so + 24), 40),
+                                                           (rd(Int32, ref, so + 28), rd(Int32, ref, so + 32), 48)])
+        for (pr, n, e) in progs
+            reads = Dict{Int,Vector{Any}}()
+            for (k, (b, Lk)) in enumerate(zip(bs, Ls))
+                sk = stage(b, Lk, s)
+                try
+                    if e isa Int                                       # input program over n_in, epilogue over n_out
+                        match!(reads, b, Lk, rd(Int32, b, sk + e - 20), ref, L, pr, n, 0, rd(Int64, b, sk + e), k)
+                        continue
+                    end
+                    for p in rd(Int32, b, sk + 12):rd(Int32, b, sk + 12)+rd(Int32, b, sk + 16)-1
+                        o = piece(b, Lk, p)
+                        lo, hi = rd(Int64, b, o), rd(Int64, b, o) + rd(Int64, b, o + 8)
+                        clo, chi = rd(Int32, b, o + 16), rd(Int32, b, o + 16) + rd(Int32, b, o + 20)
+                        a, z = max(lo, e[1]), min(hi, e[2])
+                        (a < z && max(clo, e[3]) < min(chi, e[4])) || continue
+                        rd(Int32, b, o + 28) == n || throw(Unlike())
+                        match!(reads, b, Lk, rd(Int32, b, o + 24), ref, L, pr, n, a, z, k)
+                    end
+                catch x
+                    x isa Unlike || rethrow()
+                    starts(bb, LL) = [rd(Int64, bb, piece(bb, LL, p)) for p in rd(Int32, bb, stage(bb, LL, s) + 12):rd(Int32, bb, stage(bb, LL, s) + 12)+rd(Int32, bb, stage(bb, LL, s) + 16)-1]
+                    !(e isa Int) && starts(b, Lk) != starts(ref, L) &&
+                        error("batch element $(k-1): a part of the signal starts at a frame that depends on the element's length " *
+                              "(Append after a signal of ragged length); such a batch needs one length")
+                    error("batch element $(k-1) does not lower to the same plan as element $(r-1)")
+                end
+            end
+            max_prog!(out, L, pr, reads, bs, Ls)
+        end
+        if rd(Int32, ref, so) == STAGE_MAP                            # every element's frames lie in the plan's pieces
+            for (k, (b, Lk)) in enumerate(zip(bs, Ls)), p in rd(Int32, b, stage(b, Lk, s) + 12):rd(Int32, b, stage(b, Lk, s) + 12)+rd(Int32, b, stage(b, Lk, s) + 16)-1
+                o = piece(b, Lk, p)
+                lo, hi = rd(Int64, b, o), rd(Int64, b, o) + rd(Int64, b, o + 8)
+                clo, chi = rd(Int32, b, o + 16), rd(Int32, b, o + 16) + rd(Int32, b, o + 20)
+                cover = sum(max(0, min(hi, e[2]) - max(lo, e[1])) * max(0, min(chi, e[4]) - max(clo, e[3])) for e in ext; init = 0)
+                cover == (hi - lo) * (chi - clo) ||
+                    error("batch element $(k-1): a part of the signal starts at a frame that depends on the element's length " *
+                          "(Append after a signal of ragged length); such a batch needs one length")
+            end
+        end
+    end
+    tf = Int64[bufframes(b, Lk, Lk.nin + t) for t in 0:L.ntmp-1, (b, Lk) in zip(bs, Ls)]
+    out, tf
+end
+
+# the largest valid length (and RMS divisor) any element gives each leaf; a buffer leaf whose valid length varies reads
+# zero past it for the longest element: fine for a zero pad that starts where the element's buffer ends
+function max_prog!(out, L, pr, reads, bs, Ls)
+    padname = Dict(PAD_CYCLE => "Pad(x, cycle)", PAD_MIRROR => "Pad(x, mirror)", PAD_LAST => "Pad(x, lastframe)")
+    for (q, rs) in reads
+        J = instr(out, L, pr + q)
+        if out[J+2] == LEAF_RMS
+            wr!(out, J + 40, maximum(rd(Float64, bs[k], I + 40) for (k, I, _, _) in rs))
+            continue
+        end
+        top = maximum(rd(Int64, bs[k], I + 24) for (k, I, _, _) in rs)
+        wr!(out, J + 24, top)
+        out[J+2] == LEAF_STAGE && continue
+        for (k, I, a, z) in rs
+            b = bs[k]
+            i1 = rd(Int64, b, I + 24)
+            (i1 == top || z + rd(Int64, b, I + 16) <= i1) && continue
+            pad, d0 = (b[I+4] >> 1) & 3, rd(Float64, b, I + 40)
+            (pad != PAD_CONST || d0 != 0.0) &&
+                error("batch element $(k-1): $(get(padname, pad, "a pad with the constant $d0 (Pad(x, one), or Amplify / * of signals of different lengths)")) " *
+                      "extends a signal of ragged length; such a batch needs one length")
+            i1 < bufframes(b, Ls[k], rd(Int32, b, I + 4)) &&
+                error("batch element $(k-1): reads a buffer past a valid length shorter than the buffer; such a batch needs one length")
+        end
+    end
 end
 
 # `sink(x, "file.wav")` (src/sink.jl:139-142, src/WAV.jl:3-7) on the GPU sink: the device transposes the result to
